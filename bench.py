@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (NumPy oracle)
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/<name>.npy
 
 A "step" = one pass of the hot path over one batch of synthetic images on every
 rank: InceptionV1 encode -> key projection -> rnn init -> 60-step beam-3 decode
@@ -51,7 +52,14 @@ def parse_args():
                     help='engine arithmetic mode (include/comic_b200.h comic_set_precision)')
     ap.add_argument('--opt', action='append', default=[], help='engine tunable name=value (Engine.set_option)')
     ap.add_argument('--breakdown', action='store_true', help='also print a per-kernel-class time table to stderr')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the decode outputs of the last timed step to DIR/<name>.npy (rank 0; see beam_outputs)')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what the CUDA path computed (--impl ours)')
+    return args
 
 
 def make_config(workload):
@@ -334,6 +342,36 @@ def load_traffic(tag):
     return None
 
 
+DUMP_BYTES = 60 << 20         # --dump-outputs stays under 64 MB, npy headers included
+
+
+def beam_outputs(r, T):
+    """Host copies of what Engine.decode_beam returned (r), for --dump-outputs: the T executed steps only (the rows
+    after them are never written), ids and lengths as float64 (exact), scores and attention maps as float32.  When all
+    of it exceeds DUMP_BYTES (the attention maps of one 512-image step alone are 192 MB), every array is cut to the same
+    fixed, seeded sample of images, listed in `images`; the sample depends on the batch shape only."""
+    import torch
+    B = r['lengths'].shape[0]
+    itemsize = dict(predicted_ids=8, step_ids=8, parent_ids=8, scores=4, lengths=8, attn=4)     # as written
+    per_image = sum(r[k].numel() * s for k, s in itemsize.items()) // B + 8                    # + its `images` entry
+    n = min(B, DUMP_BYTES // per_image)
+    idx = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    sel = torch.from_numpy(idx).to(r['lengths'].device)
+    out = {k: r[k][:T].index_select(1, sel).cpu().numpy().astype(np.float64)
+           for k in ('predicted_ids', 'step_ids', 'parent_ids')}
+    out['scores'] = r['scores'][:T].index_select(1, sel).cpu().numpy().astype(np.float32)
+    out['lengths'] = r['lengths'].index_select(0, sel).cpu().numpy().astype(np.float64)
+    out['attn'] = r['attn'].index_select(0, sel)[:, :, :T].cpu().numpy().astype(np.float32)
+    out['images'] = idx.astype(np.float64)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 # ---------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------
@@ -453,6 +491,9 @@ def run_ours(args):
     sampler.stop()
     ms_total = ev0.elapsed_time(ev1)
     launches = eng.launch_count() - launches0
+    from comic_b200.engine import executed_steps
+    # r lives in the graph's output buffers, which the next step overwrites: copy the last timed step's outputs now
+    dumped = beam_outputs(r, executed_steps(r['T'])) if args.dump_outputs and rank == 0 else None
     # ---- timed region 1b: the same K steps launched one by one with CUDA events around every launch of the two largest
     # kernel classes (events cannot be captured into the graph): the roofline block's launch durations and shares
     eng.profile_enable([dominant, runner_up])
@@ -466,7 +507,6 @@ def run_ours(args):
     dom_ms, dom_n = eng.profile_read(dominant)
     run_ms, run_n = eng.profile_read(runner_up)
     eng.profile_enable([])
-    from comic_b200.engine import executed_steps
     T_exec = executed_steps(r['T'])
 
     # ---- timed region 2: end to end through CaptionModel.run_stream from pinned host memory
@@ -603,6 +643,8 @@ def run_ours(args):
                                               % (args.cpu_sample, T, beam)}
         if train is not None:
             line['train'] = train
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

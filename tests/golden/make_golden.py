@@ -1,16 +1,25 @@
 """Generates the committed golden fixtures in this directory from the NumPy oracle.
 
-    python tests/golden/make_golden.py            # rewrites *.npz
+    python tests/golden/make_golden.py [REFERENCE_CHECKOUT]    # rewrites *.npz (and the reference's records)
 
-The reference itself (TF 1.9 / Python 2.7) cannot run in this container, so the
+The reference itself (TF 1.9 / Python 2.7) cannot run under Python 3, so the
 fixtures are outputs of `oracle/` on seeded inputs, not of the reference; they
 freeze the oracle (tests/test_oracle_known_answers.py) and give the CUDA path a
-target that does not move (tests/test_gpu_parity.py::test_golden_*).  The only
-piece of the reference that imports under Python 3 is its CIDEr-D scorer
-(common/scst/cider_ruotianluo/pyciderevalcap/ciderD); `ciderd_case()` records
-ITS outputs (generated here with /root/reference importable) for the SCST reward.
+target that does not move (tests/test_gpu_parity.py::test_golden_*).  Two
+records come from a checkout of the reference and are rewritten only when one
+is given:
+- ciderd_reference.npz: outputs of the reference's CIDEr-D scorer
+  (common/scst/cider_ruotianluo/pyciderevalcap/ciderD, the one piece of it that
+  imports under Python 3) for the SCST reward;
+- reference_cli_flags.json: name, type, default and choices of every flag of
+  the reference's src/train.py and src/infer.py parsers.  The committed table
+  was written from comic_b200.cli's parsers after they had been matched flag by
+  flag against those sources by `reference_cli_flags()`.
 """
+import ast
+import json
 import os
+import re
 import sys
 
 import numpy as np
@@ -75,12 +84,12 @@ def scst_sentences(seed=11, n_img=6, n_ref=5, n_hyp=3, vocab=40):
     return refs, hyps
 
 
-def ciderd_case():
-    """CIDEr-D scores from the REFERENCE's own scorer (the one module of /root/reference that
-    imports under Python 3), cached-DF mode (the mode train_fn_scst uses).  Needs /root/reference."""
+def ciderd_case(reference):
+    """CIDEr-D scores from the REFERENCE's own scorer (the one module of the reference checkout that
+    imports under Python 3), cached-DF mode (the mode train_fn_scst uses)."""
     import pickle
     import tempfile
-    sys.path.insert(0, '/root/reference/common/scst/cider_ruotianluo')
+    sys.path.insert(0, os.path.join(reference, 'common', 'scst', 'cider_ruotianluo'))
     from pyciderevalcap.ciderD.ciderD import CiderD as RefCiderD
     from comic_b200 import scst as S
     refs, hyps = scst_sentences()
@@ -96,13 +105,50 @@ def ciderd_case():
     return dict(cached=np.asarray(sc_c, np.float64), mean_cached=np.float64(mean_c))
 
 
-def main():
+PATH_FLAGS = ('infer_checkpoints_dir', 'dataset_dir')      # defaults are path expressions of the reference's checkout
+
+
+def reference_cli_flags(reference):
+    """{'train.py' | 'infer.py': {flag: {'type', 'default', 'choices'}}} parsed from the add_argument calls of the
+    reference's src/train.py and src/infer.py (no default recorded for PATH_FLAGS)."""
+    out = {}
+    for fname in ('train.py', 'infer.py'):
+        with open(os.path.join(reference, 'src', fname)) as f:
+            src = f.read()
+        flags = {}
+        for m in re.finditer(r"add_argument\(\s*'--(\w+)'(.*?)help=", src, re.S):
+            name, body = m.group(1), m.group(2)
+            t = re.search(r"type=(\w+)", body)
+            d = re.search(r"default=(.+?),\s*(?:choices=|$)", body.strip(), re.S)
+            c = re.search(r"choices=(\[.*?\])", body, re.S)
+            spec = {'type': t.group(1) if t else None}
+            if name not in PATH_FLAGS:
+                spec['default'] = eval(d.group(1).strip().rstrip(',')) if d else None
+            spec['choices'] = ast.literal_eval(c.group(1)) if c else None
+            flags[name] = spec
+        out[fname] = flags
+    return out
+
+
+def write_reference_cli_flags(table, path):
+    """One line per flag, so that a change of the table reads as a change of that flag."""
+    lines = []
+    for fname, flags in table.items():
+        rows = ['  %s: %s' % (json.dumps(name), json.dumps(spec)) for name, spec in flags.items()]
+        lines.append(' %s: {\n%s\n }' % (json.dumps(fname), ',\n'.join(rows)))
+    with open(path, 'w') as f:
+        f.write('{\n%s\n}\n' % ',\n'.join(lines))
+
+
+def main(argv):
     np.savez_compressed(os.path.join(HERE, 'decoder_beam_comic256.npz'), **decoder_beam_case())
     np.savez_compressed(os.path.join(HERE, 'encoder_2img.npz'), **encoder_case())
-    if os.path.isdir('/root/reference'):
-        np.savez_compressed(os.path.join(HERE, 'ciderd_reference.npz'), **ciderd_case())
+    if argv:
+        reference = argv[0]
+        np.savez_compressed(os.path.join(HERE, 'ciderd_reference.npz'), **ciderd_case(reference))
+        write_reference_cli_flags(reference_cli_flags(reference), os.path.join(HERE, 'reference_cli_flags.json'))
     print('wrote fixtures to', HERE)
 
 
 if __name__ == '__main__':
-    main()
+    main(sys.argv[1:])

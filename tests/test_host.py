@@ -1,15 +1,22 @@
 """Host-side logic (CPU): config.pkl contract, flag defaults against the
-reference's argparse (when /root/reference is mounted), radix helpers."""
+reference's argparse (recorded in tests/golden/reference_cli_flags.json), radix helpers."""
+import json
 import os
 import pickle
-import re
 
 import pytest
 
 import comic_b200  # noqa: F401
 from comic_b200 import configuration as conf
 
-REF = '/root/reference/src'
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+PATH_FLAGS = ('infer_checkpoints_dir', 'dataset_dir')      # defaults are path expressions of the reference's checkout
+
+
+def _reference_cli():
+    """{'train.py' | 'infer.py': {flag: {'type', 'default', 'choices'}}} of the reference's two argparse parsers."""
+    with open(os.path.join(GOLDEN, 'reference_cli_flags.json')) as f:
+        return json.load(f)
 
 
 def test_config_pickle_round_trip(tmp_path):
@@ -54,32 +61,17 @@ def test_none_string_becomes_none_and_mode_overrides():
     assert leg.rnn_init_method == 'project_hidden' and leg.attn_keep_prob == 1.0 and leg.adam_epsilon == 1e-6
 
 
-def _argparse_defaults(path):
-    """(flag -> default literal) scraped from the reference's add_argument calls."""
-    src = open(path).read()
-    out = {}
-    for m in re.finditer(r"add_argument\(\s*'--(\w+)'(.*?)\)\s*\n", src, flags=re.S):
-        d = re.search(r"default=([^,\n]+)", m.group(2))
-        if d:
-            out[m.group(1)] = d.group(1).strip()
-    return out
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not mounted')
 def test_flag_defaults_match_reference_cli():
     """Every flag of src/train.py:29-162 / src/infer.py:27-72 exists with the same default."""
-    import ast
+    ref_cli = _reference_cli()
     for fname, table in (('train.py', conf.TRAIN_DEFAULTS), ('infer.py', conf.INFER_DEFAULTS)):
-        ref = _argparse_defaults(os.path.join(REF, fname))
+        ref = ref_cli[fname]
         assert len(ref) > 10
-        for flag, lit in ref.items():
-            if flag in ('gpu', 'per_process_gpu_memory_fraction', 'dataset_dir', 'infer_checkpoints_dir'):
+        for flag, spec in ref.items():
+            if flag in ('gpu', 'per_process_gpu_memory_fraction') + PATH_FLAGS:
                 continue
             assert flag in table, '%s: flag --%s missing' % (fname, flag)
-            try:
-                val = ast.literal_eval(lit)
-            except Exception:
-                continue
+            val = spec['default']
             ours = table[flag]
             if flag == 'cnn_input_size':
                 val = [int(v) for v in val.split(',')]
@@ -110,24 +102,7 @@ def test_synthetic_vocab_layout():
 # ---------------------------------------------------------------------------
 # CLI mirror (src/train.py:25-164, src/infer.py:23-74)
 # ---------------------------------------------------------------------------
-def _reference_flags(path):
-    """(name -> (type name, default literal, choices literal)) parsed from an argparse source file."""
-    import ast
-    import re
-    src = open(path).read()
-    out = {}
-    for m in re.finditer(r"add_argument\(\s*'--(\w+)'(.*?)help=", src, re.S):
-        name, body = m.group(1), m.group(2)
-        t = re.search(r"type=(\w+)", body)
-        d = re.search(r"default=(.+?),\s*(?:choices=|$)", body.strip(), re.S)
-        c = re.search(r"choices=(\[.*?\])", body, re.S)
-        out[name] = (t.group(1) if t else None, d.group(1).strip().rstrip(',') if d else None,
-                     ast.literal_eval(c.group(1)) if c else None)
-    return out
-
-
 def test_cli_parsers_mirror_reference_flags():
-    import os
     from comic_b200 import cli
     tp, ip = cli.create_train_parser(), cli.create_infer_parser()
     ours_t = {a.dest: a for a in tp._actions if a.dest != 'help'}
@@ -137,19 +112,17 @@ def test_cli_parsers_mirror_reference_flags():
     assert ours_t['attn_num_heads'].default == 8 and ours_t['scst_beam_size'].default == 7
     assert ours_t['cnn_input_size'].default == '224,224' and ours_t['adam_epsilon'].default == 1e-2
     assert ours_i['infer_beam_size'].default == 3 and ours_i['batch_size_infer'].default == 25
-    ref_dir = '/root/reference/src'
-    if not os.path.exists(os.path.join(ref_dir, 'train.py')):
-        return
+    ref_cli = _reference_cli()
     for ours, fname in ((ours_t, 'train.py'), (ours_i, 'infer.py')):
-        ref = _reference_flags(os.path.join(ref_dir, fname))
+        ref = ref_cli[fname]
         assert set(ref) == set(ours), (set(ref) ^ set(ours))
-        for name, (tname, dflt, choices) in ref.items():
+        for name, spec in ref.items():
             a = ours[name]
-            assert a.type.__name__ == tname, name
-            assert (list(a.choices) if a.choices else None) == choices, name
-            if name in ('infer_checkpoints_dir', 'dataset_dir'):
-                continue                                   # path expressions of the reference's checkout
-            assert a.default == eval(dflt), (name, a.default, dflt)
+            assert a.type.__name__ == spec['type'], name
+            assert (list(a.choices) if a.choices else None) == spec['choices'], name
+            if name in PATH_FLAGS:
+                continue
+            assert a.default == spec['default'], (name, a.default, spec['default'])
 
 
 def test_cli_config_assembly():
