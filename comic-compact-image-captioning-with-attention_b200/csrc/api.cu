@@ -193,10 +193,30 @@ extern "C" int comic_packed_bytes(comic_handle_t h, size_t* bytes) {
   COMIC_REQUIRE(h && bytes, COMIC_E_BADARG, "packed_bytes: null argument");
   Carver cv(nullptr);
   comic::Packed keep = h->pk;
+  h->sized = true;
   decoder_pack(h, cv, 0, true);
   encoder_pack(h, cv, 0, true);
   h->pk = keep;
   *bytes = cv.off + 256;
+  return COMIC_OK;
+}
+
+extern "C" int comic_set_rnn_cell(comic_handle_t h, int cell) {
+  COMIC_REQUIRE(h, COMIC_E_BADARG, "set_rnn_cell: null handle");
+  COMIC_REQUIRE(cell == COMIC_CELL_LSTM || cell == COMIC_CELL_GRU, COMIC_E_UNSUPPORTED,
+                "set_rnn_cell: cell %d is not built (0 LSTM, 1 GRU)", cell);
+  COMIC_REQUIRE(!h->bound && !h->sized, COMIC_E_BADARG,
+                "set_rnn_cell: call it before any size query or binding (packed and workspace layouts depend on the cell)");
+  h->cell = cell;
+  return COMIC_OK;
+}
+
+extern "C" int comic_bind_gru_candidate(comic_handle_t h, const float* kernel, const float* bias) {
+  COMIC_REQUIRE(h && kernel && bias, COMIC_E_BADARG, "bind_gru_candidate: null argument");
+  COMIC_REQUIRE(h->cell == COMIC_CELL_GRU, COMIC_E_BADARG, "bind_gru_candidate: the handle's cell is not GRU");
+  h->gru_cand_kernel = kernel;
+  h->gru_cand_bias = bias;
+  h->bound = false;   // the packed panels were built from the previous candidate: decoding waits for comic_bind_weights
   return COMIC_OK;
 }
 
@@ -212,6 +232,9 @@ extern "C" int comic_bind_weights(comic_handle_t h, const comic_weights_t* w, in
   if (h->cfg.alignment == 0)
     COMIC_REQUIRE(w->attention_v && w->ln_gamma && w->ln_beta && w->temperature, COMIC_E_BADARG,
                   "bind_weights: missing add_LN attention tensor");
+  if (h->cell == COMIC_CELL_GRU)
+    COMIC_REQUIRE(h->gru_cand_kernel && h->gru_cand_bias, COMIC_E_BADARG,
+                  "bind_weights: GRU cell without candidate/{kernel, bias} (comic_bind_gru_candidate)");
   if (h->cfg.fm_projection == 2) COMIC_REQUIRE(w->value_kernel, COMIC_E_BADARG, "bind_weights: missing value_layer");
   if (h->cfg.context_layer) COMIC_REQUIRE(w->a_layer, COMIC_E_BADARG, "bind_weights: missing a_layer");
   if (with_cnn) {
@@ -238,6 +261,7 @@ extern "C" int comic_bind_weights(comic_handle_t h, const comic_weights_t* w, in
 extern "C" int comic_workspace_bytes(comic_handle_t h, int mode, int B, int k, int T, size_t* bytes) {
   COMIC_REQUIRE(h && bytes, COMIC_E_BADARG, "workspace_bytes: null argument");
   COMIC_REQUIRE(B > 0 && k > 0 && T >= 0, COMIC_E_SHAPE, "workspace_bytes: bad B=%d k=%d T=%d", B, k, T);
+  h->sized = true;
   if (mode == 0) return encoder_workspace_bytes(h, B, bytes);
   if (mode == 5) {   // gemm_f32 tensor-path scratch: B = N, k = K of the GEMM (B^T hi/lo pack)
     *bytes = 2 * (size_t)round_up(B, 16) * round_up(k, tc::BK) * sizeof(float) + 2048;

@@ -54,6 +54,10 @@ struct Packed {
   tc::TcWeight tc_lstm, tc_outq, tc_mem, tc_val, tc_init;
   tc::TcWeight tc_lstm_il;       // lstm kernel with gate-interleaved columns (fused LSTM epilogue of the gate GEMM)
   float* lstm_bias_il = nullptr; // [4R] bias in the same column order
+  // GRU cell: [gates/kernel | candidate/kernel x-rows ; 0] panel [W+A+R, 3R] of the gate GEMM, and the tensor-path packs
+  // of that panel and of the candidate kernel's h-rows [R, R]
+  float* gru_gx = nullptr;
+  tc::TcWeight tc_gru_g, tc_gru_c;
   tc::TcWeight tc_stem_s2d;      // Conv2d_1a_7x7 as a 4x4 conv over the space-to-depth image: W2 [4,4,16,64]
 };
 
@@ -70,7 +74,11 @@ struct comic_handle_s {
   int num_sms = 148;
   int R, W, H, C, M, E, V, Vp, A, VAL, LQ, KX;
   comic_weights_t w;
+  int cell = COMIC_CELL_LSTM;              // comic_set_rnn_cell
+  const float* gru_cand_kernel = nullptr;  // GRU candidate/{kernel [W+A+R, R], bias [R]} (comic_bind_gru_candidate);
+  const float* gru_cand_bias = nullptr;    // gates/{kernel, bias} travel in w.lstm_kernel / w.lstm_bias
   bool bound = false, cnn_bound = false;
+  bool sized = false;                      // a packed / workspace size was handed out (laid out for `cell`)
   int precision = 1;   // 0: fp32 FFMA everywhere; 1: tcgen05 split-precision GEMMs with M >= 128; 2: 1 + tanh.approx
   int fused_min_images = 48;   // fused attention kernel (one CTA per image) from this batch size on
   int attn2_min_images = 12;   // streaming kernel (attention2.cuh) from this batch size on while fused_min_images is at its
@@ -213,6 +221,7 @@ struct StepBufs {
   uint16_t *hp_hi, *hp_lo;   // [N][R]
   ATma xmaps, hmaps;
   bool tma_a;
+  float* gru;          // GRU cell only: [3][N][R] = r * h[src], u, x . candidate/kernel x-rows
 };
 
 struct StepIO {
@@ -244,6 +253,7 @@ struct StepIO {
 };
 
 int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int k, cudaStream_t st);
+int gru_init_step(comic_handle_t h, const float* x0, int B, float* part, float* gru, float* h0, float* tape, cudaStream_t st);
 // Once per decode call (keys fixed): decides whether the streaming attention kernel applies to (B, k) and, if so, fills
 // sb.kstats / sb.abound and points io at them.  Returns < 0 on error.
 int attn2_prepare(comic_handle_t h, StepIO& io, const StepBufs& sb, int B, int k, bool masks, cudaStream_t st);

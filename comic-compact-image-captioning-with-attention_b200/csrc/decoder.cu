@@ -19,6 +19,8 @@
 #include <float.h>
 #include <math.h>
 
+#include <algorithm>
+
 #include "attention.cuh"
 #include "beam_warp.cuh"
 #include "attention2.cuh"
@@ -115,6 +117,90 @@ lstm_pointwise4_kernel(const float* __restrict__ gates, const float* __restrict_
     *reinterpret_cast<uint2*>(h_hi + (size_t)n * R + j) = hi;
     *reinterpret_cast<uint2*>(h_lo + (size_t)n * R + j) = lo;
   }
+}
+
+// ---------------------------------------------------------------------------
+// D3, GRU cell (TF r1.9 GRUCell, src/model_base.py:622-629):
+//   [r, u] = sigmoid([x, h] . gates/kernel + gates/bias)
+//   c      = tanh([x, r*h] . candidate/kernel + candidate/bias)
+//   h'     = u*h + (1-u)*c
+// The gate GEMM multiplies [x, h] by the panel [gates/kernel | candidate/kernel x-rows ; 0] into split-K partials
+// [nz][N][3R] (r, u pre-activations, then x . Kc_x).  gru_gate_kernel sums them in a fixed order, takes the sigmoids and
+// writes r * h[src] (the A operand of the candidate GEMM), u and x . Kc_x to [3][N][R]; the candidate GEMM adds
+// (r*h) . Kc_h and gru_update_kernel forms c and h'.  h_prev == nullptr is the zero state (first_input init step).
+// FAST (tensor path): sigmoid / tanh through ex2.approx + rcp.approx, as lstm_pointwise4_kernel<true>.
+// ---------------------------------------------------------------------------
+template <bool FAST>
+__global__ void __launch_bounds__(256)
+gru_gate_kernel(const float* __restrict__ gp, int nz, size_t zstride, const float* __restrict__ bias,
+                const float* __restrict__ h_prev, const int* __restrict__ src, int src_limit, int N, int R,
+                float* __restrict__ gru, const int* fin_count, int t, int n_rows, float* __restrict__ tape = nullptr) {
+  if (step_stopped(fin_count, t, n_rows)) return;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N * R) return;
+  const int n = i / R, j = i - n * R;
+  const float* g = gp + (size_t)n * 3 * R + j;
+  float s[3];
+#pragma unroll
+  for (int q = 0; q < 3; ++q) {
+    float v = 0.f;
+    for (int z = 0; z < nz; ++z) v += g[z * zstride + q * R];
+    s[q] = v;
+  }
+  const float r = sig_<FAST>(s[0] + bias[j]);
+  const float u = sig_<FAST>(s[1] + bias[R + j]);
+  float hp = 0.f;
+  if (h_prev) {
+    const int row = src ? src[n] : n;
+    if (row >= 0 && row < src_limit) hp = h_prev[(size_t)row * R + j];
+  }
+  const size_t NR = (size_t)N * R;
+  gru[i] = r * hp;
+  gru[NR + i] = u;
+  gru[2 * NR + i] = s[2];
+  if (tape) {   // training tape, row [r | u | r*h | c] (c: gru_update_kernel)
+    float* tr = tape + (size_t)n * 4 * R + j;
+    tr[0] = r; tr[R] = u; tr[2 * R] = r * hp;
+  }
+}
+
+// cp: split-K partials [nz][N][R] of (r*h) . Kc_h (nz = 0: r*h is zero).  Output dropout as lstm_pointwise_kernel.
+template <bool FAST>
+__global__ void __launch_bounds__(256)
+gru_update_kernel(const float* __restrict__ cp, int nz, size_t zstride, const float* __restrict__ gru,
+                  const float* __restrict__ bias, const float* __restrict__ h_prev, const int* __restrict__ src, int src_limit,
+                  float* __restrict__ h_new, float* __restrict__ h_drop, const float* __restrict__ out_mask, float out_keep,
+                  int N, int R, const int* fin_count, int t, int n_rows, float* __restrict__ tape = nullptr) {
+  if (step_stopped(fin_count, t, n_rows)) return;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N * R) return;
+  const int n = i / R, j = i - n * R;
+  const size_t NR = (size_t)N * R;
+  float s = gru[2 * NR + i];
+  for (int z = 0; z < nz; ++z) s += cp[z * zstride + i];
+  const float c = tanh_<FAST>(s + bias[j]);
+  if (tape) tape[(size_t)n * 4 * R + 3 * R + j] = c;
+  const float u = gru[NR + i];
+  float hp = 0.f;
+  if (h_prev) {
+    const int row = src ? src[n] : n;
+    if (row >= 0 && row < src_limit) hp = h_prev[(size_t)row * R + j];
+  }
+  const float hn = u * hp + (1.f - u) * c;
+  h_new[i] = hn;
+  if (h_drop) h_drop[i] = out_mask ? (hn / out_keep) * out_mask[i] : hn;
+}
+
+// [gates/kernel | candidate/kernel x-rows ; 0]: the [W+A+R, 3R] B operand of the GRU gate GEMM.
+__global__ void pack_gru_gates_kernel(const float* __restrict__ kg, const float* __restrict__ kc, float* __restrict__ out,
+                                      int KX, int XA, int R) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (size_t)KX * 3 * R) return;
+  const int row = (int)(i / (3 * R)), col = (int)(i % (3 * R));
+  float v;
+  if (col < 2 * R) v = kg[(size_t)row * 2 * R + col];
+  else v = row < XA ? kc[(size_t)row * R + (col - 2 * R)] : 0.f;
+  out[i] = v;
 }
 
 // x = [emb(tok) ; ctx[src] ; h[src]] of one decode step as bf16 (hi, lo) planes [N][W + A + R] for the gate GEMM's TMA-staged A
@@ -762,12 +848,18 @@ __global__ void interleave_gate_bias_kernel(const float* __restrict__ bias, floa
 static int decoder_pack_tc(comic_handle_t h, Carver& cv, cudaStream_t st, bool dry) {
   int rc;
   const int XA = h->W + h->A;
-  if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm, st, dry))) return rc;
-  if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm_il, st, dry, h->R))) return rc;
-  h->pk.lstm_bias_il = cv.take<float>((size_t)4 * h->R);
-  if (!dry) {
-    interleave_gate_bias_kernel<<<(4 * h->R + 255) / 256, 256, 0, st>>>(h->w.lstm_bias, h->pk.lstm_bias_il, h->R);
-    COMIC_CHECK_CUDA(cudaGetLastError());
+  if (h->cell == COMIC_CELL_GRU) {
+    if ((rc = pack_tc_weight(h, cv, h->pk.gru_gx, h->KX, 3 * h->R, 3 * h->R, 1, 1, h->pk.tc_gru_g, st, dry))) return rc;
+    if ((rc = pack_tc_weight(h, cv, h->gru_cand_kernel + (size_t)XA * h->R, h->R, h->R, h->R, 1, 1, h->pk.tc_gru_c, st, dry)))
+      return rc;
+  } else {
+    if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm, st, dry))) return rc;
+    if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm_il, st, dry, h->R))) return rc;
+    h->pk.lstm_bias_il = cv.take<float>((size_t)4 * h->R);
+    if (!dry) {
+      interleave_gate_bias_kernel<<<(4 * h->R + 255) / 256, 256, 0, st>>>(h->w.lstm_bias, h->pk.lstm_bias_il, h->R);
+      COMIC_CHECK_CUDA(cudaGetLastError());
+    }
   }
   if ((rc = pack_tc_weight(h, cv, h->pk.outq, h->R, h->LQ, h->LQ, 1, 1, h->pk.tc_outq, st, dry))) return rc;
   if ((rc = pack_tc_weight(h, cv, h->w.memory_kernel, h->C, h->R, h->R, 1, 1, h->pk.tc_mem, st, dry))) return rc;
@@ -781,11 +873,18 @@ static int decoder_pack_tc(comic_handle_t h, Carver& cv, cudaStream_t st, bool d
 int decoder_pack(comic_handle_t h, Carver& cv, cudaStream_t st, bool dry) {
   h->pk.outq = cv.take<float>((size_t)h->R * h->LQ);
   h->pk.outq_bias = cv.take<float>(h->LQ);
+  if (h->cell == COMIC_CELL_GRU) h->pk.gru_gx = cv.take<float>((size_t)h->KX * 3 * h->R);
   if (dry) return decoder_pack_tc(h, cv, st, true);
   size_t n = (size_t)h->R * h->LQ;
   pack_outq_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(h->w.out_kernel, h->w.out_bias, h->w.query_kernel,
                                                                h->pk.outq, h->pk.outq_bias, h->R, h->V, h->Vp);
   COMIC_CHECK_CUDA(cudaGetLastError());
+  if (h->cell == COMIC_CELL_GRU) {
+    const size_t ng = (size_t)h->KX * 3 * h->R;
+    pack_gru_gates_kernel<<<(unsigned)((ng + 255) / 256), 256, 0, st>>>(h->w.lstm_kernel, h->gru_cand_kernel, h->pk.gru_gx,
+                                                                       h->KX, h->W + h->A, h->R);
+    COMIC_CHECK_CUDA(cudaGetLastError());
+  }
   return decoder_pack_tc(h, cv, st, false);
 }
 
@@ -975,6 +1074,76 @@ int attn2_prepare(comic_handle_t h, StepIO& io, const StepBufs& sb, int B, int k
   return COMIC_OK;
 }
 
+static int step_tail(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int k, bool tma_lq, cudaStream_t st);
+
+// The GRU cell of one step (see gru_gate_kernel): gate GEMM, gate kernel, candidate GEMM, update kernel.  The two GEMMs
+// take the tensor / FFMA paths and split-K choices of the LSTM gate GEMM; their partials share StepBufs::gates.
+static int run_gru_cell(comic_handle_t h, const StepIO& io, const StepBufs& sb, const APlain& a, int N, cudaStream_t st) {
+  const int R = h->R, tot = N * R;
+  const int* stop = io.fin_count ? io.fin_count + (io.t > 0 ? io.t - 1 : 0) : nullptr;
+  const int stop_n = (io.fin_count && io.t > 0) ? io.n_rows : 0x7fffffff;
+  const bool tc1 = use_tc_step(h, h->pk.tc_gru_g, N, 3 * R, h->KX, 1);
+  GemmPlan p1 = plan_gemm(N, 3 * R, h->KX, h->num_sms, true);
+  const int ks1 = tc1 ? tc_ksplit(h, N, 3 * R, h->KX, 1) : 1;
+  const int nz1 = tc1 ? ks1 : gemm_num_partials(h->KX, p1);
+  Epi e1{};
+  e1.nroute = 1;
+  e1.r[0] = Route{0, 3 * R, sb.gates, 3 * R, 0};
+  e1.split_stride = (long long)N * 3 * R;
+  e1.ksplit = ks1;
+  e1.stop = stop;
+  e1.stop_n = stop_n;
+  e1.pdl = 1;
+  {
+    Prof pf(h, T_GATES, st);
+    if (tc1) COMIC_CHECK_CUDA((tc::launch_gemm_tc<0>(a, h->pk.tc_gru_g, N, 3 * R, e1, h->num_sms, st)));
+    else COMIC_CHECK_CUDA((launch_gemm<0, 4>(a, h->pk.gru_gx, 3 * R, N, 3 * R, h->KX, e1, p1, st)));
+  }
+  {
+    Prof pf(h, T_LSTM, st);
+    if (tc1)
+      gru_gate_kernel<true><<<(tot + 255) / 256, 256, 0, st>>>(sb.gates, nz1, (size_t)N * 3 * R, h->w.lstm_bias, io.h_prev, io.src,
+                                                              io.src_limit, N, R, sb.gru, io.fin_count, io.t, io.n_rows, io.gates_save);
+    else
+      gru_gate_kernel<false><<<(tot + 255) / 256, 256, 0, st>>>(sb.gates, nz1, (size_t)N * 3 * R, h->w.lstm_bias, io.h_prev, io.src,
+                                                               io.src_limit, N, R, sb.gru, io.fin_count, io.t, io.n_rows, io.gates_save);
+  }
+  // candidate GEMM: (r*h) . candidate/kernel h-rows
+  APlain ac{};
+  ac.nseg = 1;
+  ac.seg[0] = ASeg{sb.gru, nullptr, R, R, N};
+  const float* kc_h = h->gru_cand_kernel + (size_t)(h->W + h->A) * R;
+  const bool tc2 = use_tc_step(h, h->pk.tc_gru_c, N, R, R, 1);
+  GemmPlan p2 = plan_gemm(N, R, R, h->num_sms, true);
+  const int ks2 = tc2 ? tc_ksplit(h, N, R, R, 1) : 1;
+  const int nz2 = tc2 ? ks2 : gemm_num_partials(R, p2);
+  Epi e2{};
+  e2.nroute = 1;
+  e2.r[0] = Route{0, R, sb.gates, R, 0};
+  e2.split_stride = (long long)N * R;
+  e2.ksplit = ks2;
+  e2.stop = stop;
+  e2.stop_n = stop_n;
+  {
+    Prof pf(h, T_GATES, st);
+    if (tc2) COMIC_CHECK_CUDA((tc::launch_gemm_tc<0>(ac, h->pk.tc_gru_c, N, R, e2, h->num_sms, st)));
+    else COMIC_CHECK_CUDA((launch_gemm<0, 4>(ac, kc_h, R, N, R, R, e2, p2, st)));
+  }
+  {
+    Prof pf(h, T_LSTM, st);
+    if (tc1 || tc2)
+      gru_update_kernel<true><<<(tot + 255) / 256, 256, 0, st>>>(sb.gates, nz2, (size_t)N * R, sb.gru, h->gru_cand_bias, io.h_prev,
+                                                                io.src, io.src_limit, io.h_new, io.h_drop, io.out_mask, io.out_keep,
+                                                                N, R, io.fin_count, io.t, io.n_rows, io.gates_save);
+    else
+      gru_update_kernel<false><<<(tot + 255) / 256, 256, 0, st>>>(sb.gates, nz2, (size_t)N * R, sb.gru, h->gru_cand_bias, io.h_prev,
+                                                                 io.src, io.src_limit, io.h_new, io.h_drop, io.out_mask, io.out_keep,
+                                                                 N, R, io.fin_count, io.t, io.n_rows, io.gates_save);
+  }
+  COMIC_CHECK_CUDA(cudaGetLastError());
+  return COMIC_OK;
+}
+
 // One attention-wrapper step on N = B*k rows.
 int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int k, cudaStream_t st) {
   const int N = B * k, R = h->R, W = h->W, A = h->A;
@@ -998,6 +1167,11 @@ int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int 
     a.seg[0] = ASeg{h->w.embedding_map, io.tok, W, W, h->V};
     a.seg[1] = ASeg{io.ctx_prev, io.src, A, A, io.src_limit};
     a.seg[2] = ASeg{io.h_prev, io.src, R, R, io.src_limit};
+  }
+  if (h->cell == COMIC_CELL_GRU) {
+    const int rc = run_gru_cell(h, io, sb, a, N, st);
+    if (rc) return rc;
+    return step_tail(h, io, sb, B, k, false, st);
   }
   const bool tc1 = use_tc_step(h, h->pk.tc_lstm, N, 4 * R, h->KX, 1);
   GemmPlan p1 = plan_gemm(N, 4 * R, h->KX, h->num_sms, true);
@@ -1062,6 +1236,15 @@ int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int 
                                                           io.h_drop, io.out_mask, io.out_keep, N, R, io.fin_count,
                                                           io.t, io.n_rows, io.gates_save);
   }
+  return step_tail(h, io, sb, B, k, tma_lq, st);
+}
+
+// [logits | q] GEMM and attention of a step, after the cell has written h' (io.h_new / io.h_drop).
+static int step_tail(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int k, bool tma_lq, cudaStream_t st) {
+  const int N = B * k, R = h->R, A = h->A;
+  Epi e1{};   // stop condition of the step's launches
+  e1.stop = io.fin_count ? io.fin_count + (io.t > 0 ? io.t - 1 : 0) : nullptr;
+  e1.stop_n = (io.fin_count && io.t > 0) ? io.n_rows : 0x7fffffff;
   // --- [logits | q] = h_out . [W_o | W_q] + [b_o | 0] ---
   const float* hq = io.h_drop ? io.h_drop : io.h_new;
   APlain a2{};
@@ -1129,13 +1312,47 @@ int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int 
   return COMIC_OK;
 }
 
+// GRU step from the zero state (first_input init, src/model_base.py:675-686): h0 = (1 - u0) * tanh(x0 . Kc_x + b_c), from the
+// gate panel's x-rows; r * h is zero, so there is no candidate GEMM.  part: >= 16 * B * 3R floats of split-K partials,
+// gru: [3][B][R]; tape (training) receives the rows [r0 | u0 | 0 | c0].
+int gru_init_step(comic_handle_t h, const float* x0, int B, float* part, float* gru, float* h0, float* tape, cudaStream_t st) {
+  const int R = h->R, XA = h->W + h->A;
+  APlain a{};
+  a.nseg = 1;
+  a.seg[0] = ASeg{x0, nullptr, XA, XA, B};
+  GemmPlan pg = plan_gemm(B, 3 * R, XA, h->num_sms, true);
+  const int nz = gemm_num_partials(XA, pg);
+  Epi eg{};
+  eg.nroute = 1;
+  eg.stop_n = 0x7fffffff;
+  eg.r[0] = Route{0, 3 * R, part, 3 * R, 0};
+  eg.split_stride = (long long)B * 3 * R;
+  COMIC_CHECK_CUDA((launch_gemm<0, 4>(a, h->pk.gru_gx, 3 * R, B, 3 * R, XA, eg, pg, st)));
+  const int tot = B * R;
+  gru_gate_kernel<false><<<(tot + 255) / 256, 256, 0, st>>>(part, nz, (size_t)B * 3 * R, h->w.lstm_bias, nullptr, nullptr, 0, B, R,
+                                                           gru, nullptr, 0, 0, tape);
+  gru_update_kernel<false><<<(tot + 255) / 256, 256, 0, st>>>(nullptr, 0, 0, gru, h->gru_cand_bias, nullptr, nullptr, 0, h0, nullptr,
+                                                             nullptr, 1.f, B, R, nullptr, 0, 0, tape);
+  h->launches += 3;
+  COMIC_CHECK_CUDA(cudaGetLastError());
+  return COMIC_OK;
+}
+
 void carve_step(comic_handle_t h, Carver& cv, int N, StepBufs& sb, bool train_masks) {
   GemmPlan p1 = plan_gemm(N, 4 * h->R, h->KX, h->num_sms, true);
   int nz1 = gemm_num_partials(h->KX, p1);
   { const int ks = tc_ksplit_shape(h->num_sms, N, 4 * h->R, h->KX); if (nz1 < ks) nz1 = ks; }   // tensor-path split-K partials
   GemmPlan p2 = plan_gemm(N, h->LQ, h->R, h->num_sms, true);
   int nz2 = gemm_num_partials(h->R, p2);
-  sb.gates = cv.take<float>((size_t)nz1 * N * 4 * h->R);
+  size_t ngates = (size_t)nz1 * N * 4 * h->R;
+  if (h->cell == COMIC_CELL_GRU) {   // partials of the gate GEMM [N][3R] and, after the gate kernel, of the candidate GEMM [N][R]
+    GemmPlan pg = plan_gemm(N, 3 * h->R, h->KX, h->num_sms, true), pc = plan_gemm(N, h->R, h->R, h->num_sms, true);
+    const int nzg = std::max(gemm_num_partials(h->KX, pg), tc_ksplit_shape(h->num_sms, N, 3 * h->R, h->KX));
+    const int nzc = std::max(gemm_num_partials(h->R, pc), tc_ksplit_shape(h->num_sms, N, h->R, h->R));
+    ngates = std::max((size_t)nzg * N * 3 * h->R, (size_t)nzc * N * h->R);
+  }
+  sb.gates = cv.take<float>(ngates);
+  sb.gru = (h->cell == COMIC_CELL_GRU) ? cv.take<float>((size_t)3 * N * h->R) : nullptr;
   { const int ks = tc_ksplit_shape(h->num_sms, N, h->LQ, h->R); if (nz2 < ks) nz2 = ks; }
   sb.lq_part = cv.take<float>(nz2 > 1 ? (size_t)nz2 * N * h->LQ : 1);
   sb.lq = cv.take<float>((size_t)N * h->LQ);
@@ -1148,7 +1365,7 @@ void carve_step(comic_handle_t h, Carver& cv, int N, StepBufs& sb, bool train_ma
   sb.a2_scratch = cv.take<float>(a2ok ? a2::scratch_floats(h->num_sms) : 1);
   sb.a2_counters = cv.take<int>(a2ok ? (size_t)N : 1);
   // TMA-staged A planes (see StepBufs); the maps are encoded when the workspace is real
-  const bool planes = h->tma_a && !train_masks && N >= 128 && h->KX % 8 == 0 && h->R % 8 == 0 && h->W % 4 == 0 && h->A % 4 == 0;
+  const bool planes = h->tma_a && h->cell == COMIC_CELL_LSTM && !train_masks && N >= 128 && h->KX % 8 == 0 && h->R % 8 == 0 && h->W % 4 == 0 && h->A % 4 == 0;
   sb.xp_hi = cv.take<uint16_t>(planes ? (size_t)N * h->KX : 8);
   sb.xp_lo = cv.take<uint16_t>(planes ? (size_t)N * h->KX : 8);
   sb.hp_hi = cv.take<uint16_t>(planes ? (size_t)N * h->R : 8);
@@ -1179,7 +1396,7 @@ static void carve_loop(comic_handle_t h, Carver& cv, int B, int k, int T, bool w
   int N = B * k;
   carve_step(h, cv, N, lb.sb, false);
   for (int i = 0; i < 2; ++i) {
-    lb.c[i] = cv.take<float>((size_t)N * h->R);
+    lb.c[i] = (h->cell == COMIC_CELL_GRU) ? nullptr : cv.take<float>((size_t)N * h->R);
     lb.h[i] = cv.take<float>((size_t)N * h->R);
     lb.ctx[i] = cv.take<float>((size_t)N * h->A);
   }
@@ -1282,6 +1499,7 @@ extern "C" int comic_rnn_init(comic_handle_t h, const float* im_embed, int B, fl
     e.r[0] = Route{0, R, h0, R, 0};
     GemmPlan p = plan_gemm(B, R, h->E, h->num_sms, false);
     COMIC_CHECK_CUDA((launch_gemm<0, 4>(a, h->w.init_weight, R, B, R, h->E, e, p, st)));
+    if (h->cell == COMIC_CELL_GRU) return COMIC_OK;   // state h only
     COMIC_CHECK_CUDA(cudaMemsetAsync(c0, 0, (size_t)B * R * sizeof(float), st));
     h->launches++;
     return COMIC_OK;
@@ -1299,6 +1517,7 @@ extern "C" int comic_rnn_init(comic_handle_t h, const float* im_embed, int B, fl
   APlain a2{};
   a2.nseg = 1;
   a2.seg[0] = ASeg{x0, nullptr, XA, XA, B};
+  if (h->cell == COMIC_CELL_GRU) return gru_init_step(h, x0, B, gates, gates + (size_t)B * 3 * R * 16, h0, nullptr, st);
   GemmPlan p2 = plan_gemm(B, 4 * R, XA, h->num_sms, true);
   int nz = gemm_num_partials(XA, p2);
   Epi e2{};
@@ -1321,7 +1540,7 @@ extern "C" int comic_decode_step(comic_handle_t h, const float* keys, const floa
                                  const float* in_mask, const float* out_mask, const float* att_mask, float in_keep,
                                  float out_keep, float att_keep, void* ws, size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && h->bound, COMIC_E_BADARG, "decode_step: weights not bound");
-  COMIC_REQUIRE(keys && tokens && c_in && h_in && ctx_in && c_out && h_out && ctx_out, COMIC_E_BADARG,
+  COMIC_REQUIRE(keys && tokens && h_in && ctx_in && h_out && ctx_out && (h->cell == COMIC_CELL_GRU || (c_in && c_out)), COMIC_E_BADARG,
                 "decode_step: null argument");
   COMIC_REQUIRE(B > 0 && k > 0 && k <= 16, COMIC_E_SHAPE, "decode_step: bad B=%d k=%d", B, k);
   cudaStream_t st = (cudaStream_t)stream;
@@ -1361,7 +1580,7 @@ extern "C" int comic_decode_greedy(comic_handle_t h, const float* keys, const fl
                                    const float* h0, int B, int max_it, int32_t* ids_out, float* logits_out,
                                    float* attn_out, int32_t* T_out, void* ws, size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && h->bound, COMIC_E_BADARG, "decode_greedy: weights not bound");
-  COMIC_REQUIRE(keys && c0 && h0 && ids_out && T_out, COMIC_E_BADARG, "decode_greedy: null argument");
+  COMIC_REQUIRE(keys && (c0 || h->cell == COMIC_CELL_GRU) && h0 && ids_out && T_out, COMIC_E_BADARG, "decode_greedy: null argument");
   COMIC_REQUIRE(B > 0 && max_it >= 0, COMIC_E_SHAPE, "decode_greedy: bad B=%d max_it=%d", B, max_it);
   cudaStream_t st = (cudaStream_t)stream;
   size_t need;
@@ -1436,7 +1655,7 @@ extern "C" int comic_decode_beam(comic_handle_t h, const float* keys, const floa
                                  int64_t* lengths_out, float* attn_top_out, int32_t* T_out, void* ws,
                                  size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && h->bound, COMIC_E_BADARG, "decode_beam: weights not bound");
-  COMIC_REQUIRE(keys && c0 && h0 && pred_ids_out && T_out, COMIC_E_BADARG, "decode_beam: null argument");
+  COMIC_REQUIRE(keys && (c0 || h->cell == COMIC_CELL_GRU) && h0 && pred_ids_out && T_out, COMIC_E_BADARG, "decode_beam: null argument");
   COMIC_REQUIRE(B > 0 && k > 0 && k <= 16 && max_it >= 0, COMIC_E_SHAPE, "decode_beam: bad B=%d k=%d max_it=%d", B, k, max_it);
   COMIC_REQUIRE(k <= h->V, COMIC_E_SHAPE, "decode_beam: beam %d exceeds vocab %d", k, h->V);
   cudaStream_t st = (cudaStream_t)stream;

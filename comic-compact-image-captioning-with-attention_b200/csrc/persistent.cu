@@ -668,6 +668,7 @@ static PersistPlan persist_plan(comic_handle_t h, int B, int k, bool greedy) {
   PersistPlan p;
   const int N = B * k, R = h->R, M = h->M, VAL = h->VAL, H = h->H;
   if (h->persist_max_rows <= 0 || N > h->persist_max_rows || N > 8 * kPMaxRPL) return p;
+  if (h->cell != COMIC_CELL_LSTM) return p;   // the loop's phase A is the LSTM cell; GRU decodes take the per-step path
   if (R != 512 || h->cfg.alignment != 0 || h->cfg.context_layer || k > 16) return p;
   if (!(H == 1 || H == 2 || H == 4 || H == 8 || H == 16) || VAL % (4 * H) != 0 || h->KX % 4 != 0 || h->W % 4 != 0 ||
       h->A % 4 != 0 || h->LQ % 4 != 0 || h->Vp % 4 != 0 || h->A != VAL)

@@ -667,6 +667,53 @@ __global__ void lstm_bwd_kernel(const float* __restrict__ gates, const float* __
   gH_pass[i] = fin ? gh : 0.f;
 }
 
+// GRU cell backward (TF r1.9 GRUCell; tape row [r | u | r*h | c], gradient row dG = [dR | dU | dC | dh'] of the r / u / candidate
+// pre-activations, the last quarter a scratch copy of dh').
+// Part a: dh' = dHout (split-K partials, output dropout) + (fin ? 0 : gH);  dC = dh' (1 - u)(1 - c^2).
+__global__ void gru_bwd_a_kernel(const float* __restrict__ tape, const float* __restrict__ dhout, const float* __restrict__ out_mask,
+                                 float out_keep, const int* __restrict__ lens, int t, const float* __restrict__ gH,
+                                 float* __restrict__ dgates, int B, int R, int nz = 1, size_t zstride = 0) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B * R) return;
+  int b = i / R, j = i - b * R;
+  const bool fin = lens && t >= lens[b];
+  float dh = dhout ? dhout[i] : 0.f;
+  for (int z = 1; z < nz; ++z) dh += dhout[z * zstride + i];      // split-K partials of the producing GEMM, fixed order
+  if (out_mask) dh = (dh / out_keep) * out_mask[i];
+  if (!fin) dh += gH[i];
+  const float* tr = tape + (size_t)b * 4 * R;
+  const float u = tr[R + j], c = tr[3 * R + j];
+  float* dg = dgates + (size_t)b * 4 * R;
+  dg[2 * R + j] = dh * (1.0f - u) * (1.0f - c * c);
+  dg[3 * R + j] = dh;
+}
+
+// Part b, after d(r*h) = dC . candidate/kernel[h rows]^T (split-K partials drh; NULL = zero, the init step):
+//   dR = d(rh) h r (1 - r),  dU = dh' (h - c) u (1 - u);
+//   gH_pass = dh' u + d(rh) r + (fin ? gH : 0): what reaches h_prev outside the [x, h] . gates/kernel product (dx_split adds
+//   that product's share).  h_prev: the state the step read (NULL = zero).
+__global__ void gru_bwd_b_kernel(const float* __restrict__ tape, const float* __restrict__ h_prev, const float* __restrict__ drh, int nz,
+                                 size_t zstride, const int* __restrict__ lens, int t, const float* __restrict__ gH,
+                                 float* __restrict__ gH_pass, float* __restrict__ dgates, int B, int R) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B * R) return;
+  int b = i / R, j = i - b * R;
+  const bool fin = lens && t >= lens[b];
+  const float* tr = tape + (size_t)b * 4 * R;
+  const float r = tr[j], u = tr[R + j], c = tr[3 * R + j];
+  const float hp = h_prev ? h_prev[i] : 0.f;
+  float d = 0.f;
+  if (drh) {
+    d = drh[i];
+    for (int z = 1; z < nz; ++z) d += drh[z * zstride + i];
+  }
+  float* dg = dgates + (size_t)b * 4 * R;
+  const float dh = dg[3 * R + j];
+  dg[j] = d * hp * r * (1.0f - r);
+  dg[R + j] = dh * (hp - c) * u * (1.0f - u);
+  gH_pass[i] = dh * u + d * r + (fin ? gH[i] : 0.f);
+}
+
 // dxh [B, KX] -> demb [B, W], gCtx [B, A], gH [B, R] (input dropout backward + pass-through of finished rows)
 __global__ void dx_split_kernel(const float* __restrict__ dxh, int KX, int W, int A, int R,
                                 const float* __restrict__ in_mask, float in_keep, const int* __restrict__ lens, int t,
@@ -704,6 +751,17 @@ __global__ void build_xh_kernel(const float* __restrict__ xd, const float* __res
   if (j < XA) v = xd[r * XA + j];
   else v = (r < (size_t)B) ? 0.f : hst[(r - B) * R + (j - XA)];   // state after step t-1 = h[t] slot (0 = init)
   xh[i] = v;
+}
+
+// GRU candidate-kernel rows: block 0 = [x0 ; 0], block 1+t = [x_t ; r_t * h_{t-1}] (r*h from the tape, zero at the init step).
+__global__ void build_xrh_kernel(const float* __restrict__ xd, const float* __restrict__ tape, int XA, int R,
+                                 float* __restrict__ xh, size_t rows) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int KX = XA + R;
+  if (i >= rows * KX) return;
+  size_t r = i / KX;
+  int j = (int)(i % KX);
+  xh[i] = (j < XA) ? xd[r * XA + j] : tape[r * 4 * R + 2 * R + (j - XA)];
 }
 
 // Deterministic embedding gradient: dE[id, :] = sum over rows with ids[row] == id.
@@ -909,7 +967,7 @@ struct TrainBufs {
   // backward
   float *dlq, *dG, *demb, *gH, *gC, *gCtx, *gHp, *dHout, *dxh, *ds, *dqpart, *cpart, *dTacc, *maprows, *rowloss;
   float *dkeys, *dvals, *keys, *vals, *dx0;
-  float *KT, *outqT, *xh, *xhT, *hdT, *fmT, *embT, *dOutQ, *part, *scal;
+  float *KT, *KcT, *outqT, *xh, *xhT, *hdT, *fmT, *embT, *dOutQ, *part, *scal;
   float *encT, *dfm_tmp;   // cnn_finetune: transposed W_k / W_v / W_I, second dfm term (independent)
   // variants: raw scores per step (signorm), context-layer input / masked output gradient per step, a_layer^T
   float *stape, *ctxraw, *gctx_tape, *dctxraw, *aT, *ctxrawT;
@@ -963,7 +1021,8 @@ static void carve_train(comic_handle_t h, Carver& cv, int B, int T_run, TrainBuf
   tb.keys = cv.take<float>((size_t)B * h->M * R);
   tb.vals = cv.take<float>(h->cfg.fm_projection == 2 ? (size_t)B * h->M * R : 1);
   tb.dx0 = cv.take<float>((size_t)((B + 3) / 4 * 4) * XA);
-  tb.KT = cv.take<float>((size_t)4 * R * KX);
+  tb.KT = cv.take<float>((size_t)4 * R * KX);                 // GRU: [3R, KX] transpose of the gate panel
+  tb.KcT = (h->cell == COMIC_CELL_GRU) ? cv.take<float>((size_t)R * R) : nullptr;
   tb.outqT = cv.take<float>((size_t)LQ * R);
   tb.xh = cv.take<float>((size_t)tb.rows_pad * KX);
   tb.xhT = cv.take<float>((size_t)KX * tb.rows_pad);
@@ -1003,6 +1062,7 @@ using namespace comic;
 
 extern "C" int comic_train_workspace_bytes(comic_handle_t h, int B, int T_run, size_t* bytes) {
   COMIC_REQUIRE(h && bytes && B > 0 && T_run >= 0, COMIC_E_BADARG, "train_workspace_bytes: bad argument");
+  h->sized = true;
   return train_workspace_bytes(h, B, T_run, bytes);
 }
 
@@ -1023,6 +1083,8 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
                                    float map_loss_scale, float* loss_out, float* logits_out, float* attn_out,
                                    const comic_decoder_grads_t* grads, void* ws, size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && h->bound, COMIC_E_BADARG, "train_fwd_bwd: weights not bound");
+  COMIC_REQUIRE(h->cell == COMIC_CELL_LSTM || !grads || (grads->cand_kernel && grads->cand_bias), COMIC_E_BADARG,
+                "train_fwd_bwd: GRU cell needs the candidate/{kernel, bias} gradient buffers");
   COMIC_REQUIRE(fm && im_embed && inputs_tm && targets_tm && coef_tm && lens && loss_out, COMIC_E_BADARG,
                 "train_fwd_bwd: null argument");   // grads == NULL: forward only (evaluation perplexity)
   COMIC_REQUIRE(B > 0 && T > 0 && T_run > 0 && T_run <= T, COMIC_E_SHAPE, "train_fwd_bwd: bad B=%d T=%d T_run=%d", B, T, T_run);
@@ -1041,7 +1103,9 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
   const comic_train_masks_t mk = masks ? *masks : comic_train_masks_t{};
   const float in_keep = masks ? mk.in_keep : 1.f, out_keep = masks ? mk.out_keep : 1.f, att_keep = masks ? mk.att_keep : 1.f;
   const size_t T1 = (size_t)T_run + 1;
+  const bool gru = h->cell == COMIC_CELL_GRU;   // tape row [r | u | r*h | c] in place of the LSTM's 4R gate pre-activations
   int rc;
+  if (gru) COMIC_CHECK_CUDA(cudaMemsetAsync(tb.c, 0, T1 * B * R * sizeof(float), st));   // no c state: the imputation copies zeros
 
   // ---- keys / values: D0 (ops_rnn.py:441-477) ----
   float* keys_buf = tb.keys;
@@ -1082,22 +1146,27 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
       size_t nx = (size_t)B * XA;
       mask_scale_kernel<<<(unsigned)((nx + 255) / 256), 256, 0, st>>>(tb.xd, mk.init_in, in_keep, nx);
     }
-    APlain a2{};
-    a2.nseg = 1;
-    a2.seg[0] = ASeg{tb.xd, nullptr, XA, XA, B};
-    GemmPlan p2 = plan_gemm(B, 4 * R, XA, h->num_sms, true);
-    int nz = gemm_num_partials(XA, p2);
-    Epi e2{};
-    e2.nroute = 1;
-    e2.stop_n = 0x7fffffff;
-    e2.r[0] = Route{0, 4 * R, tb.sb.gates, 4 * R, 0};
-    e2.split_stride = (long long)B * 4 * R;
-    COMIC_CHECK_CUDA((launch_gemm<0, 4>(a2, h->w.lstm_kernel, 4 * R, B, 4 * R, XA, e2, p2, st)));
-    int tot = B * R;
-    lstm_init_fwd_kernel<<<(tot + 255) / 256, 256, 0, st>>>(tb.sb.gates, nz, (size_t)B * 4 * R, h->w.lstm_bias, tb.gates,
-                                                          tb.c, tb.h, B, R);
+    if (gru) {
+      if ((rc = gru_init_step(h, tb.xd, B, tb.part, tb.sb.gru, tb.h, tb.gates, st))) return rc;
+    } else {
+      APlain a2{};
+      a2.nseg = 1;
+      a2.seg[0] = ASeg{tb.xd, nullptr, XA, XA, B};
+      GemmPlan p2 = plan_gemm(B, 4 * R, XA, h->num_sms, true);
+      int nz = gemm_num_partials(XA, p2);
+      Epi e2{};
+      e2.nroute = 1;
+      e2.stop_n = 0x7fffffff;
+      e2.r[0] = Route{0, 4 * R, tb.sb.gates, 4 * R, 0};
+      e2.split_stride = (long long)B * 4 * R;
+      COMIC_CHECK_CUDA((launch_gemm<0, 4>(a2, h->w.lstm_kernel, 4 * R, B, 4 * R, XA, e2, p2, st)));
+      int tot = B * R;
+      lstm_init_fwd_kernel<<<(tot + 255) / 256, 256, 0, st>>>(tb.sb.gates, nz, (size_t)B * 4 * R, h->w.lstm_bias, tb.gates,
+                                                            tb.c, tb.h, B, R);
+      h->launches += 2;
+    }
     COMIC_CHECK_CUDA(cudaMemsetAsync(tb.ctx, 0, (size_t)B * A * sizeof(float), st));
-    h->launches += 4;
+    h->launches += 2;
   }
 
   // ---- forward over T_run steps ----
@@ -1152,7 +1221,13 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
   }
 
   // ---- transposed weights for the per-step backward GEMMs ----
-  transpose(h->w.lstm_kernel, KX, 4 * R, 4 * R, tb.KT, KX, st);
+  if (gru) {
+    transpose(h->pk.gru_gx, KX, 3 * R, 3 * R, tb.KT, KX, st);                           // [gates | cand x-rows ; 0]^T [3R, KX]
+    transpose(h->gru_cand_kernel + (size_t)XA * R, R, R, R, tb.KcT, R, st);              // candidate h-rows^T
+    h->launches++;
+  } else {
+    transpose(h->w.lstm_kernel, KX, 4 * R, 4 * R, tb.KT, KX, st);
+  }
   transpose(h->pk.outq, R, LQ, LQ, tb.outqT, R, st);
   COMIC_CHECK_CUDA(cudaMemsetAsync(tb.gH, 0, (size_t)B * R * sizeof(float), st));
   COMIC_CHECK_CUDA(cudaMemsetAsync(tb.gC, 0, (size_t)B * R * sizeof(float), st));
@@ -1235,10 +1310,24 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
     int nzh = 1, nzx = 1;
     if ((rc = train_gemm(h, dlq_t, LQ, tb.outqT, R, tb.dHout, R, B, R, LQ, tb.part, tb.part_floats, st, &nzh))) return rc;
     float* dG_t = tb.dG + (size_t)(t + 1) * B * 4 * R;
-    lstm_bwd_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tb.gates + (size_t)(t + 1) * B * 4 * R, tb.c + (size_t)t * B * R,
-                                                        nzh > 1 ? tb.part : tb.dHout, mk.out ? mk.out + (size_t)t * B * R : nullptr,
-                                                        out_keep, lens, t, tb.gH, tb.gC, tb.gHp, dG_t, B, R, nzh, (size_t)B * R);
-    if ((rc = train_gemm(h, dG_t, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 4 * R, tb.part, tb.part_floats, st, &nzx))) return rc;
+    const float* tape_t = tb.gates + (size_t)(t + 1) * B * 4 * R;
+    if (gru) {
+      gru_bwd_a_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tape_t, nzh > 1 ? tb.part : tb.dHout,
+                                                           mk.out ? mk.out + (size_t)t * B * R : nullptr, out_keep, lens, t, tb.gH,
+                                                           dG_t, B, R, nzh, (size_t)B * R);
+      int nzr = 1;   // d(r*h) = dC . Kc_h^T
+      if ((rc = train_gemm(h, dG_t + 2 * R, 4 * R, tb.KcT, R, tb.dHout, R, B, R, R, tb.part, tb.part_floats, st, &nzr))) return rc;
+      gru_bwd_b_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tape_t, tb.h + (size_t)t * B * R, nzr > 1 ? tb.part : tb.dHout, nzr,
+                                                           (size_t)B * R, lens, t, tb.gH, tb.gHp, dG_t, B, R);
+      h->launches += 2;
+      // d[x, h] = [dR | dU | dC] . [gates | cand x-rows ; 0]^T
+      if ((rc = train_gemm(h, dG_t, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 3 * R, tb.part, tb.part_floats, st, &nzx))) return rc;
+    } else {
+      lstm_bwd_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tape_t, tb.c + (size_t)t * B * R,
+                                                          nzh > 1 ? tb.part : tb.dHout, mk.out ? mk.out + (size_t)t * B * R : nullptr,
+                                                          out_keep, lens, t, tb.gH, tb.gC, tb.gHp, dG_t, B, R, nzh, (size_t)B * R);
+      if ((rc = train_gemm(h, dG_t, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 4 * R, tb.part, tb.part_floats, st, &nzx))) return rc;
+    }
     dx_split_kernel<<<(unsigned)(((size_t)B * KX + 255) / 256), 256, 0, st>>>(
         nzx > 1 ? tb.part : tb.dxh, KX, W, A, R, mk.inp ? mk.inp + (size_t)t * B * XA : nullptr, in_keep, lens, t,
         tb.demb + (size_t)t * B * W, tb.gCtx, tb.gH, tb.gHp, B, nzx, (size_t)B * KX);
@@ -1253,9 +1342,16 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
     copy2d_kernel<<<(unsigned)(((size_t)B * R + 255) / 256), 256, 0, st>>>(tb.gH, R, dx0, R, B, R);
     h->launches += 1;
   } else {
-    lstm_bwd_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tb.gates, nullptr, nullptr, nullptr, 1.f, nullptr, 0, tb.gH, tb.gC,
-                                                        tb.gHp, tb.dG, B, R);
-    if ((rc = train_gemm(h, tb.dG, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 4 * R, tb.part, tb.part_floats, st))) return rc;
+    if (gru) {
+      gru_bwd_a_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tb.gates, nullptr, nullptr, 1.f, nullptr, 0, tb.gH, tb.dG, B, R);
+      gru_bwd_b_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tb.gates, nullptr, nullptr, 0, 0, nullptr, 0, tb.gH, tb.gHp, tb.dG, B, R);
+      h->launches++;
+      if ((rc = train_gemm(h, tb.dG, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 3 * R, tb.part, tb.part_floats, st))) return rc;
+    } else {
+      lstm_bwd_kernel<<<(B * R + 255) / 256, 256, 0, st>>>(tb.gates, nullptr, nullptr, nullptr, 1.f, nullptr, 0, tb.gH, tb.gC,
+                                                          tb.gHp, tb.dG, B, R);
+      if ((rc = train_gemm(h, tb.dG, 4 * R, tb.KT, KX, tb.dxh, KX, B, KX, 4 * R, tb.part, tb.part_floats, st))) return rc;
+    }
     // dx0 = dxh[:, :XA] * init mask / keep
     copy2d_kernel<<<(unsigned)(((size_t)B * XA + 255) / 256), 256, 0, st>>>(tb.dxh, KX, dx0, XA, B, XA);
     if (mk.init_in) {
@@ -1281,9 +1377,23 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
     build_xh_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(tb.xd, tb.h, XA, R, tb.xh, rows, B);
   }
   transpose(tb.xh, rows, KX, KX, tb.xhT, rows_pad, st);
-  if ((rc = train_gemm(h, tb.xhT, rows_pad, tb.dG, 4 * R, grads->lstm_kernel, 4 * R, KX, 4 * R, rows_pad, tb.part,
-                       tb.part_floats, st))) return rc;
-  colsum_kernel<<<(4 * R + 31) / 32, 256, 0, st>>>(tb.dG, rows, 4 * R, 4 * R, grads->lstm_bias, 0);
+  if (gru) {
+    // d gates/kernel = [x, h_prev]^T . [dR | dU];  d candidate/kernel = [x, r*h]^T . dC  (one GEMM each over all rows)
+    if ((rc = train_gemm(h, tb.xhT, rows_pad, tb.dG, 4 * R, grads->lstm_kernel, 2 * R, KX, 2 * R, rows_pad, tb.part,
+                         tb.part_floats, st))) return rc;
+    colsum_kernel<<<(2 * R + 31) / 32, 256, 0, st>>>(tb.dG, rows, 2 * R, 4 * R, grads->lstm_bias, 0);
+    size_t n = (size_t)rows * KX;
+    build_xrh_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(tb.xd, tb.gates, XA, R, tb.xh, rows);
+    transpose(tb.xh, rows, KX, KX, tb.xhT, rows_pad, st);
+    if ((rc = train_gemm(h, tb.xhT, rows_pad, tb.dG + 2 * R, 4 * R, grads->cand_kernel, R, KX, R, rows_pad, tb.part,
+                         tb.part_floats, st))) return rc;
+    colsum_kernel<<<(R + 31) / 32, 256, 0, st>>>(tb.dG + 2 * R, rows, R, 4 * R, grads->cand_bias, 0);
+    h->launches += 3;
+  } else {
+    if ((rc = train_gemm(h, tb.xhT, rows_pad, tb.dG, 4 * R, grads->lstm_kernel, 4 * R, KX, 4 * R, rows_pad, tb.part,
+                         tb.part_floats, st))) return rc;
+    colsum_kernel<<<(4 * R + 31) / 32, 256, 0, st>>>(tb.dG, rows, 4 * R, 4 * R, grads->lstm_bias, 0);
+  }
   // d[W_o | W_q] = Hout^T . dLQ
   COMIC_CHECK_CUDA(cudaMemsetAsync(tb.hdT, 0, (size_t)R * rows_pad * sizeof(float), st));
   transpose(tb.hdrop, rows_t, R, R, tb.hdT, rows_pad, st);

@@ -22,6 +22,7 @@ FM_PROJ = {None: 0, 'none': 0, 'tied': 1, 'independent': 2}
 ALIGN = {'add_LN': 0, 'dot': 1}
 PROB = {'softmax': 0, 'sigmoid': 1}
 INIT = {'first_input': 0, 'project_hidden': 1}
+CELL = {'LSTM': 0, 'GRU': 1}                   # COMIC_CELL_*
 
 
 class ComicCfg(C.Structure):
@@ -49,7 +50,8 @@ class ComicTrainMasks(C.Structure):
 
 
 GRAD_FIELDS = ('lstm_kernel', 'lstm_bias', 'init_weight', 'memory_kernel', 'value_kernel', 'query_kernel',
-               'attention_v', 'ln_gamma', 'ln_beta', 'temperature', 'out_kernel', 'out_bias', 'embedding_map', 'a_layer')
+               'attention_v', 'ln_gamma', 'ln_beta', 'temperature', 'out_kernel', 'out_bias', 'embedding_map', 'a_layer',
+               'cand_kernel', 'cand_bias')
 
 
 class ComicDecoderGrads(C.Structure):
@@ -80,6 +82,8 @@ SIGNATURES = {
     'comic_destroy': (_I, [_P]),
     'comic_packed_bytes': (_I, [_P, C.POINTER(_SZ)]),
     'comic_bind_weights': (_I, [_P, C.POINTER(ComicWeights), _I, _P, _SZ, _P]),
+    'comic_set_rnn_cell': (_I, [_P, _I]),
+    'comic_bind_gru_candidate': (_I, [_P, _P, _P]),
     'comic_workspace_bytes': (_I, [_P, _I, _I, _I, _I, C.POINTER(_SZ)]),
     'comic_encode_fwd': (_I, [_P, _P, _I, _P, _P, _P, _P, _SZ, _P]),
     'comic_preprocess_eval': (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P]),
@@ -166,8 +170,9 @@ class Engine(object):
         torch.cuda.set_device(self.device)
         self.c = config
         d = self.dims = wts.Dims(config)
-        if config.rnn_name != 'LSTM':
-            raise ComicError('rnn_name=%s is not built (LSTM only)' % config.rnn_name)
+        if config.rnn_name not in CELL:
+            raise ComicError('rnn_name=%s is not built (LSTM and GRU are)' % config.rnn_name)
+        self.gru = config.rnn_name == 'GRU'
         if config.attn_alignment_method not in ALIGN:
             raise ValueError('Invalid alignment method.')             # src/model_base.py:133-138
         if config.attn_probability_fn not in PROB:
@@ -186,6 +191,7 @@ class Engine(object):
             go_id=self.go, eos_id=self.eos)
         self._h = C.c_void_p()
         self._check(self.lib.comic_create(C.byref(cfg), C.byref(self._h)))
+        self._check(self.lib.comic_set_rnn_cell(self._h, CELL[config.rnn_name]))
         self._dev_weights = {}
         self._packed = None
         self._ws = {}
@@ -255,8 +261,13 @@ class Engine(object):
             t = dev.get(name)
             return None if t is None else C.c_void_p(t.data_ptr())
         w = ComicWeights()
-        w.lstm_kernel = g(cs + 'kernel')
-        w.lstm_bias = g(cs + 'bias')
+        if self.gru:     # gates/{kernel, bias} travel in the LSTM fields; the candidate is bound by pointer beside them
+            w.lstm_kernel = g(cs + 'gates/kernel')
+            w.lstm_bias = g(cs + 'gates/bias')
+            self._check(self.lib.comic_bind_gru_candidate(self._h, g(cs + 'candidate/kernel'), g(cs + 'candidate/bias')))
+        else:
+            w.lstm_kernel = g(cs + 'kernel')
+            w.lstm_bias = g(cs + 'bias')
         w.init_weight = g(D + ('rnn_init_input/projection/weight' if c.rnn_init_method == 'first_input'
                                else 'rnn_initial_state/weight'))
         w.memory_kernel = g(D + 'memory_layer/kernel')
@@ -355,8 +366,9 @@ class Engine(object):
 
     # -- D1 -------------------------------------------------------------------
     def rnn_init(self, im_embed, in_mask=None, in_keep=1.0):
+        """-> (c0, h0) [B, R]; c0 is None for the GRU cell (its state is h only)."""
         B = im_embed.shape[0]
-        c0, h0 = self.f32(B, self.dims.R), self.f32(B, self.dims.R)
+        c0, h0 = (None if self.gru else self.f32(B, self.dims.R)), self.f32(B, self.dims.R)
         ws = self._workspace(4, B, 1, 1)
         self._check(self.lib.comic_rnn_init(self._h, _ptr(im_embed.contiguous()), B, _ptr(c0), _ptr(h0),
                                             _ptr(in_mask), float(in_keep), _ptr(ws), ws.numel(), self.stream()))
@@ -367,7 +379,7 @@ class Engine(object):
                     att_mask=None, keeps=(1.0, 1.0, 1.0)):
         d = self.dims
         N = B * k
-        c_out, h_out = self.f32(N, d.R), self.f32(N, d.R)
+        c_out, h_out = (None if self.gru else self.f32(N, d.R)), self.f32(N, d.R)
         ctx_out = self.f32(N, d.A)
         align = self.f32(N, d.H * d.M)
         logits = self.f32(N, d.V)
@@ -384,7 +396,7 @@ class Engine(object):
     def decode_greedy(self, keys, values, c0, h0, max_it, want_logits=True, want_attn=True):
         torch = self.torch
         d = self.dims
-        B = c0.shape[0]
+        B = h0.shape[0]
         ids = torch.empty((max(max_it, 1), B), dtype=torch.int32, device=self.device)
         logits = self.f32(max(max_it, 1), B, d.V) if want_logits else None
         attn = self.f32(B, d.H, max(max_it, 1), d.M) if want_attn else None
@@ -400,7 +412,7 @@ class Engine(object):
     def decode_beam(self, keys, values, c0, h0, beam, lpw, max_it, want_attn=True):
         torch = self.torch
         d = self.dims
-        B = c0.shape[0]
+        B = h0.shape[0]
         Tm = max(max_it, 1)
         i32 = dict(dtype=torch.int32, device=self.device)
         pred = torch.empty((Tm, B, beam), **i32)
@@ -531,14 +543,19 @@ class Engine(object):
         D = wts.DEC
         att = D + 'multi_add_attention/'
         cs = wts.cell_scope(c)
-        m = {cs + 'kernel': 'lstm_kernel', cs + 'bias': 'lstm_bias',
-             D + 'rnn_init_input/projection/weight': 'init_weight', D + 'rnn_initial_state/weight': 'init_weight',
+        if self.gru:     # gates/{kernel, bias} travel in the LSTM fields, as at binding
+            cell = {cs + 'gates/kernel': 'lstm_kernel', cs + 'gates/bias': 'lstm_bias',
+                    cs + 'candidate/kernel': 'cand_kernel', cs + 'candidate/bias': 'cand_bias'}
+        else:
+            cell = {cs + 'kernel': 'lstm_kernel', cs + 'bias': 'lstm_bias'}
+        m = {D + 'rnn_init_input/projection/weight': 'init_weight', D + 'rnn_initial_state/weight': 'init_weight',
              D + 'memory_layer/kernel': 'memory_kernel', D + 'value_layer/kernel': 'value_kernel',
              att + 'query_layer/kernel': 'query_kernel', att + 'attention_v': 'attention_v',
              att + 'LN_tanh/gamma': 'ln_gamma', att + 'LN_tanh/beta': 'ln_beta',
              D + 'softmax_temperature': 'temperature', D + 'output_projection/kernel': 'out_kernel',
              D + 'output_projection/bias': 'out_bias', D + 'embedding_map': 'embedding_map',
              D + 'a_layer/kernel': 'a_layer'}
+        m.update(cell)
         return m
 
     def dropout_masks(self, shape, keep, seed, stream_id):

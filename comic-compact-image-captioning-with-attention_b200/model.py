@@ -94,7 +94,8 @@ class ModelBase(object):
         batch_size = self.im_embed.shape[0]
         is_inference = self.mode == 'infer'
         beam_search = is_inference and c.infer_beam_size > 1
-        rnn_init = rops.LSTMStateTuple(*eng.rnn_init(self.im_embed))          # _get_rnn_init :651-689
+        c0, h0 = eng.rnn_init(self.im_embed)                                   # _get_rnn_init :651-689
+        rnn_init = h0 if c.rnn_name == 'GRU' else rops.LSTMStateTuple(c0, h0)   # GRUCell state: the h tensor
         cnn_attention = att_mech(c.rnn_size, self.cnn_fmaps, c.cnn_fm_projection, c.attn_num_heads,
                                  memory_sequence_length=None, probability_fn=c.attn_probability_fn,
                                  engine=eng)

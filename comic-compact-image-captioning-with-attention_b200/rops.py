@@ -72,7 +72,8 @@ class MultiHeadDot(MultiHeadAttV3):
 
 class MultiHeadAttentionWrapperV3(object):
     """common/ops_rnn.py:635-803.  `cell` is the (name of the) inner RNN cell;
-    `initial_cell_state` an LSTMStateTuple of per-image [B, R] tensors."""
+    `initial_cell_state` an LSTMStateTuple of per-image [B, R] tensors (LSTM) or
+    the [B, R] h tensor (GRU: TF's GRUCell state is a tensor, not a tuple)."""
 
     def __init__(self, deep_output_layer=False, context_layer=True, alignments_keep_prob=1.0,
                  cell='LSTM', attention_mechanism=None, attention_layer_size=None,
@@ -80,12 +81,14 @@ class MultiHeadAttentionWrapperV3(object):
                  initial_cell_state=None, name=None):
         if attention_mechanism is None or isinstance(attention_mechanism, (list, tuple)):
             raise ValueError('Only a single attention mechanism can be used.')   # ops_rnn.py:656-657
-        if cell != 'LSTM':
-            raise NotImplementedError('Only `LSTM` is built on the CUDA path.')
+        if cell not in ('LSTM', 'GRU'):
+            raise NotImplementedError('Only `LSTM` and `GRU` are built on the CUDA path.')
         if attention_layer_size is not None or cell_input_fn is not None or output_attention:
             raise NotImplementedError('the reference always passes attention_layer_size=None, '
                                       'cell_input_fn=None, output_attention=False (src/model_base.py:157-167)')
         eng = attention_mechanism._engine
+        if (cell == 'GRU') != eng.gru:
+            raise ValueError('cell %s does not match the engine configuration' % cell)
         if bool(context_layer) != eng.dims.context_layer:
             raise ValueError('context_layer does not match the engine configuration')
         self._attention_mechanism = attention_mechanism
@@ -119,12 +122,20 @@ class MultiHeadAttentionWrapperV3(object):
         N = inputs_ids.shape[0]
         B = N // beam
         m = masks or {}
-        r = eng.decode_step(am.keys, am.values, B, beam, inputs_ids, state.cell_state.c, state.cell_state.h,
+        c_in, h_in = _split_cell_state(eng, state.cell_state)
+        r = eng.decode_step(am.keys, am.values, B, beam, inputs_ids, c_in, h_in,
                             state.attention, m.get('inp'), m.get('out'), m.get('att'), keeps)
         new_state = AttentionWrapperState(
-            cell_state=LSTMStateTuple(r['c'], r['h']), attention=r['attention'], time=state.time + 1,
+            cell_state=r['h'] if eng.gru else LSTMStateTuple(r['c'], r['h']), attention=r['attention'], time=state.time + 1,
             alignments=r['alignments'], alignment_history=(), attention_state=r['alignments'])
         return r['h'], r['logits'], new_state
+
+
+def _split_cell_state(eng, cell_state):
+    """(c, h) of a wrapper's cell state; c is None for the GRU cell, whose state is the h tensor itself."""
+    if eng.gru:
+        return None, cell_state
+    return cell_state.c, cell_state.h
 
 
 def _check_ids(cell, start_id, end_id):
@@ -151,7 +162,7 @@ def rnn_decoder_beam_search(cell, embedding_fn, output_layer, batch_size, beam_s
     if am.batch_size != batch_size:
         raise ValueError('Non-matching batch sizes between the memory (encoder output) and the query '
                          '(decoder output).')                           # ops_rnn.py:679-690
-    c0, h0 = cell._initial_cell_state
+    c0, h0 = _split_cell_state(eng, cell._initial_cell_state)
     want_attn = getattr(cell, '_alignment_history', True)
     r = eng.decode_beam(am.keys, am.values, c0, h0, int(beam_size), float(length_penalty_weight),
                         int(maximum_iterations), want_attn=want_attn)
@@ -186,7 +197,7 @@ def rnn_decoder_search(cell, embedding_fn, output_layer, batch_size, maximum_ite
     if am.batch_size != batch_size:
         raise ValueError('Non-matching batch sizes between the memory (encoder output) and the query '
                          '(decoder output).')
-    c0, h0 = cell._initial_cell_state
+    c0, h0 = _split_cell_state(eng, cell._initial_cell_state)
     want_attn = getattr(cell, '_alignment_history', True)
     r = eng.decode_greedy(am.keys, am.values, c0, h0, int(maximum_iterations), want_attn=want_attn)
     if getattr(cell, '_defer_T', False):             # see rnn_decoder_beam_search

@@ -116,13 +116,18 @@ def decoder_shapes(c):
     d = Dims(c)
     sh = {}
     if d.init_method == 'first_input':
-        cell_scope = DEC + 'rnn_init_input/basic_lstm_cell/'
         sh[DEC + 'rnn_init_input/projection/weight'] = (d.E, d.W + d.A)
     else:
-        cell_scope = DEC + 'basic_lstm_cell/'
         sh[DEC + 'rnn_initial_state/weight'] = (d.E, d.R)
-    sh[cell_scope + 'kernel'] = (d.W + d.A + d.R, 4 * d.R)
-    sh[cell_scope + 'bias'] = (4 * d.R,)
+    cs = cell_scope(c)
+    if c.rnn_name == 'GRU':                      # TF r1.9 GRUCell: gates [r, u], candidate
+        sh[cs + 'gates/kernel'] = (d.W + d.A + d.R, 2 * d.R)
+        sh[cs + 'gates/bias'] = (2 * d.R,)
+        sh[cs + 'candidate/kernel'] = (d.W + d.A + d.R, d.R)
+        sh[cs + 'candidate/bias'] = (d.R,)
+    else:
+        sh[cs + 'kernel'] = (d.W + d.A + d.R, 4 * d.R)
+        sh[cs + 'bias'] = (4 * d.R,)
     sh[DEC + 'memory_layer/kernel'] = (d.C, d.R)
     if d.fm_projection == 'independent':
         sh[DEC + 'value_layer/kernel'] = (d.C, d.R)
@@ -152,8 +157,10 @@ def encoder_head_shapes(c):
 
 
 def cell_scope(c):
-    return (DEC + 'rnn_init_input/basic_lstm_cell/'
-            if c.rnn_init_method == 'first_input' else DEC + 'basic_lstm_cell/')
+    """Variable scope of the decoder cell (src/model_base.py:622-629): `basic_lstm_cell` (LSTM) or `gru_cell` (GRU),
+    under `rnn_init_input/` when the first_input init step created it."""
+    cell = 'gru_cell/' if c.rnn_name == 'GRU' else 'basic_lstm_cell/'
+    return DEC + ('rnn_init_input/' if c.rnn_init_method == 'first_input' else '') + cell
 
 
 def cnn_shapes():
@@ -199,8 +206,10 @@ def init_weights(c, seed=48964896, cnn_init='he', include_cnn=True):
     shapes = dict(decoder_shapes(c))
     shapes.update(encoder_head_shapes(c))
     for name, shape in shapes.items():
-        if name.endswith('basic_lstm_cell/bias') or name.endswith('LN_tanh/beta') \
-                or name.endswith('output_projection/bias'):
+        if name.endswith('gru_cell/gates/bias'):
+            w[name] = np.ones(shape, np.float32)           # GRUCell: constant 1.0 gate bias
+        elif name.endswith('basic_lstm_cell/bias') or name.endswith('gru_cell/candidate/bias') \
+                or name.endswith('LN_tanh/beta') or name.endswith('output_projection/bias'):
             w[name] = np.zeros(shape, np.float32)
         elif name.endswith('LN_tanh/gamma'):
             w[name] = np.ones(shape, np.float32)

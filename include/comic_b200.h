@@ -65,8 +65,8 @@ typedef struct {
 
 /* Device pointers to the reference's variables, TF shapes (SURVEY.md §8a). */
 typedef struct {
-  const float* lstm_kernel;      /* [W+A+R, 4R] gate order i,j,f,o */
-  const float* lstm_bias;        /* [4R] */
+  const float* lstm_kernel;      /* [W+A+R, 4R] gate order i,j,f,o; GRU cell: gates/kernel [W+A+R, 2R], r then u */
+  const float* lstm_bias;        /* [4R]; GRU cell: gates/bias [2R] */
   const float* init_weight;      /* first_input: [E, W+A]; project_hidden: [E, R] */
   const float* memory_kernel;    /* [C, R] */
   const float* value_kernel;     /* [C, R] (independent) or NULL */
@@ -108,6 +108,27 @@ int comic_packed_bytes(comic_handle_t h, size_t* bytes);
  * engine).  `with_cnn` = 0 binds the decoder only. */
 int comic_bind_weights(comic_handle_t h, const comic_weights_t* w, int with_cnn,
                        void* packed, size_t packed_bytes, void* stream);
+
+/* Recurrent cell of the decoder (c.rnn_name, src/model_base.py:622-629).  Call after comic_create and before
+ * comic_packed_bytes / comic_workspace_bytes / comic_bind_weights: the packed weights and the decode workspaces are
+ * laid out for the cell.  Any other value returns COMIC_E_UNSUPPORTED.
+ *   LSTM: BasicLSTMCell (default).
+ *   GRU:  TF r1.9 GRUCell, state h only:
+ *           [r, u] = sigmoid([x, h] . gates/kernel + gates/bias)
+ *           c      = tanh([x, r*h] . candidate/kernel + candidate/bias)
+ *           h'     = u*h + (1-u)*c
+ *         The c0 / c_in / c_out arguments of comic_rnn_init, comic_decode_step, comic_decode_greedy and
+ *         comic_decode_beam may be NULL and are neither read nor written.  Decodes take the per-step path (no
+ *         persistent loop).  Training writes the candidate gradients to comic_decoder_grads_t.cand_kernel / cand_bias. */
+#define COMIC_CELL_LSTM 0
+#define COMIC_CELL_GRU  1
+int comic_set_rnn_cell(comic_handle_t h, int cell);
+/* GRU cell: candidate/kernel [W+A+R, R] and candidate/bias [R], bound by pointer (the weights are read in place by
+ * every bind / comic_refresh_packed).  Call before comic_bind_weights, which refuses a GRU handle without them; a call
+ * after binding unbinds the weights until the next comic_bind_weights.  comic_set_rnn_cell returns COMIC_E_BADARG once
+ * a size (packed, workspace, train workspace) was queried or weights were bound;
+ * comic_weights_t.lstm_kernel / lstm_bias carry gates/kernel / gates/bias. */
+int comic_bind_gru_candidate(comic_handle_t h, const float* kernel, const float* bias);
 
 /* Arithmetic modes (all within the 1e-3 parity bound of the reference's fp32 graph):
  *   0  fp32 FFMA everywhere (the reference's fp32 arithmetic up to summation order);
@@ -303,6 +324,9 @@ typedef struct {
   float* query_kernel; float* attention_v; float* ln_gamma; float* ln_beta; float* temperature;
   float* out_kernel; float* out_bias; float* embedding_map;
   float* a_layer;                /* [VAL, R] (attn_context_layer, common/ops_rnn.py:734-739) or NULL */
+  float* cand_kernel;            /* GRU cell: candidate/kernel [W+A+R, R] (lstm_kernel / lstm_bias receive gates/{kernel,
+                                    bias}); NULL for the LSTM */
+  float* cand_bias;              /* GRU cell: candidate/bias [R] */
 } comic_decoder_grads_t;
 
 int comic_train_workspace_bytes(comic_handle_t h, int B, int T_run, size_t* bytes);
