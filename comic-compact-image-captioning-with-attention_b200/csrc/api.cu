@@ -113,7 +113,7 @@ extern "C" int comic_profile_read(comic_handle_t h, int tag, double* total_ms, i
 
 namespace comic {
 int pack_tc_weight(comic_handle_t h, Carver& cv, const float* W, int K, int N, int ldw, int cin_src, int cin_dst,
-                   tc::TcWeight& out, cudaStream_t st, bool dry, int gate_R) {
+                   tc::TcWeight& out, cudaStream_t st, bool dry) {
   (void)h;
   int ntaps = K / cin_src;
   int Kd = (cin_src == cin_dst) ? K : ntaps * cin_dst;
@@ -127,7 +127,7 @@ int pack_tc_weight(comic_handle_t h, Carver& cv, const float* W, int K, int N, i
   out.ready = false;
   if (dry) return COMIC_OK;
   tc::pack_bt_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(W, K, N, ldw, out.hi, out.lo, out.Kpad, out.Npad,
-                                                                 cin_src, cin_dst, gate_R);
+                                                                 cin_src, cin_dst);
   COMIC_CHECK_CUDA(cudaGetLastError());
   COMIC_REQUIRE(tc::make_weight_maps(out), COMIC_E_CUDA, "cuTensorMapEncodeTiled failed for a %d x %d weight", N, Kd);
   return COMIC_OK;
@@ -150,22 +150,14 @@ extern "C" int comic_set_option(comic_handle_t h, int option, int value) {
       if (value < 0) break;
       h->persist_watchdog_ms = value;
       return COMIC_OK;
-    case COMIC_OPT_ENC_PLANES: h->enc_planes = value; return COMIC_OK;
-    case COMIC_OPT_STEM_S2D: h->stem_s2d = value; return COMIC_OK;
+    case COMIC_OPT_STEM_S2D:
+      COMIC_REQUIRE(value == 0 || value == 2, COMIC_E_BADARG, "set_option: stem_s2d must be 0 (7x7 gather) or 2 (halo)");
+      h->stem_s2d = value;
+      return COMIC_OK;
     case COMIC_OPT_TC_MIN_ROWS: h->tc_min_rows = value; return COMIC_OK;
     case COMIC_OPT_TC_SPLITK: h->tc_splitk = value; return COMIC_OK;
     case COMIC_OPT_ATTN2: h->attn2 = value; return COMIC_OK;
-    case COMIC_OPT_FUSE_LSTM: h->fuse_lstm = value; return COMIC_OK;
     case COMIC_OPT_TMA_A: h->tma_a = value; return COMIC_OK;
-    case COMIC_OPT_GEMM_SMALL_TILES: tc::small_tiles() = value; return COMIC_OK;
-    case COMIC_OPT_PDL: pdl_mode() = value; return COMIC_OK;
-    case COMIC_OPT_GEMM_RESIDENT_B: tc::bres_mode() = value; return COMIC_OK;
-    case COMIC_OPT_GEMM_PAIR: tc::pair_mode() = value; return COMIC_OK;
-    case COMIC_OPT_GEMM_PAIR_MIN_TILES: tc::pair_min_tiles() = value; return COMIC_OK;
-    case COMIC_OPT_GEMM_MC:
-      if (value != 0 && value != 1 && value != 2 && value != 4) break;
-      tc::mc_mode() = value;
-      return COMIC_OK;
     case COMIC_OPT_ENC_CHUNK_STEM:
     case COMIC_OPT_ENC_CHUNK_28:
     case COMIC_OPT_ENC_CHUNK_14:

@@ -60,7 +60,6 @@
 #include <stdint.h>
 
 #include "attention.cuh"
-#include "pdl.cuh"
 
 namespace comic {
 namespace a2 {
@@ -384,7 +383,6 @@ __global__ void __launch_bounds__((NSW + kCtxWarps2 + 1 + kStatWarps) * 32, 1) a
   unsigned long long g_entry;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g_entry));
 #endif
-  pdl_launch_dependents();
   using L = Layout<K, NSW, STAGES>;
   extern __shared__ __align__(1024) unsigned char smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -457,9 +455,6 @@ __global__ void __launch_bounds__((NSW + kCtxWarps2 + 1 + kStatWarps) * 32, 1) a
     *reinterpret_cast<float4*>(sm_c + 2 * kR + c4 * 4) = make_float4(vs * v4.y, vs * v4.w, vs * v4.x, vs * v4.z);
   }
   __syncthreads();
-  // the prologue above read only weights and the per-call score bound: as a programmatic dependent it overlaps the tail of
-  // the [logits | query] GEMM; the queries (and the step gate) are read from here on
-  pdl_wait();
   if (a.fin_count != nullptr && a.t > 0 && a.fin_count[a.t - 1] >= a.n_rows) return;
   if (n_g == 0) return;
 #if COMIC_A2_TRACE
@@ -1040,7 +1035,8 @@ inline cudaError_t launch_k(const Args& a, int num_sms, int dev, cudaStream_t st
   const long long total = (long long)a.B * (a.M / kPos);
   const int grid = total < num_sms ? (int)total : num_sms;
   if (a.scratch == nullptr || a.counters == nullptr) return cudaErrorInvalidValue;
-  return launch_pdl(attn2_kernel<K, NSW, STAGES>, dim3(grid), dim3(L::kThreads), smem, st, a);
+  attn2_kernel<K, NSW, STAGES><<<grid, L::kThreads, smem, st>>>(a);
+  return cudaGetLastError();
 }
 
 inline cudaError_t launch(const Args& a, int k, int num_sms, int dev, cudaStream_t st) {

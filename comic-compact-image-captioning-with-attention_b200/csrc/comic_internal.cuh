@@ -52,8 +52,6 @@ struct Packed {
   tc::TcWeight tc_conv[COMIC_NUM_CONVS];
   tc::TcWeight tc_grp[kNumBlocks];
   tc::TcWeight tc_lstm, tc_outq, tc_mem, tc_val, tc_init;
-  tc::TcWeight tc_lstm_il;       // lstm kernel with gate-interleaved columns (fused LSTM epilogue of the gate GEMM)
-  float* lstm_bias_il = nullptr; // [4R] bias in the same column order
   // GRU cell: [gates/kernel | candidate/kernel x-rows ; 0] panel [W+A+R, 3R] of the gate GEMM, and the tensor-path packs
   // of that panel and of the candidate kernel's h-rows [R, R]
   float* gru_gx = nullptr;
@@ -85,11 +83,6 @@ struct comic_handle_s {
                                // default: its slice-granular work split fills the SMs from ~12 images (39 vs 48 us at 12
                                // images x 3 beams, 33 vs 48 at 25, profiles/r08c_attn_small_batch.txt); an explicit
                                // fused_min_images moves both thresholds
-  int fuse_lstm = 0;           // 1: gate GEMM with the LSTM point-wise update in its epilogue (tensor path, no dropout / tape).
-                               // Bit-identical to the separate kernel but measured SLOWER at 1,536 rows (gates + lstm 2.86 ->
-                               // 3.02 ms per 60 steps, profiles/r06e): the GEMM has 96 tiles on 148 SMs, one per CTA, so the
-                               // epilogue's transcendentals are not hidden behind a next tile's MMAs, while the separate
-                               // kernel spreads them over the whole chip.  Off by default.
   int tma_a = 1;               // bit 0: [logits | query] GEMM, bit 1: gate GEMM read their A operand as bf16 planes through
                                // TMA (no gather / split in the GEMM's loader warps)
   int attn2 = 1;               // streaming attention kernel (attention2.cuh) where it applies: tied values, add_LN, softmax,
@@ -105,9 +98,7 @@ struct comic_handle_s {
   int tc_min_rows = 64;        // GEMMs / convs with at least this many rows take the tensor path (precision >= 1); half-empty
                                // M tiles still beat the FFMA kernel (batch 25-32 beam-3: gate GEMM 37 -> 29 us, r02p)
   int stem_s2d = 2;            // tensor path stem conv: 2 = space-to-depth planes, im2col tile built from a shared-memory
-                               // halo patch; 1 = same conv, operand rows gathered from L2 with cp.async; 0 = 7x7/2 gather
-                               // from the fp32 NHWC4 image
-  int enc_planes = 0;          // 1: encoder activations as pre-split bf16 planes on the tensor path (0 = fp32 NHWC)
+                               // halo patch; 0 = 7x7/2 gather from the fp32 NHWC4 image
   int enc_chunk[3] = {256, 512, 512};  // images per encoder chunk: stem / 28x28 blocks / 14x14 + 7x7 blocks (measured r01p:
                                        // the GEMMs are L2->SM bound, not HBM bound, so fewer, longer launches win over L2 residency)
   comic::Packed pk;
@@ -161,7 +152,7 @@ inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 // Carve + (unless dry) fill one tensor-path weight pack from W[K][N] (row stride ldw).
 int pack_tc_weight(comic_handle_t h, Carver& cv, const float* W, int K, int N, int ldw, int cin_src, int cin_dst,
-                   tc::TcWeight& out, cudaStream_t st, bool dry, int gate_R = 0);
+                   tc::TcWeight& out, cudaStream_t st, bool dry);
 inline bool use_tc(comic_handle_t h, const tc::TcWeight& w, int M) { return h->precision >= 1 && w.ready && M >= h->tc_min_rows; }
 // Split-K factor of a tensor-path decode-step GEMM that is far from filling the chip (33..~400 rows: batch 25 x beam 3 = 75
 // rows is the reference's default inference shape, src/infer.py:72).  One 128-row tile per 128 columns leaves 16 of 148

@@ -73,8 +73,6 @@ lstm_pointwise4_kernel(const float* __restrict__ gates, const float* __restrict_
                        const int* __restrict__ src, int src_limit, float* __restrict__ c_new, float* __restrict__ h_new,
                        int N, int R, const int* fin_count, int t, int n_rows, uint16_t* __restrict__ h_hi = nullptr,
                        uint16_t* __restrict__ h_lo = nullptr, int nz = 1, size_t zstride = 0) {
-  pdl_launch_dependents();
-  pdl_wait();
   if (step_stopped(fin_count, t, n_rows)) return;
   const int R4 = R >> 2;
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -533,8 +531,6 @@ beam_step_kernel(const float* __restrict__ logits, int ld, int k, int V, int eos
 constexpr int kBeamWarpImages = 4;
 __global__ void __launch_bounds__(32 * kBeamWarpImages)
 beam_step_warp_kernel(const BeamWarpArgs g, int B, int n_rows) {
-  pdl_launch_dependents();
-  pdl_wait();
   if (step_stopped(g.fin_count, g.t, n_rows)) {
     if (blockIdx.x == 0 && threadIdx.x == 0) g.fin_count[g.t] = n_rows;
     return;
@@ -556,8 +552,6 @@ beam_step_rows_kernel(const float* __restrict__ logits, int ld, int B, int k, in
                       float* __restrict__ log_probs, uint8_t* __restrict__ finished, long long* __restrict__ lengths,
                       float* __restrict__ scores_out, int* __restrict__ word_out, int* __restrict__ parent_out,
                       int* __restrict__ tok_next, int* __restrict__ src_next, int* fin_count, int t, int n_rows) {
-  pdl_launch_dependents();
-  pdl_wait();
   if (step_stopped(fin_count, t, n_rows)) {
     if (blockIdx.x == 0 && threadIdx.x == 0) fin_count[t] = n_rows;
     return;
@@ -661,15 +655,14 @@ static void launch_beam_step(const float* logits, int ld, int B, int k, int V, i
                              int* tok_next, int* src_next, int* fin_count, int t, int n_rows, cudaStream_t st) {
   if (k * V <= 1536 && k >= 2 && k <= 8 && B >= 2 * kBeamWarpImages) {
     const size_t smem = (size_t)kBeamRowImages * (k * V + 2 * k) * sizeof(float);
-    launch_pdl(beam_step_rows_kernel, dim3((B + kBeamRowImages - 1) / kBeamRowImages), dim3(32 * k * kBeamRowImages), smem, st,
-               logits, ld, B, k, V, eos, lpw, log_probs, finished, lengths, scores_out, word_out, parent_out, tok_next, src_next,
-               fin_count, t, n_rows);
+    beam_step_rows_kernel<<<(B + kBeamRowImages - 1) / kBeamRowImages, 32 * k * kBeamRowImages, smem, st>>>(
+        logits, ld, B, k, V, eos, lpw, log_probs, finished, lengths, scores_out, word_out, parent_out, tok_next, src_next,
+        fin_count, t, n_rows);
   } else if (k * V <= 1536 && k <= 32 && B >= 2 * kBeamWarpImages) {
     const size_t smem = (size_t)kBeamWarpImages * k * V * sizeof(float);
     BeamWarpArgs g{logits, ld, k, V, eos, lpw, log_probs, finished, lengths, scores_out, word_out, parent_out, tok_next, src_next,
                    fin_count, t};
-    launch_pdl(beam_step_warp_kernel, dim3((B + kBeamWarpImages - 1) / kBeamWarpImages), dim3(32 * kBeamWarpImages), smem, st, g,
-               B, n_rows);
+    beam_step_warp_kernel<<<(B + kBeamWarpImages - 1) / kBeamWarpImages, 32 * kBeamWarpImages, smem, st>>>(g, B, n_rows);
   } else {
     beam_step_kernel<<<B, 256, 0, st>>>(logits, ld, k, V, eos, lpw, log_probs, finished, lengths, scores_out, word_out,
                                         parent_out, tok_next, src_next, fin_count, t, n_rows);
@@ -840,11 +833,6 @@ int decoder_configure() {
 }
 
 // Tensor-path (3xTF32) panels of the decoder weights.
-__global__ void interleave_gate_bias_kernel(const float* __restrict__ bias, float* __restrict__ out, int R) {
-  const int n = blockIdx.x * blockDim.x + threadIdx.x;
-  if (n < 4 * R) out[n] = bias[(n & 3) * R + (n >> 2)];
-}
-
 static int decoder_pack_tc(comic_handle_t h, Carver& cv, cudaStream_t st, bool dry) {
   int rc;
   const int XA = h->W + h->A;
@@ -854,12 +842,6 @@ static int decoder_pack_tc(comic_handle_t h, Carver& cv, cudaStream_t st, bool d
       return rc;
   } else {
     if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm, st, dry))) return rc;
-    if ((rc = pack_tc_weight(h, cv, h->w.lstm_kernel, h->KX, 4 * h->R, 4 * h->R, 1, 1, h->pk.tc_lstm_il, st, dry, h->R))) return rc;
-    h->pk.lstm_bias_il = cv.take<float>((size_t)4 * h->R);
-    if (!dry) {
-      interleave_gate_bias_kernel<<<(4 * h->R + 255) / 256, 256, 0, st>>>(h->w.lstm_bias, h->pk.lstm_bias_il, h->R);
-      COMIC_CHECK_CUDA(cudaGetLastError());
-    }
   }
   if ((rc = pack_tc_weight(h, cv, h->pk.outq, h->R, h->LQ, h->LQ, 1, 1, h->pk.tc_outq, st, dry))) return rc;
   if ((rc = pack_tc_weight(h, cv, h->w.memory_kernel, h->C, h->R, h->R, 1, 1, h->pk.tc_mem, st, dry))) return rc;
@@ -1093,7 +1075,6 @@ static int run_gru_cell(comic_handle_t h, const StepIO& io, const StepBufs& sb, 
   e1.ksplit = ks1;
   e1.stop = stop;
   e1.stop_n = stop_n;
-  e1.pdl = 1;
   {
     Prof pf(h, T_GATES, st);
     if (tc1) COMIC_CHECK_CUDA((tc::launch_gemm_tc<0>(a, h->pk.tc_gru_g, N, 3 * R, e1, h->num_sms, st)));
@@ -1184,25 +1165,15 @@ int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int 
   e1.ksplit = ks1;
   e1.stop = io.fin_count ? io.fin_count + (io.t > 0 ? io.t - 1 : 0) : nullptr;
   e1.stop_n = (io.fin_count && io.t > 0) ? io.n_rows : 0x7fffffff;
-  e1.pdl = 1;
-  // tensor path without dropout / tape: the LSTM point-wise update runs in the gate GEMM's epilogue over the
-  // gate-interleaved panel (same arithmetic, in the same order, as lstm_pointwise4_kernel<true>: bit-identical c / h)
-  const bool fused_lstm = tc1 && ks1 == 1 && h->fuse_lstm && h->pk.tc_lstm_il.ready && !io.h_drop && !io.out_mask && !io.gates_save;
   // A operands as bf16 planes through TMA (inference decode on the tensor path: no dropout, no tape)
   const bool tma_ok = sb.tma_a && h->tma_a && h->precision >= 1 && !io.in_mask && !io.force_dense && !io.h_drop &&
                       !io.out_mask && !io.gates_save;
-  const bool tma_gates = tma_ok && (h->tma_a & 2) && tc1 && ks1 == 1 && !fused_lstm;
+  const bool tma_gates = tma_ok && (h->tma_a & 2) && tc1 && ks1 == 1;
   // h' planes exist when the 4-units-per-thread LSTM kernel below runs
   const bool lstm4 = R % 4 == 0 && !io.h_drop && !io.out_mask && !io.gates_save && N >= 128 && (nz1 == 1 || (tc1 && h->precision >= 1));
-  const bool tma_lq = tma_ok && (h->tma_a & 1) && !fused_lstm && lstm4 && R % 4 == 0 && N >= 128 &&
+  const bool tma_lq = tma_ok && (h->tma_a & 1) && lstm4 && R % 4 == 0 && N >= 128 &&
                       use_tc(h, h->pk.tc_outq, N);
-  if (fused_lstm) {
-    e1.bias = h->pk.lstm_bias_il;
-    e1.lstm_c_prev = io.c_prev; e1.lstm_src = io.src; e1.lstm_src_limit = io.src_limit;
-    e1.lstm_c = io.c_new; e1.lstm_h = io.h_new; e1.lstm_R = R;
-    Prof pf(h, T_GATES, st);
-    COMIC_CHECK_CUDA((tc::launch_gemm_tc<0>(a, h->pk.tc_lstm_il, N, 4 * R, e1, h->num_sms, st)));
-  } else if (tma_gates) {
+  if (tma_gates) {
     Prof pf(h, T_GATES, st, 2);
     const int tot4 = N * (h->KX / 4);
     build_x_planes_kernel<<<(tot4 + 255) / 256, 256, 0, st>>>(h->w.embedding_map, io.tok, h->V, io.ctx_prev, io.h_prev, io.src,
@@ -1214,19 +1185,19 @@ int run_step(comic_handle_t h, const StepIO& io, const StepBufs& sb, int B, int 
     if (tc1) COMIC_CHECK_CUDA((tc::launch_gemm_tc<0>(a, h->pk.tc_lstm, N, 4 * R, e1, h->num_sms, st)));
     else COMIC_CHECK_CUDA((launch_gemm<0, 4>(a, h->w.lstm_kernel, 4 * R, N, 4 * R, h->KX, e1, p1, st)));
   }
-  if (!fused_lstm) {
+  {
     Prof pf(h, T_LSTM, st);
     int tot = N * R;
     if (lstm4) {
       const int tot4 = N * (R / 4);
       if (h->precision >= 1 && nz1 > 1)
-        launch_pdl(lstm_pointwise4_kernel<true, true>, dim3((tot4 + 255) / 256), dim3(256), 0, st, sb.gates, h->w.lstm_bias, io.c_prev,
-                   io.src, io.src_limit, io.c_new, io.h_new, N, R, io.fin_count, io.t, io.n_rows,
-                   tma_lq ? sb.hp_hi : nullptr, tma_lq ? sb.hp_lo : nullptr, nz1, (size_t)N * 4 * R);
+        lstm_pointwise4_kernel<true, true><<<(tot4 + 255) / 256, 256, 0, st>>>(
+            sb.gates, h->w.lstm_bias, io.c_prev, io.src, io.src_limit, io.c_new, io.h_new, N, R, io.fin_count, io.t, io.n_rows,
+            tma_lq ? sb.hp_hi : nullptr, tma_lq ? sb.hp_lo : nullptr, nz1, (size_t)N * 4 * R);
       else if (h->precision >= 1)
-        launch_pdl(lstm_pointwise4_kernel<true, false>, dim3((tot4 + 255) / 256), dim3(256), 0, st, sb.gates, h->w.lstm_bias, io.c_prev,
-                   io.src, io.src_limit, io.c_new, io.h_new, N, R, io.fin_count, io.t, io.n_rows,
-                   tma_lq ? sb.hp_hi : nullptr, tma_lq ? sb.hp_lo : nullptr, 1, (size_t)0);
+        lstm_pointwise4_kernel<true, false><<<(tot4 + 255) / 256, 256, 0, st>>>(
+            sb.gates, h->w.lstm_bias, io.c_prev, io.src, io.src_limit, io.c_new, io.h_new, N, R, io.fin_count, io.t, io.n_rows,
+            tma_lq ? sb.hp_hi : nullptr, tma_lq ? sb.hp_lo : nullptr, 1, (size_t)0);
       else
         lstm_pointwise4_kernel<false><<<(tot4 + 255) / 256, 256, 0, st>>>(sb.gates, h->w.lstm_bias, io.c_prev, io.src, io.src_limit,
                                                                          io.c_new, io.h_new, N, R, io.fin_count, io.t, io.n_rows);
@@ -1258,7 +1229,6 @@ static int step_tail(comic_handle_t h, const StepIO& io, const StepBufs& sb, int
   e2.nroute = 1;
   e2.stop = e1.stop;
   e2.stop_n = e1.stop_n;
-  e2.pdl = 1;
   if (nz2 == 1) {
     e2.bias = h->pk.outq_bias;
     e2.r[0] = Route{0, h->LQ, sb.lq, h->LQ, 0};

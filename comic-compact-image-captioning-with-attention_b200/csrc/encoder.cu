@@ -13,7 +13,6 @@
 // (Branch_0, Branch_1/0a, Branch_2/0a) run as ONE GEMM over a packed
 // [Cin, b0+b1a+b2a] weight panel with a 3-way routed epilogue.
 #include "comic_internal.cuh"
-#include <algorithm>
 
 namespace comic {
 
@@ -178,8 +177,8 @@ __global__ void pad_c3_c4_kernel(const float* __restrict__ x, float* __restrict_
 // 2*ho - 2 + kh = 2*(ho - 1 + (kh >> 1)) + (kh & 1): with X2[n, i, j, (a*2 + b)*3 + c] = x[n, 2i + a, 2j + b, c]
 // it is   y[ho, wo] = sum_{di, dj < 4} sum_{ch < 12} X2[ho - 1 + di, wo - 1 + dj, ch] * W2[di, dj, ch]
 // with W2[di, dj, (a*2 + b)*3 + c] = W[2di + a, 2dj + b, c] (zero where 2di + a or 2dj + b reaches 7): the same
-// products, but 16-channel taps (12 + 4 zero) that the bf16-plane loader copies with cp.async instead of
-// gathering 49 single-pixel taps per output.  X2 is stored directly as bf16 (hi, lo) planes.
+// products, but 16-channel taps (12 + 4 zero) that the halo loader (gemm_tc.cuh AMODE 3) stages in shared memory
+// instead of gathering 49 single-pixel taps per output.  X2 is stored directly as bf16 (hi, lo) planes.
 // --------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 s2d_split_kernel(const float* __restrict__ x, uint16_t* __restrict__ hi, uint16_t* __restrict__ lo, size_t npix2) {
@@ -309,101 +308,6 @@ maxpool3s1_rows_kernel(const float* __restrict__ x, float* __restrict__ y, unsig
   }
 }
 
-
-// --------------------------------------------------------------------------
-// bf16-plane activations (tensor path): every conv output is stored once as an error-compensated
-// bf16 pair (hi, lo) by the producing GEMM's epilogue, so the consuming conv's loader is a plain
-// cp.async copy into its operand tiles (gemm_tc.cuh AMODE 2) instead of an fp32 gather + split per
-// tap and per N tile.  hi + lo carries 16 mantissa bits -- exactly what the bf16x3 MMA consumes.
-// --------------------------------------------------------------------------
-struct Planes {
-  uint16_t* hi;
-  uint16_t* lo;
-};
-
-static inline Planes planes_of(float* buf, size_t cap_elems) {
-  Planes p;
-  p.hi = reinterpret_cast<uint16_t*>(buf);
-  p.lo = p.hi + cap_elems;
-  return p;
-}
-static inline Planes planes_at(Planes p, size_t off) { return Planes{p.hi + off, p.lo + off}; }
-
-__device__ __forceinline__ void unpack8(const uint4& h, const uint4& l, float (&v)[8]) {
-  const uint32_t hw[4] = {h.x, h.y, h.z, h.w}, lw[4] = {l.x, l.y, l.z, l.w};
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    v[2 * j] = __uint_as_float(hw[j] << 16) + __uint_as_float(lw[j] << 16);
-    v[2 * j + 1] = __uint_as_float(hw[j] & 0xffff0000u) + __uint_as_float(lw[j] & 0xffff0000u);
-  }
-}
-
-// max pool over NHWC activations, 8 channels per thread; input either bf16 planes or fp32, output planes.
-template <int K, bool IN_F32>
-__global__ void __launch_bounds__(256)
-maxpool_planes_kernel(const uint16_t* __restrict__ xh, const uint16_t* __restrict__ xl, const float* __restrict__ xf,
-                      uint16_t* __restrict__ yh, uint16_t* __restrict__ yl, unsigned total, int H, int W, int C8,
-                      int stride, int pad_t, int pad_l, int Ho, int Wo) {
-  unsigned i = blockIdx.x * 256u + threadIdx.x;
-  if (i >= total) return;
-  unsigned c8 = i % (unsigned)C8, p = i / (unsigned)C8;
-  unsigned wo = p % (unsigned)Wo, q = p / (unsigned)Wo;
-  unsigned ho = q % (unsigned)Ho, b = q / (unsigned)Ho;
-  const int h0 = (int)ho * stride - pad_t, w0 = (int)wo * stride - pad_l;
-  const size_t base = (size_t)b * H * W * C8 + c8;
-  float m[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) m[j] = -INFINITY;
-  if (IN_F32) {
-    float4 va[K * K], vb[K * K];
-    const float4* xb = reinterpret_cast<const float4*>(xf) + base * 2;
-#pragma unroll
-    for (int dh = 0; dh < K; ++dh)
-#pragma unroll
-      for (int dw = 0; dw < K; ++dw) {
-        const int hi = h0 + dh, wi = w0 + dw;
-        const bool ok = hi >= 0 && hi < H && wi >= 0 && wi < W;
-        const float4 ninf = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
-        va[dh * K + dw] = ok ? __ldg(xb + ((size_t)hi * W + wi) * C8 * 2) : ninf;
-        vb[dh * K + dw] = ok ? __ldg(xb + ((size_t)hi * W + wi) * C8 * 2 + 1) : ninf;
-      }
-#pragma unroll
-    for (int t = 0; t < K * K; ++t) {
-      m[0] = fmaxf(m[0], va[t].x); m[1] = fmaxf(m[1], va[t].y); m[2] = fmaxf(m[2], va[t].z); m[3] = fmaxf(m[3], va[t].w);
-      m[4] = fmaxf(m[4], vb[t].x); m[5] = fmaxf(m[5], vb[t].y); m[6] = fmaxf(m[6], vb[t].z); m[7] = fmaxf(m[7], vb[t].w);
-    }
-  } else {
-    uint4 vh[K * K], vl[K * K];
-    bool okv[K * K];
-    const uint4* hb = reinterpret_cast<const uint4*>(xh) + base;
-    const uint4* lb = reinterpret_cast<const uint4*>(xl) + base;
-#pragma unroll
-    for (int dh = 0; dh < K; ++dh)
-#pragma unroll
-      for (int dw = 0; dw < K; ++dw) {
-        const int hi = h0 + dh, wi = w0 + dw;
-        const bool ok = hi >= 0 && hi < H && wi >= 0 && wi < W;
-        okv[dh * K + dw] = ok;
-        const size_t o = ok ? ((size_t)hi * W + wi) * C8 : 0;
-        vh[dh * K + dw] = __ldg(hb + o);
-        vl[dh * K + dw] = __ldg(lb + o);
-      }
-#pragma unroll
-    for (int t = 0; t < K * K; ++t) {
-      float v[8];
-      unpack8(vh[t], vl[t], v);
-      if (okv[t]) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) m[j] = fmaxf(m[j], v[j]);
-      }
-    }
-  }
-  uint2 h0p, l0p, h1p, l1p;
-  tc::split4(make_float4(m[0], m[1], m[2], m[3]), h0p, l0p);
-  tc::split4(make_float4(m[4], m[5], m[6], m[7]), h1p, l1p);
-  reinterpret_cast<uint4*>(yh)[(size_t)p * C8 + c8] = make_uint4(h0p.x, h0p.y, h1p.x, h1p.y);
-  reinterpret_cast<uint4*>(yl)[(size_t)p * C8 + c8] = make_uint4(l0p.x, l0p.y, l1p.x, l1p.y);
-}
 
 // slim.avg_pool2d(net, [7,7], stride=1) VALID on a 7x7 map -> [B, C]
 // (common/nets/inception_v1.py:326).
@@ -597,60 +501,9 @@ int run_block(comic_handle_t h, int bi, const float* x, float* y, int B, int S, 
 }
 
 
-// ---- bf16-plane variants of the layer runners (tensor path only) -------------------------
-static int run_maxpool_p(comic_handle_t h, Planes x, const float* xf, Planes y, int B, int H, int W, int C, int k, int s,
-                         cudaStream_t st) {
-  int Ho, Wo, pt, pl;
-  same_pads(H, k, s, &Ho, &pt);
-  same_pads(W, k, s, &Wo, &pl);
-  size_t total = (size_t)B * Ho * Wo * (C / 8);
-  COMIC_REQUIRE(total < 0xffffffffull && C % 8 == 0 && (k == 2 || k == 3), COMIC_E_UNSUPPORTED,
-                "maxpool (planes): unsupported shape (total %zu, C %d, k %d)", total, C, k);
-  unsigned grid = (unsigned)((total + 255) / 256);
-  {
-    Prof pf(h, T_POOL, st);
-    if (xf) {
-      if (k == 3) maxpool_planes_kernel<3, true><<<grid, 256, 0, st>>>(nullptr, nullptr, xf, y.hi, y.lo, (unsigned)total, H, W, C / 8, s, pt, pl, Ho, Wo);
-      else maxpool_planes_kernel<2, true><<<grid, 256, 0, st>>>(nullptr, nullptr, xf, y.hi, y.lo, (unsigned)total, H, W, C / 8, s, pt, pl, Ho, Wo);
-    } else {
-      if (k == 3) maxpool_planes_kernel<3, false><<<grid, 256, 0, st>>>(x.hi, x.lo, nullptr, y.hi, y.lo, (unsigned)total, H, W, C / 8, s, pt, pl, Ho, Wo);
-      else maxpool_planes_kernel<2, false><<<grid, 256, 0, st>>>(x.hi, x.lo, nullptr, y.hi, y.lo, (unsigned)total, H, W, C / 8, s, pt, pl, Ho, Wo);
-    }
-  }
-  COMIC_CHECK_CUDA(cudaGetLastError());
-  return COMIC_OK;
-}
-
-// conv ci over plane input x [B,H,W,ldx]; output to fp32 (dst) and / or planes (dp) at channel offset coff.
-static int run_conv_p(comic_handle_t h, Planes x, int B, int H, int W, int ldx, int ci, float* dst, Planes dp, int ld_dst,
-                      int coff, cudaStream_t st) {
-  const comic_conv_desc_t& d = kConvs[ci];
-  AConvP a;
-  a.hi = x.hi; a.lo = x.lo; a.H = H; a.W = W; a.Cin = d.c_in; a.ldx = ldx;
-  a.KH = d.k; a.KW = d.k; a.stride = d.stride;
-  same_pads(H, d.k, d.stride, &a.Ho, &a.pad_t);
-  same_pads(W, d.k, d.stride, &a.Wo, &a.pad_l);
-  int M = B * a.Ho * a.Wo, N = d.c_out;
-  Epi e{};
-  e.bias = h->pk.bn_shift[ci];
-  e.scale = h->pk.bn_scale[ci];
-  e.relu = 1;
-  e.nroute = 1;
-  e.r[0] = Route{0, N, dst, ld_dst, coff, dp.hi, dp.lo};
-  cudaError_t err;
-  {
-    Prof pf(h, T_CONV, st);
-    err = tc::launch_gemm_tc<2>(a, h->pk.tc_conv[ci], M, N, e, h->num_sms, st);
-  }
-  COMIC_CHECK_CUDA(err);
-  return COMIC_OK;
-}
-
 // Stem conv on the tensor path through the space-to-depth planes (see s2d_split_kernel): images [nb,224,224,3]
-// -> Conv2d_1a_7x7 output [nb,112,112,64] as fp32 (dst) and / or bf16 planes (dhi / dlo).  `scratch` holds the
-// X2 planes: 2 * nb*112*112*16 bf16.
-static int run_stem_s2d(comic_handle_t h, const float* img, int nb, float* scratch, float* dst, uint16_t* dhi,
-                        uint16_t* dlo, cudaStream_t st) {
+// -> Conv2d_1a_7x7 output dst [nb,112,112,64].  `scratch` holds the X2 planes: 2 * nb*112*112*16 bf16.
+static int run_stem_s2d(comic_handle_t h, const float* img, int nb, float* scratch, float* dst, cudaStream_t st) {
   const size_t npix2 = (size_t)nb * 112 * 112;
   uint16_t* xh = reinterpret_cast<uint16_t*>(scratch);
   uint16_t* xl = xh + npix2 * 16;
@@ -658,138 +511,17 @@ static int run_stem_s2d(comic_handle_t h, const float* img, int nb, float* scrat
     Prof pf(h, T_POOL, st);
     s2d_split_kernel<<<(unsigned)((npix2 + 255) / 256), 256, 0, st>>>(img, xh, xl, npix2);
   }
-  AConvP a;
-  a.hi = xh; a.lo = xl; a.H = 112; a.W = 112; a.Cin = 16; a.ldx = 16;
-  a.KH = 4; a.KW = 4; a.stride = 1; a.pad_t = 1; a.pad_l = 1; a.Ho = 112; a.Wo = 112;
+  AHalo a;
+  a.hi = xh; a.lo = xl; a.nimg = nb;
   Epi e{};
   e.bias = h->pk.bn_shift[0]; e.scale = h->pk.bn_scale[0]; e.relu = 1; e.nroute = 1;
-  e.r[0] = Route{0, 64, dst, 64, 0, dhi, dlo};
+  e.r[0] = Route{0, 64, dst, 64, 0};
   cudaError_t err;
   {
     Prof pf(h, T_CONV, st);
-    if (h->stem_s2d >= 2) {
-      AHalo ah;
-      ah.hi = xh; ah.lo = xl; ah.nimg = nb;
-      err = tc::launch_stem_halo(ah, h->pk.tc_stem_s2d, e, h->num_sms, st);
-    } else {
-      err = tc::launch_gemm_tc<2>(a, h->pk.tc_stem_s2d, nb * 112 * 112, 64, e, h->num_sms, st);
-    }
+    err = tc::launch_stem_halo(a, h->pk.tc_stem_s2d, e, h->num_sms, st);
   }
   COMIC_CHECK_CUDA(err);
-  return COMIC_OK;
-}
-
-struct PBufs {
-  Planes t1, t2, p;
-};
-
-// One inception block on planes: x [B,S,S,cin] -> y (fp32 y32 and / or planes yp) [B,S,S,cout].
-static int run_block_p(comic_handle_t h, int bi, Planes x, float* y32, Planes yp, int B, int S, const PBufs& pb,
-                       cudaStream_t st) {
-  const BlockDesc& bd = block_table()[bi];
-  int cout = bd.b0 + bd.b1b + bd.b2b + bd.b3;
-  int M = B * S * S;
-  {
-    AConvP a;
-    a.hi = x.hi; a.lo = x.lo; a.H = S; a.W = S; a.Cin = bd.cin; a.ldx = bd.cin;
-    a.KH = 1; a.KW = 1; a.stride = 1; a.pad_t = 0; a.pad_l = 0; a.Ho = S; a.Wo = S;
-    int ng = bd.b0 + bd.b1a + bd.b2a;
-    Epi e{};
-    e.bias = h->pk.grp_shift[bi];
-    e.scale = h->pk.grp_scale[bi];
-    e.relu = 1;
-    e.nroute = 3;
-    e.r[0] = Route{0, bd.b0, y32, cout, 0, yp.hi, yp.lo};
-    e.r[1] = Route{bd.b0, bd.b0 + bd.b1a, nullptr, bd.b1a, 0, pb.t1.hi, pb.t1.lo};
-    e.r[2] = Route{bd.b0 + bd.b1a, ng, nullptr, bd.b2a, 0, pb.t2.hi, pb.t2.lo};
-    cudaError_t err;
-    {
-      Prof pf(h, T_CONV, st);
-      err = tc::launch_gemm_tc<2>(a, h->pk.tc_grp[bi], M, ng, e, h->num_sms, st);
-    }
-    COMIC_CHECK_CUDA(err);
-  }
-  int rc;
-  if ((rc = run_conv_p(h, pb.t1, B, S, S, bd.b1a, bd.conv[2], y32, yp, cout, bd.b0, st))) return rc;
-  if ((rc = run_conv_p(h, pb.t2, B, S, S, bd.b2a, bd.conv[4], y32, yp, cout, bd.b0 + bd.b1b, st))) return rc;
-  if ((rc = run_maxpool_p(h, x, nullptr, pb.p, B, S, S, bd.cin, 3, 1, st))) return rc;
-  if ((rc = run_conv_p(h, pb.p, B, S, S, bd.cin, bd.conv[5], y32, yp, cout, bd.b0 + bd.b1b + bd.b2b, st))) return rc;
-  return COMIC_OK;
-}
-
-// The whole forward on planes (same chunk plan and workspace carving as the fp32-activation path).
-static int encoder_forward_planes(comic_handle_t h, const float* images, int B, float* fm_out, float* im_embed_out,
-                                  float* mixed5c_out, void* ws, cudaStream_t st) {
-  const EncPlan pl = enc_plan(h, B);
-  Carver cv(ws);
-  float* fa = cv.take<float>(pl.ab);
-  float* fb = cv.take<float>(pl.ab);
-  float* ft1 = cv.take<float>(pl.t1);
-  float* ft2 = cv.take<float>(pl.t2);
-  float* fp = cv.take<float>(pl.p);
-  float* fpool2 = cv.take<float>(pl.p2);
-  float* fpool3 = cv.take<float>(pl.p3);
-  cv.take<float>(pl.head);
-  const Planes pa = planes_of(fa, pl.ab), pbn = planes_of(fb, pl.ab);
-  PBufs pb;
-  pb.t1 = planes_of(ft1, pl.t1); pb.t2 = planes_of(ft2, pl.t2); pb.p = planes_of(fp, pl.p);
-  const Planes pool2 = planes_of(fpool2, pl.p2), pool3 = planes_of(fpool3, pl.p3);
-  const Planes none{nullptr, nullptr};
-  int rc;
-  // ---- stem: the 7x7/2 conv reads the fp32 image (NHWC4 staged in buffer b), everything after it planes
-  for (int b0 = 0; b0 < B; b0 += pl.cs) {
-    int nb = (B - b0 < pl.cs) ? (B - b0) : pl.cs;
-    const float* img = images + (size_t)b0 * 224 * 224 * 3;
-    if (h->stem_s2d) {
-      if ((rc = run_stem_s2d(h, img, nb, fb, nullptr, pa.hi, pa.lo, st))) return rc;
-    } else {
-      run_pad_c3_c4(h, img, fb, (size_t)nb * 224 * 224, st);
-      const comic_conv_desc_t& d = kConvs[0];
-      AConv a;
-      a.x = fb; a.H = 224; a.W = 224; a.Cin = 4; a.ldx = 4; a.KH = d.k; a.KW = d.k; a.stride = d.stride;
-      same_pads(224, d.k, d.stride, &a.Ho, &a.pad_t);
-      same_pads(224, d.k, d.stride, &a.Wo, &a.pad_l);
-      Epi e{};
-      e.bias = h->pk.bn_shift[0]; e.scale = h->pk.bn_scale[0]; e.relu = 1; e.nroute = 1;
-      e.r[0] = Route{0, 64, nullptr, 64, 0, pa.hi, pa.lo};
-      cudaError_t err;
-      {
-        Prof pf(h, T_CONV, st);
-        err = tc::launch_gemm_tc<1>(a, h->pk.tc_conv[0], nb * 112 * 112, 64, e, h->num_sms, st);
-      }
-      COMIC_CHECK_CUDA(err);
-    }
-    if ((rc = run_maxpool_p(h, pa, nullptr, pbn, nb, 112, 112, 64, 3, 2, st))) return rc;            // 56x56x64
-    if ((rc = run_conv_p(h, pbn, nb, 56, 56, 64, 1, nullptr, pa, 64, 0, st))) return rc;
-    if ((rc = run_conv_p(h, pa, nb, 56, 56, 64, 2, nullptr, pbn, 192, 0, st))) return rc;           // 56x56x192
-    if ((rc = run_maxpool_p(h, pbn, nullptr, planes_at(pool2, (size_t)b0 * 28 * 28 * 192), nb, 56, 56, 192, 3, 2, st)))
-      return rc;
-  }
-  // ---- Mixed_3b, 3c @28
-  for (int b0 = 0; b0 < B; b0 += pl.c3) {
-    int nb = (B - b0 < pl.c3) ? (B - b0) : pl.c3;
-    if ((rc = run_block_p(h, 0, planes_at(pool2, (size_t)b0 * 28 * 28 * 192), nullptr, pbn, nb, 28, pb, st))) return rc;
-    if ((rc = run_block_p(h, 1, pbn, nullptr, pa, nb, 28, pb, st))) return rc;
-    if ((rc = run_maxpool_p(h, pa, nullptr, planes_at(pool3, (size_t)b0 * 14 * 14 * 480), nb, 28, 28, 480, 3, 2, st)))
-      return rc;
-  }
-  // ---- Mixed_4b..4f @14, Mixed_5b, 5c @7, head
-  for (int b0 = 0; b0 < B; b0 += pl.c4) {
-    int nb = (B - b0 < pl.c4) ? (B - b0) : pl.c4;
-    if ((rc = run_block_p(h, 2, planes_at(pool3, (size_t)b0 * 14 * 14 * 480), nullptr, pa, nb, 14, pb, st))) return rc;
-    if ((rc = run_block_p(h, 3, pa, nullptr, pbn, nb, 14, pb, st))) return rc;
-    if ((rc = run_block_p(h, 4, pbn, nullptr, pa, nb, 14, pb, st))) return rc;
-    if ((rc = run_block_p(h, 5, pa, nullptr, pbn, nb, 14, pb, st))) return rc;
-    float* fm = fm_out + (size_t)b0 * 196 * 832;
-    if ((rc = run_block_p(h, 6, pbn, fm, none, nb, 14, pb, st))) return rc;            // Mixed_4f -> fp32 feature map
-    if ((rc = run_maxpool_p(h, none, fm, pa, nb, 14, 14, 832, 2, 2, st))) return rc;   // 7x7x832
-    if ((rc = run_block_p(h, 7, pa, nullptr, pbn, nb, 7, pb, st))) return rc;
-    // Mixed_5c in fp32 (average pool input); buffer a is free again once Mixed_5b has read it
-    float* m5c = mixed5c_out ? mixed5c_out + (size_t)b0 * 49 * 1024 : fa;
-    if ((rc = run_block_p(h, 8, pbn, m5c, none, nb, 7, pb, st))) return rc;
-    run_avgpool_global(h, m5c, im_embed_out + (size_t)b0 * 1024, nb, 49, 1024, st);
-    COMIC_CHECK_CUDA(cudaGetLastError());
-  }
   return COMIC_OK;
 }
 
@@ -801,13 +533,6 @@ int encoder_forward(comic_handle_t h, const float* images, int B, float* fm_out,
   encoder_workspace_bytes(h, B, &need);
   COMIC_REQUIRE(ws_bytes >= need, COMIC_E_WORKSPACE, "encode_fwd: workspace %zu < %zu", ws_bytes, need);
   const EncPlan pl = enc_plan(h, B);
-  {
-    // bf16-plane activations whenever every launch of every chunk takes the tensor path (>= 128 rows)
-    auto tail = [](int n, int c) { return n % c ? n % c : c; };
-    const int min_imgs = std::min(std::min(tail(B, pl.cs), tail(B, pl.c3)), tail(B, pl.c4));
-    if (h->precision >= 1 && h->enc_planes && !h->cfg.legacy && h->pk.tc_conv[0].ready && min_imgs * 49 >= 128)
-      return encoder_forward_planes(h, images, B, fm_out, im_embed_out, mixed5c_out, ws, st);
-  }
   Carver cv(ws);
   EncBufs eb;
   eb.a = cv.take<float>(pl.ab); eb.b = cv.take<float>(pl.ab);
@@ -822,7 +547,7 @@ int encoder_forward(comic_handle_t h, const float* images, int B, float* fm_out,
     const float* img = images + (size_t)b0 * 224 * 224 * 3;
     int Ho, Wo;
     if (use_tc(h, h->pk.tc_stem_s2d, nb * 112 * 112) && h->stem_s2d) {
-      if ((rc = run_stem_s2d(h, img, nb, eb.b, eb.a, nullptr, nullptr, st))) return rc;
+      if ((rc = run_stem_s2d(h, img, nb, eb.b, eb.a, st))) return rc;
     } else if (use_tc(h, h->pk.tc_conv[0], nb * 112 * 112)) {
       size_t npix = (size_t)nb * 224 * 224;
       {

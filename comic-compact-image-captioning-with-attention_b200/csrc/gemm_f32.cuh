@@ -18,8 +18,6 @@
 // buffering through shared memory, 128-bit loads/stores.
 #pragma once
 #include <cuda.h>
-
-#include "pdl.cuh"
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -64,14 +62,9 @@ struct AConv {
 
 struct Route {
   int n0, n1;   // column range [n0, n1)
-  float* dst;   // fp32 destination (nullable on the tensor path when only the bf16 planes are wanted)
+  float* dst;
   int ld;
   int coff;
-  // tensor path only: the same element also as an error-compensated bf16 pair (hi = bf16(v),
-  // lo = bf16(v - hi)) in two planes with the row stride / channel offset above; the next conv's
-  // loader copies these straight into its shared-memory operand tiles (gemm_tc.cuh AConvP)
-  uint16_t* hi;
-  uint16_t* lo;
 };
 
 struct Epi {
@@ -85,17 +78,6 @@ struct Epi {
                            // z of tile (m, n) goes to route dst + z * split_stride (0 / 1 = off); no bias / scale then
   const int* stop;         // optional device flag: skip the launch when *stop >= stop_n
   int stop_n;              // (decode loops: every beam finished in the previous step)
-  int pdl;                 // host side only: launch as a programmatic dependent (tensor path, launch_one)
-  // LSTM epilogue (tensor path, gate GEMM over a GATE-INTERLEAVED weight panel: column 4 u + g = gate g of unit u, so
-  // the four consecutive columns an epilogue lane owns are i, j, f, o of one unit).  lstm_h != nullptr: instead of
-  // storing the pre-activations the epilogue adds `bias` (interleaved the same way), applies the BasicLSTMCell
-  // point-wise update (forget_bias 1.0) against c_prev[src[m]] and writes c / h [M, lstm_R].
-  const float* lstm_c_prev;
-  const int* lstm_src;
-  int lstm_src_limit;
-  float* lstm_c;
-  float* lstm_h;
-  int lstm_R;
 };
 
 // sigmoid / tanh of the big-batch decode path (engine precision >= 1): ex2.approx + rcp, relative error ~1e-6 against
@@ -114,14 +96,6 @@ __device__ __forceinline__ float tanh_(float x) {
   return tanhf(x);
 }
 
-// NHWC activations stored pre-split as two bf16 planes (tensor path, gemm_tc.cuh).
-struct AConvP {
-  const uint16_t* hi;
-  const uint16_t* lo;   // [B, H, W, ldx] each, channels [0, Cin), Cin % 8 == 0
-  int H, W, Cin, ldx;
-  int KH, KW, stride, pad_t, pad_l, Ho, Wo;
-};
-
 // Stem conv over the space-to-depth image (bf16 planes [nimg,112,112,16]) with the im2col tile built from a
 // shared-memory halo patch instead of 16 L2 reads per input element (tensor path, gemm_tc.cuh AMODE 3).
 struct AHalo {
@@ -133,7 +107,6 @@ struct AHalo {
 template <int AMODE> struct AParam;
 template <> struct AParam<0> { typedef APlain type; };
 template <> struct AParam<1> { typedef AConv type; };
-template <> struct AParam<2> { typedef AConvP type; };
 template <> struct AParam<3> { typedef AHalo type; };
 // AMODE 4 (tensor path only): the A operand exists as bf16 (hi, lo) planes [rows, K] in global memory and is staged by
 // TMA like the weights -- no loader warps, no per-CTA gather / split (decoder GEMMs: gemm_tc.cuh, decoder.cu)

@@ -142,82 +142,11 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-// ---- CTA-pair helpers (tcgen05 cta_group::2) ---------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t rank) {
-  uint32_t remote;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t addr = smem_u32(bar);
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-  } while (!done);
-}
-// TMA load whose completion bytes are counted on the LEADER CTA's barrier (peer bit of the
-// shared::cluster address cleared), destination in the executing CTA's shared memory.
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t smem_dst, const CUtensorMap* tm, uint64_t* bar, int c0,
-                                                 int c1) {
-  const uint32_t leader_bar = smem_u32(bar) & 0xFEFFFFFFu;
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tm)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                               uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"((uint16_t)3)
-      : "memory");
-}
-// ---- weight-tile multicast (MC CTAs of a cluster share an N tile) ---------------------------------
-// TMA load delivered to the same shared-memory offset of every CTA in `mask`; each destination's barrier (same offset)
-// receives the bytes of the box.
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t smem_dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// one arrival on the barrier at this offset in every CTA of `mask` when this CTA's earlier UMMAs retire
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ void sts_v2(uint32_t addr, uint32_t a, uint32_t b) {
   asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
 }
 
-// One im2col row of the tile (AMODE 1 / 2): pointer to channel 0 of the receptive field's top-left
+// One im2col row of the tile (AMODE 1): pointer to channel 0 of the receptive field's top-left
 // pixel (it may lie outside the image: only dereferenced for taps whose mask bit is set) and the
 // validity of each of the KH*KW taps (TF SAME padding; rows beyond M have mask 0).
 struct RowEntry {
@@ -225,22 +154,15 @@ struct RowEntry {
   unsigned long long mask;
 };
 
-// PAIR = false: one CTA per 128 x BN tile.  PAIR = true: the two CTAs of a cluster compute a
-// 256 x BN tile with M = 256 UMMAs issued by the leader (rank 0); each CTA loads its own 128 rows
-// of A and HALF of the weight tile, so a CTA pulls half the weight bytes per output and its stage
-// shrinks (BN = 256: 96 -> 64 KB, 3 stages instead of 2).  full_a / full_b / tmem_empty then live in
-// the leader and collect (remote) arrivals of both CTAs; empty / tmem_full exist in both CTAs and
-// are signalled by the leader's multicast tcgen05.commit.  Operand layouts, epilogue and the UMMA
-// order per accumulator element are the same in both modes: results are bit-identical.
 // halo patch of the stem conv (AMODE 3): an 8 x 16 tile of outputs of the 4 x 4 stride-1 conv reads 11 x 19 input
 // pixels of 16 channels; per plane 11 * 19 * 32 bytes, hi + lo, double buffered
 constexpr int kHaloRows = 11, kHaloCols = 19;
 constexpr int kHaloPlaneBytes = ((kHaloRows * kHaloCols * 32 + 127) / 128) * 128;   // 6784
 constexpr int kHaloBytes = 2 * 2 * kHaloPlaneBytes;
 
-template <int BN, int STAGES, bool PAIR, int NKRES = 0, bool HALO = false>
+template <int BN, int STAGES, int NKRES = 0, bool HALO = false>
 struct SmemLayout {
-  static constexpr int B_TILE_BYTES = (PAIR ? BN / 2 : BN) * BK * 2;   // this CTA's part of one weight tile (hi or lo)
+  static constexpr int B_TILE_BYTES = BN * BK * 2;                // one weight tile (hi or lo)
   // NKRES > 0: the whole weight panel (<= NKRES K blocks, one N tile) is loaded ONCE per CTA and stays in shared
   // memory; the ring then stages only A (more stages), and the panel is not re-streamed for every M tile
   static constexpr int STAGE_BYTES = 2 * A_TILE_BYTES + (NKRES ? 0 : 2 * B_TILE_BYTES);
@@ -256,24 +178,13 @@ struct SmemLayout {
   static constexpr int TMEM_COLS = (2 * BN <= 32) ? 32 : (2 * BN <= 64) ? 64 : (2 * BN <= 128) ? 128 : (2 * BN <= 256) ? 256 : 512;   // two accumulator buffers; allocations are powers of two
 };
 
-// MC > 1 (PAIR = false): the MC CTAs of a cluster work on MC consecutive M tiles of the SAME N tile.  Each loads 1 / MC of
-// the weight tile and multicasts it into all of them, so the panel crosses L2 -> SM once per cluster instead of once per
-// CTA (the decoder's gate GEMM and the wide convolutions are bound by exactly that traffic).  A stage may be overwritten
-// only when every CTA's UMMAs have consumed it: `empty` collects one multicast commit per CTA.
-template <int BN, int STAGES, int AMODE, bool PAIR, int NKRES = 0, int MC = 1>
+template <int BN, int STAGES, int AMODE, int NKRES = 0>
 __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::type& a, const CUtensorMap* tm_hi,
                                                  const CUtensorMap* tm_lo, int M, int N, int K, const Epi& epi) {
-  static_assert(!(PAIR && NKRES), "resident weight panel: single-CTA kernel only");
-  static_assert(MC == 1 || (!PAIR && NKRES == 0 && AMODE != 3 && (BN / MC) % 64 == 0), "multicast: plain kernel, slices of >= 64 rows");
-  static_assert(AMODE != 4 || (!PAIR && NKRES == 0 && MC == 1), "TMA-staged A: plain kernel only");
-  constexpr bool CL = PAIR || MC > 1;           // launched as a cluster
-  constexpr uint16_t kMcMask = (uint16_t)((1u << MC) - 1u);
+  static_assert(AMODE != 4 || NKRES == 0, "TMA-staged A: plain kernel only");
   static_assert(AMODE != 3 || (NKRES > 0 && BN == 64), "halo loader: resident-panel stem kernel only");
-  using L = SmemLayout<BN, STAGES, PAIR, NKRES, AMODE == 3>;
-  constexpr int TM = (PAIR ? 2 : MC) * BM;      // rows per (pair / cluster) tile
-  constexpr int MMA_M = PAIR ? 2 * BM : BM;
+  using L = SmemLayout<BN, STAGES, NKRES, AMODE == 3>;
   extern __shared__ uint8_t smem_raw[];
-  pdl_launch_dependents();           // the next kernel of the stream may start its own prologue (it waits before it reads)
   const uint32_t smem = (smem_u32(smem_raw) + 1023u) & ~1023u;      // shared-window address of the tiles
   uint8_t* smem_g = smem_raw + (smem - smem_u32(smem_raw));
   uint8_t* rowtab0 = smem_g + L::TILES_BYTES;
@@ -286,54 +197,41 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES + 4);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t rank = CL ? cluster_ctarank() : 0u;
-  const bool leader = PAIR ? rank == 0 : true;
   const int nk = (K + BK - 1) / BK;
   const int n_tiles = (N + BN - 1) / BN;
-  const int m_tiles = (M + TM - 1) / TM;          // AMODE 3: M = nimg * 112 * 112 = nimg * 98 tiles of 8 x 16 outputs
+  const int m_tiles = (M + BM - 1) / BM;          // AMODE 3: M = nimg * 112 * 112 = nimg * 98 tiles of 8 x 16 outputs
   // split-K (launches of one or two M tiles, e.g. the decoder GEMMs at 33..128 rows, where a tile's K loop is a chain of
   // ~1.3 us operand-staging latencies): work item = (K range z, tile mn); the partial sums go to dst + z * split_stride
   // and are added in a fixed order by the consumer
-  const int ksplit = (AMODE == 0 && !PAIR && MC == 1 && NKRES == 0 && epi.ksplit > 1) ? epi.ksplit : 1;
+  const int ksplit = (AMODE == 0 && NKRES == 0 && epi.ksplit > 1) ? epi.ksplit : 1;
   const int mn_tiles = m_tiles * n_tiles;
   const int total_tiles = mn_tiles * ksplit;
-  const int first_tile = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x / MC;
-  const int tile_step = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x / MC;
+  const int first_tile = (int)blockIdx.x;
+  const int tile_step = (int)gridDim.x;
 
   // ---- one-time setup ----
   if (tid == 0) {
     for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_a[s], (AMODE >= 2 ? 256 : 128) * (PAIR ? 2 : 1));
+      mbar_init(&full_a[s], AMODE >= 3 ? 256 : 128);
       mbar_init(&full_b[s], 1);
-      mbar_init(&empty[s], MC);
+      mbar_init(&empty[s], 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tmem_full[i], 1);
-      mbar_init(&tmem_empty[i], PAIR ? 2 * kEpiWarps : kEpiWarps);
+      mbar_init(&tmem_empty[i], kEpiWarps);
     }
     fence_barrier_init();
   }
   if (warp == kMmaWarp) {
-    if constexpr (PAIR) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                   "r"((uint32_t)L::TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                   "r"((uint32_t)L::TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
+                 "r"((uint32_t)L::TMEM_COLS)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (CL) cluster_sync_all();     // every CTA's barriers exist before any remote arrive / multicast
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // everything above touched only this CTA's shared / tensor memory: a programmatic dependent launch overlaps it with the
-  // predecessor's tail.  From here on global memory is read and written.
-  pdl_wait();
   const bool stopped = epi.stop != nullptr && *epi.stop >= epi.stop_n;      // uniform over the grid
 
   if (stopped) {
@@ -358,7 +256,7 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
     int iter = 0;
     for (int tile = first_tile; tile < total_tiles; tile += tile_step, ++iter) {
       const int kz = tile / mn_tiles, mn = tile - kz * mn_tiles;
-      const int m0 = (mn / n_tiles) * TM + (int)rank * BM;
+      const int m0 = (mn / n_tiles) * BM;
       const int n0 = (mn % n_tiles) * BN;
       const int acc = iter & 1;
       const int n_umma = min(BN, ((N - n0) + 15) & ~15);
@@ -376,36 +274,9 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
           return mw + row;
         }
       };
-      // LSTM epilogue: the rows this lane stores are fixed for the tile -> resolve the state-row indirection once, and
-      // fetch c_prev one column block ahead (the dependent src -> c_prev loads would otherwise sit in every iteration)
-      const float* cprow[4] = {nullptr, nullptr, nullptr, nullptr};
-      float cp_next[4] = {0.f, 0.f, 0.f, 0.f};
-      if (epi.lstm_h != nullptr && epi.lstm_c_prev != nullptr) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const int m = row_to_m(q * 8 + srow);
-          if (m < M) {
-            const int rr = epi.lstm_src ? epi.lstm_src[m] : m;
-            if (rr >= 0 && rr < epi.lstm_src_limit) cprow[q] = epi.lstm_c_prev + (size_t)rr * epi.lstm_R;
-          }
-        }
-        const int u0 = (n0 + half * 16 + scol) >> 2;
-        if (n0 + half * 16 + scol < N) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) if (cprow[q]) cp_next[q] = __ldg(cprow[q] + u0);
-        }
-      }
 #pragma unroll 1
       for (int c0 = half * 16; c0 < n_umma; c0 += 32) {
         uint32_t r[16];
-        float cp_cur[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) cp_cur[q] = cp_next[q];
-        if (epi.lstm_h != nullptr && c0 + 32 < n_umma && n0 + c0 + 32 + scol < N) {
-          const int un = (n0 + c0 + 32 + scol) >> 2;
-#pragma unroll
-          for (int q = 0; q < 4; ++q) cp_next[q] = cprow[q] ? __ldg(cprow[q] + un) : 0.f;
-        }
         uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BN + c0);
         asm volatile(
             "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, "
@@ -424,31 +295,10 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
         if (n < N) {
           const int rt = n >= b2 ? 2 : (n >= b1 ? 1 : 0);
           float* const fdst = epi.r[rt].dst;
-          uint16_t* const hdst = epi.r[rt].hi;
-          uint16_t* const ldst = epi.r[rt].lo;
           const long long ld = epi.r[rt].ld;
           const long long cofs = (long long)epi.r[rt].coff - epi.r[rt].n0 + n + (long long)kz * epi.split_stride;
           const float4 sc = epi.scale ? ldg4(epi.scale + n) : make_float4(1.f, 1.f, 1.f, 1.f);
           const float4 bs = epi.bias ? ldg4(epi.bias + n) : make_float4(0.f, 0.f, 0.f, 0.f);
-          if (epi.lstm_h != nullptr) {
-            // gate-interleaved panel: columns n .. n + 3 are the i, j, f, o pre-activations of unit n / 4
-            const int u = n >> 2;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const int row = q * 8 + srow;
-              const int m = row_to_m(row);
-              if (m < M) {
-                const float4 v = *reinterpret_cast<const float4*>(stage_buf + row * L::EPI_STRIDE + scol);
-                const float cp = cp_cur[q];
-                const float cn = cp * sig_<true>((v.z + bs.z) + 1.0f) + sig_<true>(v.x + bs.x) * tanh_<true>(v.y + bs.y);
-                const float hn = tanh_<true>(cn) * sig_<true>(v.w + bs.w);
-                epi.lstm_c[(size_t)m * epi.lstm_R + u] = cn;
-                epi.lstm_h[(size_t)m * epi.lstm_R + u] = hn;
-              }
-            }
-            __syncwarp();
-            continue;
-          }
 #pragma unroll
           for (int q = 0; q < 4; ++q) {
             const int row = q * 8 + srow;
@@ -461,13 +311,7 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
                 v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f);
               }
               const long long o = (long long)m * ld + cofs;
-              if (fdst) *reinterpret_cast<float4*>(fdst + o) = v;
-              if (hdst) {
-                uint2 sh, sl;
-                split4(v, sh, sl);
-                *reinterpret_cast<uint2*>(hdst + o) = sh;
-                *reinterpret_cast<uint2*>(ldst + o) = sl;
-              }
+              *reinterpret_cast<float4*>(fdst + o) = v;
             }
           }
         }
@@ -476,14 +320,11 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
       // accumulator buffer drained -> the MMA warp may overwrite it
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (PAIR) mbar_arrive_cluster(&tmem_empty[acc], 0);
-        else mbar_arrive(&tmem_empty[acc]);
-      }
+      if (lane == 0) mbar_arrive(&tmem_empty[acc]);
     }
   } else if (warp == kMmaWarp) {
-    // =====================  MMA issuer (PAIR: leader CTA only)  =====================
-    if (leader && lane == 0) {
+    // =====================  MMA issuer  =====================
+    if (lane == 0) {
       int iter = 0;
       uint32_t it = 0;
       if constexpr (NKRES > 0) mbar_wait(&full_b[0], 0);      // resident weight panel landed
@@ -493,21 +334,15 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
         const int n0 = (mn % n_tiles) * BN;
         const int acc = iter & 1;
         const int n_umma = min(BN, ((N - n0) + 15) & ~15);
-        const uint32_t idesc = make_idesc_bf16(MMA_M, n_umma);
+        const uint32_t idesc = make_idesc_bf16(BM, n_umma);
         const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BN);
-        if constexpr (PAIR) mbar_wait_cluster(&tmem_empty[acc], (uint32_t)(((iter >> 1) & 1) ^ 1));
-        else mbar_wait(&tmem_empty[acc], (uint32_t)(((iter >> 1) & 1) ^ 1));
+        mbar_wait(&tmem_empty[acc], (uint32_t)(((iter >> 1) & 1) ^ 1));
         tc_fence_after();
         for (int kt = kt0; kt < kt1; ++kt, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1;
-          if constexpr (PAIR) {
-            mbar_wait_cluster(&full_a[s], ph);
-            mbar_wait_cluster(&full_b[s], ph);
-          } else {
-            if constexpr (AMODE != 4) mbar_wait(&full_a[s], ph);      // AMODE 4: A arrives with B on full_b
-            if constexpr (NKRES == 0) mbar_wait(&full_b[s], ph);
-          }
+          if constexpr (AMODE != 4) mbar_wait(&full_a[s], ph);      // AMODE 4: A arrives with B on full_b
+          if constexpr (NKRES == 0) mbar_wait(&full_b[s], ph);
           tc_fence_after();
           const uint32_t a_hi = smem + s * L::STAGE_BYTES;
           const uint32_t a_lo = a_hi + A_TILE_BYTES;
@@ -519,29 +354,18 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
           for (int k16 = 0; k16 < BK / 16; ++k16) {
             const uint64_t adv = (uint64_t)((k16 * 16 * 2) >> 4);    // 32 bytes per K=16 step inside the swizzle row
             const uint32_t first = (kt > kt0 || k16 > 0) ? 1u : 0u;
-            if constexpr (PAIR) {
-              umma_bf16_pair(d_tmem, dah + adv, dbh + adv, idesc, first);
-              umma_bf16_pair(d_tmem, dal + adv, dbh + adv, idesc, 1u);
-              umma_bf16_pair(d_tmem, dah + adv, dbl + adv, idesc, 1u);
-            } else {
-              umma_bf16(d_tmem, dah + adv, dbh + adv, idesc, first);
-              umma_bf16(d_tmem, dal + adv, dbh + adv, idesc, 1u);
-              umma_bf16(d_tmem, dah + adv, dbl + adv, idesc, 1u);
-            }
+            umma_bf16(d_tmem, dah + adv, dbh + adv, idesc, first);
+            umma_bf16(d_tmem, dal + adv, dbh + adv, idesc, 1u);
+            umma_bf16(d_tmem, dah + adv, dbl + adv, idesc, 1u);
           }
-          // frees the stage (PAIR: in both CTAs) when the MMAs above retire
-          if constexpr (PAIR) umma_commit_pair(&empty[s]);
-          else if constexpr (MC > 1) umma_commit_mc(&empty[s], kMcMask);
-          else umma_commit(&empty[s]);
+          umma_commit(&empty[s]);             // frees the stage when the MMAs above retire
         }
-        // accumulator complete -> epilogue (PAIR: of both CTAs)
-        if constexpr (PAIR) umma_commit_pair(&tmem_full[acc]);
-        else umma_commit(&tmem_full[acc]);
+        umma_commit(&tmem_full[acc]);         // accumulator complete -> epilogue
       }
     }
     __syncwarp();
   } else if (warp == kTmaWarp) {
-    // =====================  TMA producer (this CTA's part of the weight tile)  =====================
+    // =====================  TMA producer (weight tiles)  =====================
     if constexpr (NKRES > 0) {
       if (lane == 0 && first_tile < total_tiles) {
         mbar_arrive_expect_tx(&full_b[0], (uint32_t)nk * 2u * L::B_TILE_BYTES);
@@ -558,44 +382,32 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
         const int kz = tile / mn_tiles, mn = tile - kz * mn_tiles;
         const int kt0 = (int)(((long long)kz * nk) / ksplit), kt1 = (int)(((long long)(kz + 1) * nk) / ksplit);
         const int n0 = (mn % n_tiles) * BN;
-        const int n_umma = min(BN, ((N - n0) + 15) & ~15);
-        const int nrow = PAIR ? n0 + (int)rank * (n_umma >> 1) : n0 + (int)rank * (BN / MC);   // first row of B^T this CTA loads
         for (int kt = kt0; kt < kt1; ++kt, ++it) {
           const int s = it % STAGES;
           const uint32_t ph = (it / STAGES) & 1;
           mbar_wait(&empty[s], ph ^ 1);
           const uint32_t b_hi = smem + s * L::STAGE_BYTES + 2 * A_TILE_BYTES;
           const uint32_t b_lo = b_hi + L::B_TILE_BYTES;
-          if constexpr (PAIR) {
-            if (leader) mbar_arrive_expect_tx(&full_b[s], 4 * L::B_TILE_BYTES);   // both CTAs' hi + lo boxes
-            tma_load_2d_pair(b_hi, tm_hi, &full_b[s], kt * BK, nrow);
-            tma_load_2d_pair(b_lo, tm_lo, &full_b[s], kt * BK, nrow);
-          } else if constexpr (MC > 1) {
-            // the whole tile lands here: this CTA's slice + the peers' (their complete_tx may precede this arrive)
-            mbar_arrive_expect_tx(&full_b[s], 2 * L::B_TILE_BYTES);
-            const uint32_t slice = rank * (uint32_t)((BN / MC) * BK * 2);
-            tma_load_2d_mc(b_hi + slice, tm_hi, &full_b[s], kt * BK, nrow, kMcMask);
-            tma_load_2d_mc(b_lo + slice, tm_lo, &full_b[s], kt * BK, nrow, kMcMask);
-          } else if constexpr (AMODE == 4) {
+          if constexpr (AMODE == 4) {
             // both operands by TMA: 128 rows of the (hi, lo) A planes + the weight tile, one transaction
-            const int m0 = (mn / n_tiles) * TM;
+            const int m0 = (mn / n_tiles) * BM;
             const uint32_t a_hi = smem + s * L::STAGE_BYTES;
             mbar_arrive_expect_tx(&full_b[s], 2 * L::B_TILE_BYTES + 2 * A_TILE_BYTES);
             tma_load_2d(a_hi, &a.hi, &full_b[s], kt * BK, m0);
             tma_load_2d(a_hi + A_TILE_BYTES, &a.lo, &full_b[s], kt * BK, m0);
-            tma_load_2d(b_hi, tm_hi, &full_b[s], kt * BK, nrow);
-            tma_load_2d(b_lo, tm_lo, &full_b[s], kt * BK, nrow);
+            tma_load_2d(b_hi, tm_hi, &full_b[s], kt * BK, n0);
+            tma_load_2d(b_lo, tm_lo, &full_b[s], kt * BK, n0);
           } else {
             mbar_arrive_expect_tx(&full_b[s], 2 * L::B_TILE_BYTES);
-            tma_load_2d(b_hi, tm_hi, &full_b[s], kt * BK, nrow);
-            tma_load_2d(b_lo, tm_lo, &full_b[s], kt * BK, nrow);
+            tma_load_2d(b_hi, tm_hi, &full_b[s], kt * BK, n0);
+            tma_load_2d(b_lo, tm_lo, &full_b[s], kt * BK, n0);
           }
         }
       }
     }
     __syncwarp();
   } else {
-    // =====================  A loaders (this CTA's 128 rows)  =====================
+    // =====================  A loaders  =====================
     if constexpr (AMODE == 4) {
       // the TMA warp stages A: nothing to do
     } else if constexpr (AMODE == 3) {
@@ -660,83 +472,6 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
         }
       }
       asm volatile("cp.async.wait_group 0;" ::: "memory");
-    } else if constexpr (AMODE == 2) {
-      // Pre-split bf16 planes: no conversion and no register staging.  All 8 loader warps copy every K
-      // block (thread: 4 rows x one 16-byte chunk = 8 channels, per plane) with cp.async straight into the
-      // swizzled tiles, and up to STAGES blocks stay in flight: block `it` is retired (wait_group ->
-      // proxy fence -> full_a arrive) only when block it + STAGES - 1 has been issued, so the bytes in
-      // flight are bounded by the shared-memory ring, not by registers.
-      const int lw = warp - kFirstLoaderWarp;                 // 0..7
-      const int tg = lw * 32 + lane;                          // 0..255
-      const int c8 = lane & 7, r4 = lane >> 3;
-      RowEntry* re = reinterpret_cast<RowEntry*>(rowtab0);
-      uint32_t it = 0, retired = 0;
-      auto retire = [&]() {
-        fence_proxy_async();
-        uint64_t* bar = &full_a[retired % STAGES];
-        if constexpr (PAIR) mbar_arrive_cluster(bar, 0);
-        else mbar_arrive(bar);
-        ++retired;
-      };
-      for (int tile = first_tile; tile < total_tiles; tile += tile_step) {
-        const int m0 = (tile / n_tiles) * TM + (int)rank * BM;
-        named_bar_sync(1, 256);
-        if (tg < BM) {
-          const int m = m0 + tg;
-          RowEntry e;
-          e.ptr = nullptr; e.mask = 0ull;
-          if (m < M) {
-            const int hw = a.Ho * a.Wo;
-            const int b = m / hw, rem = m - b * hw;
-            const int ho = rem / a.Wo, wo = rem - ho * a.Wo;
-            const int hi0 = ho * a.stride - a.pad_t, wi0 = wo * a.stride - a.pad_l;
-            e.ptr = reinterpret_cast<const void*>((((long long)b * a.H + hi0) * a.W + wi0) * a.ldx);   // element offset
-            for (int kh = 0; kh < a.KH; ++kh)
-              for (int kw = 0; kw < a.KW; ++kw) {
-                const int hi = hi0 + kh, wi = wi0 + kw;
-                if (hi >= 0 && hi < a.H && wi >= 0 && wi < a.W) e.mask |= 1ull << (kh * a.KW + kw);
-              }
-          }
-          re[tg] = e;
-        }
-        named_bar_sync(1, 256);
-        for (int kt = 0; kt < nk; ++kt, ++it) {
-          const int s = it % STAGES;
-          const uint32_t ph = (it / STAGES) & 1;
-          const uint32_t a_hi = smem + s * L::STAGE_BYTES;
-          const int kk8 = kt * BK + c8 * 8;
-          unsigned long long bit = 0ull;
-          long long tapoff = 0;
-          if (kk8 < K) {
-            const int tap = kk8 / a.Cin, ci = kk8 - tap * a.Cin;
-            const int kh = tap / a.KW, kw = tap - kh * a.KW;
-            bit = 1ull << tap;
-            tapoff = ((long long)kh * a.W + kw) * a.ldx + ci;
-          }
-          mbar_wait(&empty[s], ph ^ 1);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const int row = lw * 16 + i * 4 + r4;
-            const RowEntry e = re[row];
-            const bool ok = (e.mask & bit) != 0ull;
-            const long long go = ok ? reinterpret_cast<long long>(e.ptr) + tapoff : 0;
-            const uint32_t so = (uint32_t)row * 128u + ((uint32_t)(c8 ^ (row & 7)) << 4);
-            const uint32_t nbytes = ok ? 16u : 0u;      // src-size 0 -> 16 zero bytes (SAME padding, K tail)
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a_hi + so), "l"(a.hi + go), "r"(nbytes)
-                         : "memory");
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a_hi + A_TILE_BYTES + so), "l"(a.lo + go),
-                         "r"(nbytes)
-                         : "memory");
-          }
-          asm volatile("cp.async.commit_group;" ::: "memory");
-          if (it + 1 - retired == (uint32_t)STAGES) {
-            asm volatile("cp.async.wait_group %0;" ::"n"(STAGES - 1) : "memory");
-            retire();
-          }
-        }
-      }
-      asm volatile("cp.async.wait_group 0;" ::: "memory");
-      while (retired < it) retire();
     } else {
     const int grp = (warp - kFirstLoaderWarp) >> 2;         // loader group
     const int wg = (warp - kFirstLoaderWarp) & 3;           // warp inside the group
@@ -746,7 +481,7 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
     for (int tile = first_tile; tile < total_tiles; tile += tile_step) {
       const int kz = tile / mn_tiles, mn = tile - kz * mn_tiles;
       const int kt0 = (int)(((long long)kz * nk) / ksplit), kt1 = (int)(((long long)(kz + 1) * nk) / ksplit);
-      const int m0 = (mn / n_tiles) * TM + (int)rank * BM;
+      const int m0 = (mn / n_tiles) * BM;
       // per-tile row table (this group's private copy)
       named_bar_sync(1 + grp, 128);
       {
@@ -763,7 +498,7 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
             }
             rp[s * BM + tg] = p;
           }
-        } else {   // AMODE 1 (fp32 NHWC) and 2 (bf16 planes): im2col row table
+        } else {   // AMODE 1: im2col row table
           RowEntry* re = reinterpret_cast<RowEntry*>(rowtab);
           RowEntry e;
           e.ptr = nullptr; e.mask = 0ull;
@@ -772,9 +507,7 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
             const int b = m / hw, rem = m - b * hw;
             const int ho = rem / a.Wo, wo = rem - ho * a.Wo;
             const int hi0 = ho * a.stride - a.pad_t, wi0 = wo * a.stride - a.pad_l;
-            const long long off = (((long long)b * a.H + hi0) * a.W + wi0) * a.ldx;
-            if constexpr (AMODE == 1) e.ptr = a.x + off;
-            else e.ptr = reinterpret_cast<const void*>(off);       // element offset, shared by both planes
+            e.ptr = a.x + (((long long)b * a.H + hi0) * a.W + wi0) * a.ldx;
             for (int kh = 0; kh < a.KH; ++kh)
               for (int kw = 0; kw < a.KW; ++kw) {
                 const int hi = hi0 + kh, wi = wi0 + kw;
@@ -848,33 +581,26 @@ __device__ __forceinline__ void gemm_bf16x3_body(const typename AParam<AMODE>::t
             sts_v2(dst + A_TILE_BYTES, l.x, l.y);
           }
           fence_proxy_async();          // generic-proxy stores -> visible to the tensor core (async proxy)
-          if constexpr (PAIR) mbar_arrive_cluster(&full_a[s], 0);   // the leader counts both CTAs' loader threads
-          else mbar_arrive(&full_a[s]);
+          mbar_arrive(&full_a[s]);
         }
       }
     }
-    }   // AMODE != 2
+    }
   }
 
-  // ---- teardown (PAIR: the peer's shared / tensor memory is in use until the leader's last UMMA retired) ----
+  // ---- teardown ----
   tc_fence_before();
   __syncthreads();
-  if constexpr (CL) cluster_sync_all();
-  if (warp == kMmaWarp) {
-    if constexpr (PAIR)
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)L::TMEM_COLS)
-                   : "memory");
-    else
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)L::TMEM_COLS)
-                   : "memory");
-  }
+  if (warp == kMmaWarp)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)L::TMEM_COLS)
+                 : "memory");
 }
 
 template <int BN, int STAGES, int AMODE>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_bf16x3_kernel(const __grid_constant__ typename AParam<AMODE>::type a, const __grid_constant__ CUtensorMap tm_hi,
                    const __grid_constant__ CUtensorMap tm_lo, int M, int N, int K, const __grid_constant__ Epi epi) {
-  gemm_bf16x3_body<BN, STAGES, AMODE, false>(a, &tm_hi, &tm_lo, M, N, K, epi);
+  gemm_bf16x3_body<BN, STAGES, AMODE>(a, &tm_hi, &tm_lo, M, N, K, epi);
 }
 
 // weights resident in shared memory (N <= 64, K <= NKRES * 64): see SmemLayout
@@ -882,25 +608,8 @@ template <int STAGES, int NKRES, int AMODE>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_bf16x3_bres_kernel(const __grid_constant__ typename AParam<AMODE>::type a, const __grid_constant__ CUtensorMap tm_hi,
                         const __grid_constant__ CUtensorMap tm_lo, int M, int N, int K, const __grid_constant__ Epi epi) {
-  gemm_bf16x3_body<64, STAGES, AMODE, false, NKRES>(a, &tm_hi, &tm_lo, M, N, K, epi);
+  gemm_bf16x3_body<64, STAGES, AMODE, NKRES>(a, &tm_hi, &tm_lo, M, N, K, epi);
 }
-
-// MC CTAs per cluster share the weight tiles (cluster shape given at launch)
-template <int BN, int STAGES, int AMODE, int MC>
-__global__ void __launch_bounds__(kThreads, 1)
-gemm_bf16x3_mc_kernel(const __grid_constant__ typename AParam<AMODE>::type a, const __grid_constant__ CUtensorMap tm_hi,
-                      const __grid_constant__ CUtensorMap tm_lo, int M, int N, int K, const __grid_constant__ Epi epi) {
-  gemm_bf16x3_body<BN, STAGES, AMODE, false, 0, MC>(a, &tm_hi, &tm_lo, M, N, K, epi);
-}
-
-template <int BN, int STAGES, int AMODE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-gemm_bf16x3_pair_kernel(const __grid_constant__ typename AParam<AMODE>::type a, const __grid_constant__ CUtensorMap tm_hi,
-                        const __grid_constant__ CUtensorMap tm_lo, int M, int N, int K,
-                        const __grid_constant__ Epi epi) {
-  gemm_bf16x3_body<BN, STAGES, AMODE, true>(a, &tm_hi, &tm_lo, M, N, K, epi);
-}
-
 
 // ---------------------------------------------------------------------------
 // Host side.
@@ -954,16 +663,12 @@ inline bool make_weight_maps(TcWeight& w) {
 
 // B^T bf16 hi/lo packing: src W[k][n] (row stride ldw); optional channel padding of an
 // HWIO conv kernel (cin_src -> cin_dst, e.g. 3 -> 4 for the NHWC4 stem input).
-// gate_R > 0: the source is an LSTM kernel [K, 4 gate_R] in gate order i | j | f | o; packed row n takes source column
-// (n & 3) * gate_R + (n >> 2), i.e. the panel is gate-INTERLEAVED (see Epi::lstm_h).
 static __global__ void pack_bt_kernel(const float* __restrict__ W, int K, int N, int ldw, uint16_t* __restrict__ hi,
-                                      uint16_t* __restrict__ lo, int Kpad, int Npad, int cin_src, int cin_dst,
-                                      int gate_R = 0) {
+                                      uint16_t* __restrict__ lo, int Kpad, int Npad, int cin_src, int cin_dst) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)Npad * Kpad) return;
   int n = (int)(i / Kpad), kp = (int)(i % Kpad);
   float v = 0.f;
-  const int n_src = gate_R > 0 ? (n & 3) * gate_R + (n >> 2) : n;
   if (n < N) {
     int k = kp;
     bool ok = kp < K;
@@ -972,7 +677,7 @@ static __global__ void pack_bt_kernel(const float* __restrict__ W, int K, int N,
       ok = ci < cin_src && tap < K / cin_src;
       k = tap * cin_src + ci;
     }
-    if (ok) v = W[(size_t)k * ldw + n_src];
+    if (ok) v = W[(size_t)k * ldw + n];
   }
   uint32_t h = pack_bf16x2(v, 0.f) & 0xffffu;
   float hf = __uint_as_float(h << 16);
@@ -984,7 +689,7 @@ static __global__ void pack_bt_kernel(const float* __restrict__ W, int K, int N,
 template <int BN, int STAGES, int AMODE>
 inline cudaError_t launch_one(const typename AParam<AMODE>::type& a, const TcWeight& w, int bn_idx, int M, int N,
                               const Epi& epi, int num_sms, cudaStream_t st) {
-  using L = SmemLayout<BN, STAGES, false>;
+  using L = SmemLayout<BN, STAGES>;
   static PerDeviceOnce once;
   {
     cudaError_t e = once([&] { return cudaFuncSetAttribute(gemm_bf16x3_kernel<BN, STAGES, AMODE>,
@@ -993,8 +698,6 @@ inline cudaError_t launch_one(const typename AParam<AMODE>::type& a, const TcWei
   }
   int tiles = ((N + BN - 1) / BN) * ((M + BM - 1) / BM) * ((AMODE == 0 && epi.ksplit > 1) ? epi.ksplit : 1);
   int grid = tiles < num_sms ? tiles : num_sms;
-  if (epi.pdl) return launch_pdl(gemm_bf16x3_kernel<BN, STAGES, AMODE>, dim3(grid), dim3(kThreads), L::TOTAL, st, a,
-                                 w.tm_hi[bn_idx], w.tm_lo[bn_idx], M, N, w.K, epi);
   gemm_bf16x3_kernel<BN, STAGES, AMODE><<<grid, kThreads, L::TOTAL, st>>>(a, w.tm_hi[bn_idx], w.tm_lo[bn_idx], M,
                                                                           N, w.K, epi);
   return cudaGetLastError();
@@ -1031,7 +734,7 @@ inline int pick_bn(int M, int N, int num_sms, bool small_ok = false) {
 template <int STAGES, int NKRES, int AMODE>
 inline cudaError_t launch_bres(const typename AParam<AMODE>::type& a, const TcWeight& w, int M, int N, const Epi& epi,
                                int num_sms, cudaStream_t st) {
-  using L = SmemLayout<64, STAGES, false, NKRES>;
+  using L = SmemLayout<64, STAGES, NKRES>;
   static_assert(L::TOTAL <= 232448, "resident-panel kernel exceeds the shared memory of an SM");
   static PerDeviceOnce once;
   {
@@ -1047,7 +750,7 @@ inline cudaError_t launch_bres(const typename AParam<AMODE>::type& a, const TcWe
 
 // Stem conv (AMODE 3): a: space-to-depth planes; w: the W2 panel [64, 256]; output rows M = nimg * 12544.
 inline cudaError_t launch_stem_halo(const AHalo& a, const TcWeight& w, const Epi& epi, int num_sms, cudaStream_t st) {
-  using L = SmemLayout<64, 3, false, 4, true>;
+  using L = SmemLayout<64, 3, 4, true>;
   static_assert(L::TOTAL <= 232448, "halo stem kernel exceeds the shared memory of an SM");
   static PerDeviceOnce once;
   {
@@ -1059,74 +762,6 @@ inline cudaError_t launch_stem_halo(const AHalo& a, const TcWeight& w, const Epi
   gemm_bf16x3_bres_kernel<3, 4, 3><<<grid, kThreads, L::TOTAL, st>>>(a, w.tm_hi[0], w.tm_lo[0], a.nimg * 12544, 64, 256, epi);
   return cudaGetLastError();
 }
-
-inline int& bres_mode() { static int v = 1; return v; }      // 0: always stream the weights (A/B experiment switch)
-
-template <int BN, int STAGES, int AMODE>
-inline cudaError_t launch_pair(const typename AParam<AMODE>::type& a, const TcWeight& w, int half_idx, int M, int N,
-                               const Epi& epi, int num_sms, cudaStream_t st) {
-  using L = SmemLayout<BN, STAGES, true>;
-  static PerDeviceOnce once;
-  {
-    cudaError_t e = once([&] { return cudaFuncSetAttribute(gemm_bf16x3_pair_kernel<BN, STAGES, AMODE>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL); });
-    if (e != cudaSuccess) return e;
-  }
-  int tiles = ((N + BN - 1) / BN) * ((M + 2 * BM - 1) / (2 * BM));
-  int grid = 2 * tiles < (num_sms & ~1) ? 2 * tiles : (num_sms & ~1);
-  // the half-width TMA boxes (BN/2 rows) are the maps of the next smaller BN
-  gemm_bf16x3_pair_kernel<BN, STAGES, AMODE><<<grid, kThreads, L::TOTAL, st>>>(a, w.tm_hi[half_idx], w.tm_lo[half_idx],
-                                                                               M, N, w.K, epi);
-  return cudaGetLastError();
-}
-
-// Weight-tile multicast launch: box_idx = tensor map whose box holds BN / MC rows.
-template <int BN, int STAGES, int AMODE, int MC>
-inline cudaError_t launch_mc(const typename AParam<AMODE>::type& a, const TcWeight& w, int box_idx, int M, int N,
-                             const Epi& epi, int num_sms, cudaStream_t st) {
-  using L = SmemLayout<BN, STAGES, false>;
-  auto kern = gemm_bf16x3_mc_kernel<BN, STAGES, AMODE, MC>;
-  static PerDeviceOnce once;
-  {
-    cudaError_t e = once([&] {
-      cudaError_t e1 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL);
-      if (e1 != cudaSuccess) return e1;
-      return cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 0);
-    });
-    if (e != cudaSuccess) return e;
-  }
-  const int super_tiles = ((N + BN - 1) / BN) * ((M + MC * BM - 1) / (MC * BM));
-  const int max_clusters = num_sms / MC;
-  const int clusters = super_tiles < max_clusters ? super_tiles : max_clusters;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(clusters * MC), 1, 1);
-  cfg.blockDim = dim3(kThreads, 1, 1);
-  cfg.dynamicSmemBytes = L::TOTAL;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = MC;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  int K = w.K;
-  return cudaLaunchKernelEx(&cfg, kern, a, w.tm_hi[box_idx], w.tm_lo[box_idx], M, N, K, epi);
-}
-
-// 1 (default): plain GEMMs that are less than one wave of 256-wide tiles pick their tile width by pick_bn's cost rule.
-inline int& small_tiles() { static int v = 1; return v; }
-
-// Multicast cluster size for launches with enough M tiles (0 / 1 = off, 2, 4): process-wide, set through comic_set_option.
-// Off by default: measured at the benchmarked shapes (profiles/r08c_bench512_mc*.json) clusters of 2 change nothing
-// (conv 7.07 vs 7.10 ms, gate GEMM 37.2 vs 36.8 us) and clusters of 4 lose 40 % on the encoder -- the CTAs of a cluster
-// advance in lock-step through the shared `empty` barriers, which costs what the halved weight traffic saves.
-inline int& mc_mode() { static int v = 0; return v; }
-
-// 0: single-CTA kernels only; 1: CTA-pair (cta_group::2) kernel for launches with at least
-// `pair_min_tiles` 256-row pair tiles (process-wide switch, set through comic_set_option).
-inline int& pair_mode() { static int v = 0; return v; }
-inline int& pair_min_tiles() { static int v = 74; return v; }
 
 // Tensor maps of a bf16 (hi, lo) A operand [rows, K] (row stride K elements; K % 8 == 0), box = one 128 x 64 A tile.
 inline bool make_a_maps(ATma& a, const uint16_t* hi, const uint16_t* lo, int rows, int K) {
@@ -1148,19 +783,7 @@ inline bool make_a_maps(ATma& a, const uint16_t* hi, const uint16_t* lo, int row
 template <int AMODE>
 inline cudaError_t launch_gemm_tc(const typename AParam<AMODE>::type& a, const TcWeight& w, int M, int N,
                                   const Epi& epi, int num_sms, cudaStream_t st) {
-  if constexpr (AMODE != 2 && AMODE != 4) {
-    if (pair_mode() && N > 64) {
-      bool planes = false;
-      for (int r = 0; r < epi.nroute; ++r) planes = planes || epi.r[r].hi != nullptr;
-      const int mp = (M + 2 * BM - 1) / (2 * BM);
-      const int bnp = (N <= 128) ? 128 : 256;
-      if (!planes && mp * ((N + bnp - 1) / bnp) >= pair_min_tiles()) {
-        if (bnp == 128) return launch_pair<128, 4, AMODE>(a, w, 0, M, N, epi, num_sms, st);
-        return launch_pair<256, 3, AMODE>(a, w, 1, M, N, epi, num_sms, st);
-      }
-    }
-  }
-  int bn = pick_bn(M, N, num_sms, (AMODE == 0 || AMODE == 4) && small_tiles());
+  int bn = pick_bn(M, N, num_sms, AMODE == 0 || AMODE == 4);
   if constexpr (AMODE == 0) {
     if (epi.ksplit > 1) return launch_one<128, 3, 0>(a, w, 1, M, N, epi, num_sms, st);    // tc_ksplit() assumed 128-wide tiles
   }
@@ -1170,28 +793,17 @@ inline cudaError_t launch_gemm_tc(const typename AParam<AMODE>::type& a, const T
   if constexpr (AMODE == 1) {
     // convolutions a little wider than one 256-column tile (Mixed_4e / 4f 3x3: N = 288 / 320): two tiles of 176 + rest
     // instead of 256 + a 32..64-column tile that pays a full pass over the im2col operand for a sliver of MMA work
-    if (small_tiles() && N > 256 && N <= 352 && w.K >= 512) return launch_one<176, 2, 1>(a, w, 3, M, N, epi, num_sms, st);
+    if (N > 256 && N <= 352 && w.K >= 512) return launch_one<176, 2, 1>(a, w, 3, M, N, epi, num_sms, st);
     // 3x3 convolutions with exactly 192 outputs and one 64-channel block per tap (Conv2d_2c): a 192-column tile leaves
     // 40 KB less shared memory allocated, the L1 carve-out grows from 28 to 60 KB and the horizontally neighbouring taps of
     // consecutive K blocks (same pixels shifted by one, 32 KB apart) hit L1 instead of L2
-    if (small_tiles() && N == 192 && a.KH == 3 && a.Cin == 64) return launch_one<192, 2, 1>(a, w, 4, M, N, epi, num_sms, st);
-  }
-  if constexpr (AMODE != 0 && AMODE != 4) {
+    if (N == 192 && a.KH == 3 && a.Cin == 64) return launch_one<192, 2, 1>(a, w, 4, M, N, epi, num_sms, st);
     // narrow convs (N <= 64): the whole weight panel fits beside the A ring -> load it once per CTA
-    if (bn == 64 && bres_mode() && (M + BM - 1) / BM >= 2 * num_sms) {
+    if (bn == 64 && (M + BM - 1) / BM >= 2 * num_sms) {
       const int nkb = (w.K + BK - 1) / BK;
-      if (nkb <= 4) return launch_bres<4, 4, AMODE>(a, w, M, N, epi, num_sms, st);
-      if (nkb <= 6) return launch_bres<3, 6, AMODE>(a, w, M, N, epi, num_sms, st);
-      if (nkb <= 8) return launch_bres<2, 8, AMODE>(a, w, M, N, epi, num_sms, st);
-    }
-  }
-  if constexpr (AMODE != 2 && AMODE != 3 && AMODE != 4) {
-    const int mc = mc_mode();
-    const int m_tiles = (M + BM - 1) / BM;
-    if (mc >= 2 && bn >= 128 && m_tiles >= 2 * mc) {
-      if (bn == 128) return launch_mc<128, 3, AMODE, 2>(a, w, 0, M, N, epi, num_sms, st);
-      if (mc >= 4) return launch_mc<256, 2, AMODE, 4>(a, w, 0, M, N, epi, num_sms, st);
-      return launch_mc<256, 2, AMODE, 2>(a, w, 1, M, N, epi, num_sms, st);
+      if (nkb <= 4) return launch_bres<4, 4, 1>(a, w, M, N, epi, num_sms, st);
+      if (nkb <= 6) return launch_bres<3, 6, 1>(a, w, M, N, epi, num_sms, st);
+      if (nkb <= 8) return launch_bres<2, 8, 1>(a, w, M, N, epi, num_sms, st);
     }
   }
   if (bn == 64) return launch_one<64, 4, AMODE>(a, w, 0, M, N, epi, num_sms, st);

@@ -466,7 +466,7 @@ class Engine(object):
         self._check(self.lib.comic_set_precision(self._h, {'f32': 0, 'tf32x3': 1, 'split': 1, 'fast': 2}[mode]))
 
     def set_option(self, name, value):
-        self._check(self.lib.comic_set_option(self._h, {'fused_attn_min_images': 0, 'enc_chunk_stem': 1, 'enc_chunk_28': 2, 'enc_chunk_14': 3, 'persistent_max_rows': 4, 'persistent_trace': 5, 'enc_planes': 6, 'gemm_pair': 7, 'gemm_pair_min_tiles': 8, 'stem_s2d': 9, 'gemm_resident_b': 10, 'tc_min_rows': 11, 'attn2': 12, 'fuse_lstm': 13, 'gemm_mc': 14, 'tma_a': 15, 'gemm_small_tiles': 16, 'pdl': 17, 'persistent_watchdog_ms': 18, 'tc_splitk': 19}[name], int(value)))
+        self._check(self.lib.comic_set_option(self._h, {'fused_attn_min_images': 0, 'enc_chunk_stem': 1, 'enc_chunk_28': 2, 'enc_chunk_14': 3, 'persistent_max_rows': 4, 'persistent_trace': 5, 'stem_s2d': 9, 'tc_min_rows': 11, 'attn2': 12, 'tma_a': 15, 'persistent_watchdog_ms': 18, 'tc_splitk': 19}[name], int(value)))
 
     def decode_trace(self, max_steps=256):
         """Per-phase clock stamps of the last persistent decode call: int64 array [steps, 2, 16]."""

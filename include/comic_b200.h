@@ -140,7 +140,7 @@ int comic_bind_gru_candidate(comic_handle_t h, const float* kernel, const float*
  * Small-row GEMMs (M < 128, e.g. batch-8 decode) always use the FFMA kernel. */
 int comic_set_precision(comic_handle_t h, int mode);
 
-/* Engine tunables (no reference counterpart). */
+/* Engine tunables (no reference counterpart).  Ids 6-8, 10, 13, 14, 16 and 17 are retired and refused. */
 #define COMIC_OPT_FUSED_ATTN_MIN_IMAGES 0   /* one-CTA-per-image fused attention from this batch on (default 48) */
 #define COMIC_OPT_ENC_CHUNK_STEM 1          /* images per encoder chunk, stem convs (default 256) */
 #define COMIC_OPT_ENC_CHUNK_28 2            /* ... Mixed_3b/3c (default 512) */
@@ -148,47 +148,23 @@ int comic_set_precision(comic_handle_t h, int mode);
 #define COMIC_OPT_PERSISTENT_MAX_ROWS 4      /* decode loops with batch*beam <= this run as ONE cooperative kernel
                                              * (default 32, the kernel's limit; 0 = always one launch per step op) */
 #define COMIC_OPT_PERSISTENT_TRACE 5         /* 1: the persistent loop records per-phase clock stamps (diagnostics) */
-#define COMIC_OPT_ENC_PLANES 6               /* 1: on the tensor path the encoder keeps its activations as
-                                             * error-compensated bf16 (hi, lo) planes written by each conv's epilogue
-                                             * (cp.async operand loader, no conversion in the consumer);
-                                             * 0 (default): fp32 NHWC activations, split by every consumer.  Measured
-                                             * r01f: the GEMM is L2->SM-bandwidth bound either way, planes 12% slower */
-#define COMIC_OPT_GEMM_PAIR 7                /* 1: tensor-path GEMMs / convs on CTA pairs (tcgen05 cta_group::2, 256-row
-                                             * tiles, each CTA loads half of the weight tile); process-wide */
-#define COMIC_OPT_GEMM_PAIR_MIN_TILES 8      /* ... for launches with at least this many 256-row tiles (default 74) */
 #define COMIC_OPT_STEM_S2D 9                 /* tensor-path stem conv: 2 (default) = 4x4 stride-1 conv over the space-to-depth
                                              * image stored as bf16 planes, each 8x16-pixel tile's im2col rows built from a
                                              * shared-memory halo patch (one L2 read per input element per tile instead of
-                                             * 16); 1 = same conv, rows gathered from L2; 0 = 7x7/2 gather from NHWC4 fp32 */
-#define COMIC_OPT_GEMM_RESIDENT_B 10         /* 1 (default): convs with <= 64 output channels and K <= 512 keep their whole
-                                             * weight panel in shared memory (loaded once per CTA); 0: stream it per M tile */
+                                             * 16); 0 = 7x7/2 gather from NHWC4 fp32; other values are refused */
 #define COMIC_OPT_ATTN2 12                   /* 1 (default): large-batch decode steps use the streaming attention kernel
                                                 (TMA-staged key slices, one HBM pass per step) where it applies: tied
                                                 values, add_LN, softmax, rnn_size 512, 8 heads, beam <= 3; 0: never */
-#define COMIC_OPT_FUSE_LSTM 13               /* 1: on the tensor path the LSTM point-wise update runs in the gate GEMM's epilogue
-                                                (gate-interleaved weight panel; bit-identical results); 0 (default): separate
-                                                kernel -- measured faster at the benchmarked shape, see comic_internal.cuh */
 #define COMIC_OPT_TMA_A 15                   /* bit 0: [logits | query] GEMM, bit 1: gate GEMM -- on the tensor path the GEMM reads its A
                                                operand as bf16 (hi, lo) planes through TMA (h' planes are written by the LSTM kernel;
                                                x = [emb ; ctx ; h] is gathered and split once per step by a small kernel) instead of
                                                gathering and splitting fp32 rows in every N tile's loader warps.  Default 1. */
-#define COMIC_OPT_GEMM_SMALL_TILES 16        /* 1 (default): plain GEMMs smaller than one wave of 256-wide tiles choose the tile width
-                                               (256 / 176 / 128 / 64) that minimises waves x width; 0: round-1 rule */
-#define COMIC_OPT_PDL 17                     /* 1 (default 0: measured 3.5 % slower under graph replay): the kernels of a decode step (gate GEMM, LSTM, [logits | query] GEMM, streaming
-                                               attention, beam step) are launched as programmatic dependents: each runs its
-                                               prologue (barrier / tensor-memory set-up, constants) under the tail of its
-                                               predecessor and waits (griddepcontrol.wait) before it touches global memory */
 #define COMIC_OPT_PERSISTENT_WATCHDOG_MS 18   /* how long a CTA of the persistent decode loop may spin at a grid barrier before the
                                                launch is declared dead (T_out = -1); default 2000, 0 = never (time-sliced GPUs,
                                                debuggers) */
 #define COMIC_OPT_TC_SPLITK 19                /* bit 0: gate GEMM, bit 1: [logits | query] GEMM (default 3): tensor-path decoder GEMMs with at most 128 rows (batch 25 x beam 3 = 75,
                                                the reference's default inference shape) cut their K loop into up to 8 ranges,
                                                one CTA each; the partial sums are added in a fixed order by the consumer */
-#define COMIC_OPT_GEMM_MC 14                 /* tensor-path GEMMs / convs with >= 2 x value M tiles: clusters of `value` CTAs (2 or 4;
-                                               0 = off, default) work on consecutive M tiles of one N tile and multicast the
-                                               weight tile (each loads 1 / value of it): the panel crosses L2 -> SM once per
-                                               cluster.  Bit-identical to the single-CTA kernel; measured no faster (2) /
-                                               slower (4) at the benchmarked shapes, kept as an option. */
 #define COMIC_OPT_TC_MIN_ROWS 11             /* GEMMs / convs with at least this many rows run on the tensor path when
                                              * precision >= 1 (default 64) */
 int comic_set_option(comic_handle_t h, int option, int value);

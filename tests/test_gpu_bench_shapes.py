@@ -63,7 +63,7 @@ class _phase(object):
 
 
 # ---------------------------------------------------------------------------
-# Launch rules of gemm_tc.cuh, restated (defaults: no CTA pairs, no multicast, small_tiles on, resident panels on)
+# Launch rules of gemm_tc.cuh, restated
 # ---------------------------------------------------------------------------
 def _cdiv(a, b):
     return -(-a // b)

@@ -232,53 +232,6 @@ def test_run_stream_raw_pixels_and_optional_attention_maps(torch_mod):
     np.testing.assert_array_equal(p, refs[0][0])
 
 
-def test_lstm_epilogue_fusion_is_bit_identical(torch_mod):
-    """The LSTM point-wise update inside the gate GEMM's epilogue (gate-interleaved weight panel) against the separate
-    point-wise kernel: the same fp32 operations in the same order, so every output of a decode must be identical."""
-    c = comic_config()
-    W = make_weights(c, include_cnn=False)
-    im, fm = fake_features(50, seed=19)
-    outs = []
-    for fuse in (1, 0):
-        eng = _engine(c, W)
-        eng.set_option('tma_a', 0)                     # (its once-per-step operand kernel would change the launch count)
-        eng.set_option('fuse_lstm', fuse)
-        eng.set_option('tc_splitk', 0)                 # (150 rows would take the K-split gate GEMM, which has no LSTM epilogue)
-        keys, values = eng.project_fm(eng.to_dev(fm))
-        c0, h0 = eng.rnn_init(eng.to_dev(im))
-        n0 = eng.launch_count()
-        outs.append(eng.decode_beam(keys, values, c0, h0, 3, 0.0, 10))
-        outs[-1]['launches'] = eng.launch_count() - n0
-    a, b = outs
-    assert a['launches'] == b['launches'] - 10            # one launch per step less
-    for key in ('step_ids', 'parent_ids', 'predicted_ids', 'lengths', 'scores', 'attn'):
-        assert torch_mod.equal(a[key], b[key]), key
-
-
-def test_weight_multicast_gemm_is_bit_identical(torch_mod):
-    """Clusters of 2 / 4 CTAs that multicast the weight tile (option gemm_mc) run the same UMMAs per accumulator element
-    in the same order as the single-CTA kernel: encoder output and a whole beam decode must be identical, including the
-    shapes whose last cluster is only partly inside M (70 images: 428.75 tiles of 128 rows at 28 x 28)."""
-    from _common import images
-    c = comic_config()
-    W = make_weights(c)
-    img = images(70, seed=23)
-    outs = []
-    for mc in (0, 2, 4):
-        eng = _engine(c, W, with_cnn=True)
-        eng.set_option('gemm_mc', mc)
-        emb, fm = eng.encode(eng.to_dev(img))
-        keys, values = eng.project_fm(fm)
-        c0, h0 = eng.rnn_init(emb)
-        dec = eng.decode_beam(keys, values, c0, h0, 3, 0.0, 8)
-        outs.append((emb, fm, keys, dec))
-    eng.set_option('gemm_mc', 0)                     # process-wide switch: back to the default
-    for emb, fm, keys, dec in outs[1:]:
-        assert torch_mod.equal(fm, outs[0][1]) and torch_mod.equal(emb, outs[0][0]) and torch_mod.equal(keys, outs[0][2])
-        for key in ('step_ids', 'parent_ids', 'predicted_ids', 'lengths', 'scores', 'attn'):
-            assert torch_mod.equal(dec[key], outs[0][3][key]), key
-
-
 def test_tma_staged_a_operand_is_bit_identical(torch_mod):
     """Decoder GEMMs with their A operand staged by TMA from bf16 (hi, lo) planes (option tma_a: x gathered and split once
     per step, h' planes written by the LSTM kernel) against the loader-warp path: the same bf16 operand pairs reach the same
@@ -299,21 +252,3 @@ def test_tma_staged_a_operand_is_bit_identical(torch_mod):
         for key in ('step_ids', 'parent_ids', 'predicted_ids', 'lengths', 'scores', 'attn'):
             assert torch_mod.equal(a[key], b[key]), (B, key)
 
-
-def test_programmatic_dependent_launch_is_bit_identical(torch_mod):
-    """Option pdl: the decode-step kernels launched as programmatic dependents (prologue under the predecessor's tail,
-    griddepcontrol.wait before the first global access) must produce the same decode as ordinary stream launches."""
-    c = comic_config()
-    W = make_weights(c, include_cnn=False)
-    im, fm = fake_features(50, seed=31)
-    outs = []
-    for on in (1, 0):
-        eng = _engine(c, W)
-        eng.set_option('pdl', on)
-        keys, values = eng.project_fm(eng.to_dev(fm))
-        c0, h0 = eng.rnn_init(eng.to_dev(im))
-        outs.append(eng.decode_beam(keys, values, c0, h0, 3, 0.0, 10))
-    eng.set_option('pdl', 0)                         # process-wide switch: back to the default
-    a, b = outs
-    for key in ('step_ids', 'parent_ids', 'predicted_ids', 'lengths', 'scores', 'attn'):
-        assert torch_mod.equal(a[key], b[key]), key
