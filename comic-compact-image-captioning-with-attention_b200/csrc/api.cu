@@ -203,6 +203,21 @@ extern "C" int comic_set_rnn_cell(comic_handle_t h, int cell) {
   return COMIC_OK;
 }
 
+extern "C" int comic_set_fm_endpoint(comic_handle_t h, int endpoint) {
+  COMIC_REQUIRE(h, COMIC_E_BADARG, "set_fm_endpoint: null handle");
+  COMIC_REQUIRE(endpoint >= 0 && endpoint < kNumFmTaps, COMIC_E_UNSUPPORTED,
+                "set_fm_endpoint: end point %d is not built (0..8: MaxPool_4a_3x3, Mixed_4b..4f, MaxPool_5a_2x2, Mixed_5b, "
+                "Mixed_5c)", endpoint);
+  COMIC_REQUIRE(!h->bound && !h->sized, COMIC_E_BADARG,
+                "set_fm_endpoint: call it before any size query or binding (workspace layouts depend on the end point)");
+  const int C = kFmTapC[endpoint], S = kFmTapS[endpoint];
+  COMIC_REQUIRE(h->C == C && h->M == S * S, COMIC_E_SHAPE,
+                "set_fm_endpoint: end point %d is [%d x %d, %d] but the config has fm_positions %d, fm_channels %d", endpoint,
+                S, S, C, h->M, h->C);
+  h->fm_tap = endpoint;
+  return COMIC_OK;
+}
+
 extern "C" int comic_bind_gru_candidate(comic_handle_t h, const float* kernel, const float* bias) {
   COMIC_REQUIRE(h && kernel && bias, COMIC_E_BADARG, "bind_gru_candidate: null argument");
   COMIC_REQUIRE(h->cell == COMIC_CELL_GRU, COMIC_E_BADARG, "bind_gru_candidate: the handle's cell is not GRU");

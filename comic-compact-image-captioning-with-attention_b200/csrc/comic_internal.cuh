@@ -73,6 +73,7 @@ struct comic_handle_s {
   int R, W, H, C, M, E, V, Vp, A, VAL, LQ, KX;
   comic_weights_t w;
   int cell = COMIC_CELL_LSTM;              // comic_set_rnn_cell
+  int fm_tap = COMIC_FM_MIXED_4F;          // comic_set_fm_endpoint
   const float* gru_cand_kernel = nullptr;  // GRU candidate/{kernel [W+A+R, R], bias [R]} (comic_bind_gru_candidate);
   const float* gru_cand_bias = nullptr;    // gates/{kernel, bias} travel in w.lstm_kernel / w.lstm_bias
   bool bound = false, cnn_bound = false;
@@ -173,6 +174,19 @@ inline int tc_ksplit(comic_handle_t h, int M, int N, int K, int which) {   // wh
 // profiles/r12e_*); 32 rows and fewer belong to the persistent loop / the FFMA kernel.
 inline bool use_tc_step(comic_handle_t h, const tc::TcWeight& w, int M, int N, int K, int which) {
   return use_tc(h, w, M) || (h->precision >= 1 && w.ready && M > 32 && tc_ksplit(h, M, N, K, which) > 1);
+}
+
+// Attention end points (COMIC_FM_*, in network order): channels and side of each.
+constexpr int kNumFmTaps = 9;
+constexpr int kFmTapC[kNumFmTaps] = {480, 512, 512, 512, 528, 832, 832, 832, 1024};
+constexpr int kFmTapS[kNumFmTaps] = {14, 14, 14, 14, 14, 14, 7, 7, 7};
+// Encoder blocks (block_table() order) whose output is an end point: Mixed_4b..4f = blocks 2..6, Mixed_5b / 5c = 7 / 8.
+inline int fm_tap_block(int tap) {
+  return (tap >= COMIC_FM_MIXED_4B && tap <= COMIC_FM_MIXED_4F) ? tap + 1 : (tap >= COMIC_FM_MIXED_5B ? tap : -1);
+}
+// The config's feature map (C, M) is the selected end point's.
+inline bool fm_tap_matches(comic_handle_t h) {
+  return h->C == kFmTapC[h->fm_tap] && h->M == kFmTapS[h->fm_tap] * kFmTapS[h->fm_tap];
 }
 
 // encoder.cu

@@ -982,7 +982,9 @@ static int dispatch_fused(comic_handle_t h, const StepIO& io, const StepBufs& sb
     COMIC_CHECK_CUDA(a2::launch(aa, k, h->num_sms, h->dev, st));
     return 1;
   }
-  if (B < h->fused_min_images || h->VAL > 1024 || h->VAL % 4 != 0) return 0;
+  // the context phase gives each thread 4 channels of ONE head: a head width that is not a multiple of 4 (Mixed_4e's 528
+  // channels over 8 heads) takes the sliced kernels
+  if (B < h->fused_min_images || h->VAL > 1024 || h->VAL % 4 != 0 || (h->VAL / h->H) % 4 != 0) return 0;
   size_t smem = attn_fused_smem(k, h->R, h->H, h->M, h->VAL);
   if (smem > 200 * 1024) return 0;
   AttnArgs aa{};

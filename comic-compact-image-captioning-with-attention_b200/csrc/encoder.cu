@@ -375,7 +375,8 @@ static EncPlan enc_plan(comic_handle_t h, int B) {
   pl.c3 = B < h->enc_chunk[1] ? B : h->enc_chunk[1];
   pl.c4 = B < h->enc_chunk[2] ? B : h->enc_chunk[2];
   auto mx = [](size_t x, size_t y) { return x > y ? x : y; };
-  // ping/pong: stem conv1 112x112x64 / conv2c 56x56x192; stage 3 28x28x480; stage 4 14x14x528 (832 goes to fm_out)
+  // ping/pong: stem conv1 112x112x64 / conv2c 56x56x192; stage 3 28x28x480; stage 4 14x14x832 (Mixed_4f when it is not
+  // the end point; the end point goes to fm_out)
   pl.ab = mx(mx((size_t)pl.cs * 112 * 112 * 64, (size_t)pl.c3 * 28 * 28 * 480), (size_t)pl.c4 * 14 * 14 * 832);
   pl.t1 = mx((size_t)pl.c3 * 28 * 28 * 128, (size_t)pl.c4 * 14 * 14 * 192);
   pl.t2 = mx((size_t)pl.c3 * 28 * 28 * 32, (size_t)pl.c4 * 14 * 14 * 48);
@@ -528,7 +529,9 @@ static int run_stem_s2d(comic_handle_t h, const float* img, int nb, float* scrat
 int encoder_forward(comic_handle_t h, const float* images, int B, float* fm_out, float* im_embed_out,
                     float* mixed5c_out, void* ws, size_t ws_bytes, cudaStream_t st) {
   COMIC_REQUIRE(h->cnn_bound, COMIC_E_BADARG, "encode_fwd: CNN weights not bound");
-  COMIC_REQUIRE(h->C == 832, COMIC_E_UNSUPPORTED, "encode_fwd: only cnn_fm_attention=Mixed_4f (C=832) is built");
+  COMIC_REQUIRE(fm_tap_matches(h), COMIC_E_UNSUPPORTED,
+                "encode_fwd: feature map [%d, %d] is not end point %d's (comic_set_fm_endpoint)", h->M, h->C, h->fm_tap);
+  const int tap = h->fm_tap;
   size_t need;
   encoder_workspace_bytes(h, B, &need);
   COMIC_REQUIRE(ws_bytes >= need, COMIC_E_WORKSPACE, "encode_fwd: workspace %zu < %zu", ws_bytes, need);
@@ -540,6 +543,7 @@ int encoder_forward(comic_handle_t h, const float* images, int B, float* fm_out,
   float* pool2 = cv.take<float>(pl.p2);
   float* pool3 = cv.take<float>(pl.p3);
   float* head = cv.take<float>(pl.head);
+  if (tap == COMIC_FM_MAXPOOL_4A_3X3) pool3 = fm_out;   // [B,14,14,480] is the feature map itself
   int rc;
   // ---- stem (inception_v1.py:70-93) -> pool2 [B,28,28,192]
   for (int b0 = 0; b0 < B; b0 += pl.cs) {
@@ -575,17 +579,31 @@ int encoder_forward(comic_handle_t h, const float* images, int B, float* fm_out,
   // ---- Mixed_4b..4f @14, Mixed_5b, 5c @7, head
   for (int b0 = 0; b0 < B; b0 += pl.c4) {
     int nb = (B - b0 < pl.c4) ? (B - b0) : pl.c4;
-    if ((rc = run_block(h, 2, pool3 + (size_t)b0 * 14 * 14 * 480, eb.a, nb, 14, eb, st))) return rc;   // 512
-    if ((rc = run_block(h, 3, eb.a, eb.b, nb, 14, eb, st))) return rc;   // 512
-    if ((rc = run_block(h, 4, eb.b, eb.a, nb, 14, eb, st))) return rc;   // 512
-    if ((rc = run_block(h, 5, eb.a, eb.b, nb, 14, eb, st))) return rc;   // 528
-    // Mixed_4f -> the attention feature map, written straight to fm_out [B,196,832]
-    float* fm = fm_out + (size_t)b0 * 196 * 832;
-    if ((rc = run_block(h, 6, eb.b, fm, nb, 14, eb, st))) return rc;
-    if ((rc = run_maxpool(h, fm, eb.a, nb, 14, 14, 832, 2, 2, nullptr, nullptr, st))) return rc;    // 7x7x832
-    if ((rc = run_block(h, 7, eb.a, eb.b, nb, 7, eb, st))) return rc;    // 832
-    float* m5c = mixed5c_out ? mixed5c_out + (size_t)b0 * 49 * 1024 : eb.a;
-    if ((rc = run_block(h, 8, eb.b, m5c, nb, 7, eb, st))) return rc;     // 1024
+    // The end point is written straight to fm_out [B,M,C] and the next layer reads it there; every other output goes to
+    // whichever of the ping / pong buffers the layer does not read (at Mixed_4f: 4b..4e alternate a, b; 5a_2x2 -> a; 5b -> b)
+    float* fm = fm_out + (size_t)b0 * h->M * h->C;
+    const float* cur = pool3 + (size_t)b0 * 14 * 14 * 480;
+    auto dst = [&](int t) { return t == tap ? fm : (cur == eb.a ? eb.b : eb.a); };
+    for (int t = COMIC_FM_MIXED_4B; t <= COMIC_FM_MIXED_4F; ++t) {       // 512, 512, 512, 528, 832
+      float* y = dst(t);
+      if ((rc = run_block(h, fm_tap_block(t), cur, y, nb, 14, eb, st))) return rc;
+      cur = y;
+    }
+    {
+      float* y = dst(COMIC_FM_MAXPOOL_5A_2X2);
+      if ((rc = run_maxpool(h, cur, y, nb, 14, 14, 832, 2, 2, nullptr, nullptr, st))) return rc;    // 7x7x832
+      cur = y;
+    }
+    {
+      float* y = dst(COMIC_FM_MIXED_5B);
+      if ((rc = run_block(h, 7, cur, y, nb, 7, eb, st))) return rc;      // 832
+      cur = y;
+    }
+    float* m5c = tap == COMIC_FM_MIXED_5C ? fm : mixed5c_out ? mixed5c_out + (size_t)b0 * 49 * 1024 : dst(-1);
+    if ((rc = run_block(h, 8, cur, m5c, nb, 7, eb, st))) return rc;      // 1024
+    if (tap == COMIC_FM_MIXED_5C && mixed5c_out && mixed5c_out != fm_out)
+      COMIC_CHECK_CUDA(cudaMemcpyAsync(mixed5c_out + (size_t)b0 * 49 * 1024, fm, (size_t)nb * 49 * 1024 * sizeof(float),
+                                       cudaMemcpyDeviceToDevice, st));
     float* emb = im_embed_out + (size_t)b0 * 1024;
     if (!h->cfg.legacy) {
       Prof pf(h, T_POOL, st);

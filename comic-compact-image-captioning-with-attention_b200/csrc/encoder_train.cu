@@ -55,6 +55,13 @@ static const float* blk_input(const EncTape& tp, int i) {
   return tp.y[i - 1];
 }
 
+// The tape tensor that is attention end point `tap` (COMIC_FM_*).
+static const float* fm_tap_tensor(const EncTape& tp, int tap) {
+  if (tap == COMIC_FM_MAXPOOL_4A_3X3) return tp.p3;
+  if (tap == COMIC_FM_MAXPOOL_5A_2X2) return tp.p4;
+  return tp.y[fm_tap_block(tap)];
+}
+
 // ---------------------------------------------------------------------------
 // Backward kernels.
 // ---------------------------------------------------------------------------
@@ -277,13 +284,13 @@ __global__ void wgrad_reduce_kernel(const float* __restrict__ part, int nz, size
   out[i] = s;
 }
 
-// dx[b,h,w,c] = (add ? add[b,h,w,c] : 0) + sum over the pooling windows that contain (h,w) of
+// dx[b,h,w,c] = (add ? add[b,h,w,c] : 0) (+ add2[b,h,w,c]) + sum over the pooling windows that contain (h,w) of
 // dy[window] * [x[b,h,w,c] is the FIRST maximum of that window in row-major scan order].
 template <int K>
 __global__ void __launch_bounds__(256)
 maxpool_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, const float* add,
                    float* dx, unsigned total, int H, int W, int C4, int stride, int pad_t,
-                   int pad_l, int Ho, int Wo) {
+                   int pad_l, int Ho, int Wo, const float* __restrict__ add2) {
   unsigned i = blockIdx.x * 256u + threadIdx.x;
   if (i >= total) return;
   unsigned c4 = i % (unsigned)C4, p = i / (unsigned)C4;
@@ -295,6 +302,10 @@ maxpool_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, co
   const float4* dyb = reinterpret_cast<const float4*>(dy) + (size_t)b * Ho * Wo * C4 + c4;
   const float4 xs = __ldg(xb + ((size_t)hh * W + w) * C4);
   float4 g = add ? reinterpret_cast<const float4*>(add)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+  if (add2) {
+    const float4 a2 = __ldg(reinterpret_cast<const float4*>(add2) + i);
+    g.x += a2.x; g.y += a2.y; g.z += a2.z; g.w += a2.w;
+  }
   // windows ho with ho*stride - pad_t <= hh <= ho*stride - pad_t + K - 1
   int ho_lo = hh + pad_t - (K - 1);
   ho_lo = ho_lo <= 0 ? 0 : (ho_lo + stride - 1) / stride;
@@ -334,13 +345,17 @@ maxpool_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, co
   reinterpret_cast<float4*>(dx)[i] = g;
 }
 
-// 7x7 VALID average pool backward: dx[b, p, c] = dy[b, c] / HW
-__global__ void avgpool_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int B, int HW, int C) {
+// 7x7 VALID average pool backward: dx[b, p, c] = dy[b, c] / HW (+ add[b, p, c]: the attention feature map's gradient when
+// Mixed_5c is the end point)
+__global__ void avgpool_bwd_kernel(const float* __restrict__ dy, float* __restrict__ dx, int B, int HW, int C,
+                                   const float* __restrict__ add) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)B * HW * C) return;
   int c = (int)(i % C);
   int b = (int)(i / ((size_t)HW * C));
-  dx[i] = dy[(size_t)b * C + c] / (float)HW;
+  float v = dy[(size_t)b * C + c] / (float)HW;
+  if (add) v += add[i];
+  dx[i] = v;
 }
 
 // ---------------------------------------------------------------------------
@@ -462,7 +477,7 @@ static void flip_transpose(comic_handle_t h, const float* W, float* Wf, int k, i
 }
 
 static int maxpool_bwd(comic_handle_t h, const float* x, const float* dy, const float* add, float* dx, int B, int H,
-                       int W, int C, int k, int s, cudaStream_t st) {
+                       int W, int C, int k, int s, cudaStream_t st, const float* add2 = nullptr) {
   int Ho, Wo, pt, pl;
   same_pads(H, k, s, &Ho, &pt);
   same_pads(W, k, s, &Wo, &pl);
@@ -470,16 +485,18 @@ static int maxpool_bwd(comic_handle_t h, const float* x, const float* dy, const 
   COMIC_REQUIRE(total < 0xffffffffull && C % 4 == 0 && (k == 2 || k == 3), COMIC_E_UNSUPPORTED,
                 "maxpool_bwd: unsupported shape (total %zu, C %d, k %d)", total, C, k);
   unsigned grid = (unsigned)((total + 255) / 256);
-  if (k == 3) maxpool_bwd_kernel<3><<<grid, 256, 0, st>>>(x, dy, add, dx, (unsigned)total, H, W, C / 4, s, pt, pl, Ho, Wo);
-  else maxpool_bwd_kernel<2><<<grid, 256, 0, st>>>(x, dy, add, dx, (unsigned)total, H, W, C / 4, s, pt, pl, Ho, Wo);
+  if (k == 3)
+    maxpool_bwd_kernel<3><<<grid, 256, 0, st>>>(x, dy, add, dx, (unsigned)total, H, W, C / 4, s, pt, pl, Ho, Wo, add2);
+  else maxpool_bwd_kernel<2><<<grid, 256, 0, st>>>(x, dy, add, dx, (unsigned)total, H, W, C / 4, s, pt, pl, Ho, Wo, add2);
   h->launches++;
   COMIC_CHECK_CUDA(cudaGetLastError());
   return COMIC_OK;
 }
 
-// One inception block backward.  dy [M, cout] -> dx [M, cin]; weight / beta gradients into g.
+// One inception block backward.  dy [M, cout] -> dx [M, cin] (+ dx_add [M, cin] when the block input is also the
+// attention feature map); weight / beta gradients into g.
 static int block_bwd(comic_handle_t h, int bi, const EncTape& tp, const float* dy, float* dx, int B,
-                     const comic_cnn_grads_t* g, BwdBufs& bb, cudaStream_t st) {
+                     const comic_cnn_grads_t* g, BwdBufs& bb, cudaStream_t st, const float* dx_add = nullptr) {
   const BlockDesc& bd = block_table()[bi];
   const comic_conv_desc_t* cd = conv_table();
   const int S = kBlkS[bi], M = B * S * S, cout = blk_cout(bd), cin = bd.cin;
@@ -533,10 +550,10 @@ static int block_bwd(comic_handle_t h, int bi, const EncTape& tp, const float* d
     }
     h->launches += 3;
     if (dx) {
-      // dx = dzg . Wg^T, then += maxpool backward of Branch_3's input gradient
+      // dx = dzg . Wg^T, then += dx_add and the maxpool backward of Branch_3's input gradient
       flip_transpose(h, h->pk.grp_w[bi], bb.wflip, 1, cin, ng, st);
       if ((rc = dgrad_conv(h, bb.dzg, B, S, ng, 1, bb.wflip, cin, dx, cin, bb, st))) return rc;
-      if ((rc = maxpool_bwd(h, x, bb.dp, dx, dx, B, S, S, cin, 3, 1, st))) return rc;
+      if ((rc = maxpool_bwd(h, x, bb.dp, dx, dx, B, S, S, cin, 3, 1, st, dx_add))) return rc;
     }
   }
   COMIC_CHECK_CUDA(cudaGetLastError());
@@ -569,8 +586,9 @@ extern "C" int comic_encode_train_fwd(comic_handle_t h, const float* images, int
                                       void* tape, size_t tape_bytes, void* ws, size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && images && fm_out && im_embed_out && tape && ws && B > 0, COMIC_E_BADARG, "encode_train_fwd: bad argument");
   COMIC_REQUIRE(h->cnn_bound, COMIC_E_BADARG, "encode_train_fwd: CNN weights not bound");
-  COMIC_REQUIRE(h->C == 832 && !h->cfg.legacy, COMIC_E_UNSUPPORTED,
-                "encode_train_fwd: only cnn_fm_attention=Mixed_4f without the legacy head is built");
+  COMIC_REQUIRE(!h->cfg.legacy, COMIC_E_UNSUPPORTED, "encode_train_fwd: the legacy head is not built for cnn_finetune");
+  COMIC_REQUIRE(fm_tap_matches(h), COMIC_E_UNSUPPORTED,
+                "encode_train_fwd: feature map [%d, %d] is not end point %d's (comic_set_fm_endpoint)", h->M, h->C, h->fm_tap);
   size_t tb, wb;
   comic_encode_train_bytes(h, B, &tb, &wb);
   COMIC_REQUIRE(tape_bytes >= tb && ws_bytes >= wb, COMIC_E_WORKSPACE, "encode_train_fwd: tape %zu < %zu or workspace %zu < %zu",
@@ -599,7 +617,8 @@ extern "C" int comic_encode_train_fwd(comic_handle_t h, const float* images, int
     if (i == 1 && (rc = run_maxpool(h, tp.y[1], tp.p3, B, 28, 28, 480, 3, 2, nullptr, nullptr, st))) return rc;
     if (i == 6 && (rc = run_maxpool(h, tp.y[6], tp.p4, B, 14, 14, 832, 2, 2, nullptr, nullptr, st))) return rc;
   }
-  COMIC_CHECK_CUDA(cudaMemcpyAsync(fm_out, tp.y[6], (size_t)B * 196 * 832 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  COMIC_CHECK_CUDA(cudaMemcpyAsync(fm_out, fm_tap_tensor(tp, h->fm_tap), (size_t)B * h->M * h->C * sizeof(float),
+                                   cudaMemcpyDeviceToDevice, st));
   run_avgpool_global(h, tp.y[8], im_embed_out, B, 49, 1024, st);
   COMIC_CHECK_CUDA(cudaGetLastError());
   return COMIC_OK;
@@ -610,6 +629,8 @@ extern "C" int comic_encode_bwd(comic_handle_t h, const float* images, int B, co
                                 size_t ws_bytes, void* stream) {
   COMIC_REQUIRE(h && images && dfm && dim_embed && tape && grads && ws && B > 0, COMIC_E_BADARG, "encode_bwd: bad argument");
   COMIC_REQUIRE(h->cnn_bound, COMIC_E_BADARG, "encode_bwd: CNN weights not bound");
+  COMIC_REQUIRE(fm_tap_matches(h), COMIC_E_UNSUPPORTED,
+                "encode_bwd: feature map [%d, %d] is not end point %d's (comic_set_fm_endpoint)", h->M, h->C, h->fm_tap);
   for (int i = 0; i < COMIC_NUM_CONVS; ++i)
     COMIC_REQUIRE(grads->conv_w[i] && grads->bn_beta[i], COMIC_E_BADARG, "encode_bwd: missing gradient buffer %d", i);
   size_t tb, wb;
@@ -630,21 +651,25 @@ extern "C" int comic_encode_bwd(comic_handle_t h, const float* images, int B, co
   const comic_conv_desc_t* cd = conv_table();
   int rc;
   float *ga = bb.ga, *gb = bb.gb;
+  // The end point feeds the next layer AND the attention: dfm is an addend of the kernel that finishes the gradient at
+  // the end point (the average pool's backward at Mixed_5c, the 2x2 pool's at Mixed_4f, otherwise the last kernel of the
+  // backward of the block the end point feeds).
+  const int tap = h->fm_tap;
+  auto at = [&](int t) { return t == tap ? dfm : nullptr; };
   // head: im_embed = mean over the 7x7 positions of Mixed_5c (inception_v1.py:326)
   {
     size_t n = (size_t)B * 49 * 1024;
-    avgpool_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dim_embed, ga, B, 49, 1024);
+    avgpool_bwd_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dim_embed, ga, B, 49, 1024, at(COMIC_FM_MIXED_5C));
     h->launches++;
   }
-  if ((rc = block_bwd(h, 8, tp, ga, gb, B, grads, bb, st))) return rc;        // Mixed_5c: d(Mixed_5b out) in gb
-  if ((rc = block_bwd(h, 7, tp, gb, ga, B, grads, bb, st))) return rc;        // Mixed_5b: d(pool4) in ga
-  // Mixed_4f output feeds the 2x2 pool AND the attention feature map
-  if ((rc = maxpool_bwd(h, tp.y[6], ga, dfm, gb, B, 14, 14, 832, 2, 2, st))) return rc;
-  if ((rc = block_bwd(h, 6, tp, gb, ga, B, grads, bb, st))) return rc;
-  if ((rc = block_bwd(h, 5, tp, ga, gb, B, grads, bb, st))) return rc;
-  if ((rc = block_bwd(h, 4, tp, gb, ga, B, grads, bb, st))) return rc;
-  if ((rc = block_bwd(h, 3, tp, ga, gb, B, grads, bb, st))) return rc;
-  if ((rc = block_bwd(h, 2, tp, gb, ga, B, grads, bb, st))) return rc;        // d(pool3) in ga
+  if ((rc = block_bwd(h, 8, tp, ga, gb, B, grads, bb, st, at(COMIC_FM_MIXED_5B)))) return rc;        // d(Mixed_5b out) in gb
+  if ((rc = block_bwd(h, 7, tp, gb, ga, B, grads, bb, st, at(COMIC_FM_MAXPOOL_5A_2X2)))) return rc;  // d(pool4) in ga
+  if ((rc = maxpool_bwd(h, tp.y[6], ga, at(COMIC_FM_MIXED_4F), gb, B, 14, 14, 832, 2, 2, st))) return rc;
+  if ((rc = block_bwd(h, 6, tp, gb, ga, B, grads, bb, st, at(COMIC_FM_MIXED_4E)))) return rc;
+  if ((rc = block_bwd(h, 5, tp, ga, gb, B, grads, bb, st, at(COMIC_FM_MIXED_4D)))) return rc;
+  if ((rc = block_bwd(h, 4, tp, gb, ga, B, grads, bb, st, at(COMIC_FM_MIXED_4C)))) return rc;
+  if ((rc = block_bwd(h, 3, tp, ga, gb, B, grads, bb, st, at(COMIC_FM_MIXED_4B)))) return rc;
+  if ((rc = block_bwd(h, 2, tp, gb, ga, B, grads, bb, st, at(COMIC_FM_MAXPOOL_4A_3X3)))) return rc;  // d(pool3) in ga
   if ((rc = maxpool_bwd(h, tp.y[1], ga, nullptr, gb, B, 28, 28, 480, 3, 2, st))) return rc;
   if ((rc = block_bwd(h, 1, tp, gb, ga, B, grads, bb, st))) return rc;
   if ((rc = block_bwd(h, 0, tp, ga, gb, B, grads, bb, st))) return rc;        // d(pool2) in gb

@@ -1422,7 +1422,7 @@ extern "C" int comic_train_fwd_bwd(comic_handle_t h, const float* fm, const floa
     int bm = B * M, bmp = (bm + 3) / 4 * 4;
     COMIC_CHECK_CUDA(cudaMemsetAsync(tb.fmT, 0, (size_t)C * bmp * sizeof(float), st));
     transpose(fm, bm, C, C, tb.fmT, bmp, st);
-    const int Kd = bm;                  // B * 196 is always a multiple of 4
+    const int Kd = bm;                  // B * 49 with odd B is not a multiple of 4: train_gemm takes its scalar loader
     if ((rc = train_gemm(h, tb.fmT, bmp, tb.dkeys, R, grads->memory_kernel, R, C, R, Kd, tb.part, tb.part_floats, st))) return rc;
     if (h->cfg.fm_projection == 2 && grads->value_kernel)
       if ((rc = train_gemm(h, tb.fmT, bmp, tb.dvals, R, grads->value_kernel, R, C, R, Kd, tb.part, tb.part_floats, st))) return rc;

@@ -83,6 +83,7 @@ SIGNATURES = {
     'comic_packed_bytes': (_I, [_P, C.POINTER(_SZ)]),
     'comic_bind_weights': (_I, [_P, C.POINTER(ComicWeights), _I, _P, _SZ, _P]),
     'comic_set_rnn_cell': (_I, [_P, _I]),
+    'comic_set_fm_endpoint': (_I, [_P, _I]),
     'comic_bind_gru_candidate': (_I, [_P, _P, _P]),
     'comic_workspace_bytes': (_I, [_P, _I, _I, _I, _I, C.POINTER(_SZ)]),
     'comic_encode_fwd': (_I, [_P, _P, _I, _P, _P, _P, _P, _SZ, _P]),
@@ -192,6 +193,7 @@ class Engine(object):
         self._h = C.c_void_p()
         self._check(self.lib.comic_create(C.byref(cfg), C.byref(self._h)))
         self._check(self.lib.comic_set_rnn_cell(self._h, CELL[config.rnn_name]))
+        self._check(self.lib.comic_set_fm_endpoint(self._h, list(wts.FM_ENDPOINTS).index(config.cnn_fm_attention)))
         self._dev_weights = {}
         self._packed = None
         self._ws = {}
@@ -303,7 +305,8 @@ class Engine(object):
 
     # -- E1/E2 ----------------------------------------------------------------
     def encode(self, images, want_mixed5c=False):
-        """images [B,224,224,3] fp32 NHWC on device -> (im_embed [B,1024], fm [B,196,C])."""
+        """images [B,224,224,3] fp32 NHWC on device -> (im_embed [B,1024], fm [B,M,C]) (+ Mixed_5c [B,7,7,1024]; at
+        cnn_fm_attention=Mixed_5c that is a view of fm)."""
         torch = self.torch
         images = images.contiguous()
         if images.dim() != 4 or tuple(images.shape[1:]) != (224, 224, 3):
@@ -311,10 +314,13 @@ class Engine(object):
         B = images.shape[0]
         fm = self.f32(B, self.dims.M, self.dims.C)
         emb = self.f32(B, self.dims.E)
-        m5c = self.f32(B, 7, 7, 1024) if want_mixed5c else None
+        at_5c = self.c.cnn_fm_attention == 'Mixed_5c'
+        m5c = self.f32(B, 7, 7, 1024) if want_mixed5c and not at_5c else None
         ws = self._workspace(0, B, 1, 1)
         self._check(self.lib.comic_encode_fwd(self._h, _ptr(images), B, _ptr(fm), _ptr(emb), _ptr(m5c),
                                               _ptr(ws), ws.numel(), self.stream()))
+        if want_mixed5c and at_5c:
+            m5c = fm.view(B, 7, 7, 1024)
         return (emb, fm, m5c) if want_mixed5c else (emb, fm)
 
     def preprocess_eval(self, images_u8, out_hw=(224, 224)):
@@ -599,7 +605,7 @@ class Engine(object):
 
     # -- cnn_finetune (encoder forward-with-tape + backward) ---------------------
     def encode_train(self, images):
-        """Forward that keeps every activation: -> (im_embed [B,1024], fm [B,196,C]); the tape stays
+        """Forward that keeps every activation: -> (im_embed [B,1024], fm [B,M,C]); the tape stays
         in this engine until `encode_bwd`."""
         torch = self.torch
         images = images.contiguous()

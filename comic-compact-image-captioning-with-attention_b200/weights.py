@@ -77,10 +77,28 @@ def cnn_conv_list():
 
 
 def fm_channels(endpoint):
+    """Channels of an inception block or pool end point (a pool keeps its input's channels)."""
+    c = STEM[-1][5]
     for b in BLOCKS:
-        if b[0] == endpoint and len(b) > 3:
-            return b[2] + b[4] + b[6] + b[7]
+        if len(b) > 3:
+            c = b[2] + b[4] + b[6] + b[7]
+        if b[0] == endpoint:
+            return c
     raise ValueError('Unknown feature-map end point %s' % endpoint)
+
+
+# The end points the decoder can attend over (c.cnn_fm_attention) -> side S of the S x S map, in network order; the
+# index is the library's COMIC_FM_* id.  The 28 x 28 and earlier end points are not built.
+FM_ENDPOINTS = {'MaxPool_4a_3x3': 14, 'Mixed_4b': 14, 'Mixed_4c': 14, 'Mixed_4d': 14, 'Mixed_4e': 14, 'Mixed_4f': 14,
+                'MaxPool_5a_2x2': 7, 'Mixed_5b': 7, 'Mixed_5c': 7}
+
+
+def fm_side(endpoint):
+    """S of the S x S attention map at `endpoint`; NotImplementedError for an end point that is not built."""
+    if endpoint not in FM_ENDPOINTS:
+        raise NotImplementedError('cnn_fm_attention=%s is not built; the supported end points are %s'
+                                  % (endpoint, ', '.join(FM_ENDPOINTS)))
+    return FM_ENDPOINTS[endpoint]
 
 
 # ---------------------------------------------------------------------------
@@ -91,9 +109,9 @@ class Dims(object):
         self.R = int(c.rnn_size)
         self.W = int(c.rnn_word_size)
         self.H = int(c.attn_num_heads)
+        self.M = fm_side(c.cnn_fm_attention) ** 2
         self.C = fm_channels(c.cnn_fm_attention)
         self.E = 1024
-        self.M = 196
         self.fm_projection = c.cnn_fm_projection        # None|'tied'|'independent'
         self.context_layer = bool(c.attn_context_layer)
         if self.fm_projection is None and not self.context_layer:

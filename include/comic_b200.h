@@ -48,8 +48,8 @@ typedef struct {
   int32_t rnn_size;        /* R: c.rnn_size (512) */
   int32_t word_size;       /* W: c.rnn_word_size (256) */
   int32_t num_heads;       /* H: c.attn_num_heads */
-  int32_t fm_channels;     /* C: channels of c.cnn_fm_attention (832 for Mixed_4f) */
-  int32_t fm_positions;    /* M: 196 */
+  int32_t fm_channels;     /* C: channels of c.cnn_fm_attention (832 for Mixed_4f; see comic_set_fm_endpoint) */
+  int32_t fm_positions;    /* M: 196 for a 14x14 end point, 49 for a 7x7 one */
   int32_t embed_size;      /* E: 1024 (im_embed) */
   int32_t vocab;           /* V: softmax size (radix_base+2 | len(itow)) */
   int32_t fm_projection;   /* c.cnn_fm_projection: 0 none, 1 tied, 2 independent */
@@ -130,6 +130,30 @@ int comic_set_rnn_cell(comic_handle_t h, int cell);
  * comic_weights_t.lstm_kernel / lstm_bias carry gates/kernel / gates/bias. */
 int comic_bind_gru_candidate(comic_handle_t h, const float* kernel, const float* bias);
 
+/* InceptionV1 end point the decoder attends over (c.cnn_fm_attention, src/model_base.py:94-104): the tensor
+ * comic_encode_fwd / comic_encode_train_fwd write to fm_out and comic_encode_bwd takes dfm at.  Call after comic_create
+ * and before comic_packed_bytes / comic_workspace_bytes / comic_bind_weights (COMIC_E_BADARG afterwards).  The
+ * config's fm_channels / fm_positions must be the end point's (C, S*S), else COMIC_E_SHAPE; any other id returns
+ * COMIC_E_UNSUPPORTED (the 28x28 and earlier end points are not built).  Default COMIC_FM_MIXED_4F.
+ *   id                       S x S    C
+ *   COMIC_FM_MAXPOOL_4A_3X3  14x14   480
+ *   COMIC_FM_MIXED_4B..4D    14x14   512
+ *   COMIC_FM_MIXED_4E        14x14   528
+ *   COMIC_FM_MIXED_4F        14x14   832
+ *   COMIC_FM_MAXPOOL_5A_2X2   7x7    832
+ *   COMIC_FM_MIXED_5B         7x7    832
+ *   COMIC_FM_MIXED_5C         7x7   1024 */
+#define COMIC_FM_MAXPOOL_4A_3X3 0
+#define COMIC_FM_MIXED_4B       1
+#define COMIC_FM_MIXED_4C       2
+#define COMIC_FM_MIXED_4D       3
+#define COMIC_FM_MIXED_4E       4
+#define COMIC_FM_MIXED_4F       5
+#define COMIC_FM_MAXPOOL_5A_2X2 6
+#define COMIC_FM_MIXED_5B       7
+#define COMIC_FM_MIXED_5C       8
+int comic_set_fm_endpoint(comic_handle_t h, int endpoint);
+
 /* Arithmetic modes (all within the 1e-3 parity bound of the reference's fp32 graph):
  *   0  fp32 FFMA everywhere (the reference's fp32 arithmetic up to summation order);
  *   1  tcgen05 tensor cores with an error-compensated operand split and fp32
@@ -182,7 +206,8 @@ int comic_workspace_bytes(comic_handle_t h, int mode, int B, int k, int T, size_
 
 /* E1+E2: ModelBase._encoder src/model_base.py:56-104 (InceptionV1 forward,
  * common/nets/inception_v1.py:29-339).  images [B,224,224,3] NHWC in [-1,1];
- * fm_out [B,196,C]; im_embed_out [B,1024]; mixed5c_out optional [B,7,7,1024]. */
+ * fm_out [B,M,C] = the end point of comic_set_fm_endpoint; im_embed_out [B,1024]; mixed5c_out optional
+ * [B,7,7,1024] (at COMIC_FM_MIXED_5C it may be fm_out itself: the two are the same tensor). */
 int comic_encode_fwd(comic_handle_t h, const float* images, int B, float* fm_out,
                      float* im_embed_out, float* mixed5c_out, void* ws, size_t ws_bytes,
                      void* stream);
@@ -357,12 +382,12 @@ typedef struct {
  * scratch workspace shared by comic_encode_train_fwd and comic_encode_bwd for B images. */
 int comic_encode_train_bytes(comic_handle_t h, int B, size_t* tape_bytes, size_t* ws_bytes);
 
-/* E1+E2 forward that keeps the tape: same outputs as comic_encode_fwd. */
+/* E1+E2 forward that keeps the tape: same outputs as comic_encode_fwd (fm_out [B,M,C] = the end point). */
 int comic_encode_train_fwd(comic_handle_t h, const float* images, int B, float* fm_out, float* im_embed_out,
                            void* tape, size_t tape_bytes, void* ws, size_t ws_bytes, void* stream);
 
 /* Backward of the InceptionV1 graph (TF autodiff of common/nets/inception_v1.py:29-339 under
- * create_train_op, src/model_base.py:387-401) from dfm [B,196,832] and dim_embed [B,1024]:
+ * create_train_op, src/model_base.py:387-401) from dfm [B,M,C] (at the end point) and dim_embed [B,1024]:
  * overwrites every grads->conv_w[i] / bn_beta[i].  Max-pool gradients go to the first maximum
  * of each window; all reductions have a fixed order (bit-reproducible). */
 int comic_encode_bwd(comic_handle_t h, const float* images, int B, const float* dfm, const float* dim_embed,
