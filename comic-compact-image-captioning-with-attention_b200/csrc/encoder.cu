@@ -645,13 +645,21 @@ namespace comic {
 // inception_preprocessing_radix.py:158-201): per image an optional left-right flip of the resized RS x RS image
 // (flip[b] != 0) followed by the crop whose top-left corner is crop_yx[b] = (y0, x0); the random draws themselves are
 // the caller's (TF's random streams cannot be reproduced).
+// offsets == nullptr: one H x W size, image b at img + b * H * W * 3.  Otherwise a ragged batch: image b is
+// hw[b] = (H, W) at img + offsets[b] (comic_preprocess_ragged); the grid is the same, so a captured launch stays valid
+// whatever the sizes of the next batch.
 __global__ void __launch_bounds__(256)
 preprocess_eval_kernel(const uint8_t* __restrict__ img, int B, int H, int W, int RS, int out_h, int out_w,
                        float* __restrict__ out, const int* __restrict__ crop_yx = nullptr,
-                       const uint8_t* __restrict__ flip = nullptr) {
+                       const uint8_t* __restrict__ flip = nullptr, const int64_t* __restrict__ offsets = nullptr,
+                       const int32_t* __restrict__ hw = nullptr) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)B * out_h * out_w) return;
   const int x = (int)(i % out_w), y = (int)((i / out_w) % out_h), b = (int)(i / ((size_t)out_w * out_h));
+  if (offsets != nullptr) {
+    H = hw[2 * b];
+    W = hw[2 * b + 1];
+  }
   // crop_or_pad: crop offset = (RS - out) / 2 when out < RS, pad offset = (out - RS) / 2 otherwise
   int ry = (out_h <= RS) ? y + (RS - out_h) / 2 : y - (out_h - RS) / 2;
   int rx = (out_w <= RS) ? x + (RS - out_w) / 2 : x - (out_w - RS) / 2;
@@ -667,7 +675,7 @@ preprocess_eval_kernel(const uint8_t* __restrict__ img, int B, int H, int W, int
     const int y0 = (int)floorf(fy), x0 = (int)floorf(fx);
     const int y1 = min(y0 + 1, H - 1), x1 = min(x0 + 1, W - 1);
     const float ly = __fsub_rn(fy, (float)y0), lx = __fsub_rn(fx, (float)x0);
-    const uint8_t* p = img + (size_t)b * H * W * 3;
+    const uint8_t* p = img + (offsets != nullptr ? (size_t)offsets[b] : (size_t)b * H * W * 3);
     const float k = 1.0f / 255.0f;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
@@ -706,6 +714,21 @@ extern "C" int comic_preprocess_train(comic_handle_t h, const uint8_t* images, i
   const size_t n = (size_t)B * out_h * out_w;
   comic::preprocess_eval_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(images, B, H, W, 256,
                                                                                             out_h, out_w, out, crop_yx, flip);
+  h->launches++;
+  COMIC_CHECK_CUDA(cudaGetLastError());
+  return COMIC_OK;
+}
+
+extern "C" int comic_preprocess_ragged(comic_handle_t h, const uint8_t* bytes, int B, const int64_t* offsets,
+                                       const int32_t* hw, int out_h, int out_w, const int32_t* crop_yx,
+                                       const uint8_t* flip, float* out, void* stream) {
+  COMIC_REQUIRE(h && bytes && offsets && hw && out, COMIC_E_BADARG, "preprocess_ragged: null argument");
+  COMIC_REQUIRE(crop_yx || !flip, COMIC_E_BADARG, "preprocess_ragged: flip needs crop_yx (training)");
+  COMIC_REQUIRE(B > 0 && out_h > 0 && out_w > 0 && (!crop_yx || (out_h <= 256 && out_w <= 256)), COMIC_E_SHAPE,
+                "preprocess_ragged: bad shape B=%d out=%dx%d (tf.random_crop needs out <= 256)", B, out_h, out_w);
+  const size_t n = (size_t)B * out_h * out_w;
+  comic::preprocess_eval_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      bytes, B, 0, 0, 256, out_h, out_w, out, crop_yx, flip, offsets, hw);
   h->launches++;
   COMIC_CHECK_CUDA(cudaGetLastError());
   return COMIC_OK;

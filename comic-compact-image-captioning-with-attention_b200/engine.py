@@ -101,6 +101,7 @@ SIGNATURES = {
     'comic_set_precision': (_I, [_P, _I]),
     'comic_set_option': (_I, [_P, _I, _I]),
     'comic_preprocess_train': (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
+    'comic_preprocess_ragged': (_I, [_P, _P, _I, _P, _P, _I, _I, _P, _P, _P, _P]),
     'comic_decode_trace': (_I, [_P, _P, _I, _P, _P]),
     'comic_train_workspace_bytes': (_I, [_P, _I, _I, C.POINTER(_SZ)]),
     'comic_dropout_masks': (_I, [_P, _P, _SZ, _F, C.c_uint64, C.c_uint64, _P]),
@@ -156,6 +157,102 @@ def _ptr(t):
     if t is None:
         return None
     return C.c_void_p(t.data_ptr())
+
+
+def grown(buf, nbytes, **kw):
+    """`buf` when it holds `nbytes`, else a new uint8 buffer of max(nbytes, 1.25 x its size): a batch a little larger
+    than the last keeps the buffer (and so the CUDA graphs captured over it) for the next batches."""
+    import torch
+    if buf is not None and buf.numel() >= nbytes:
+        return buf
+    return torch.empty(max(nbytes, 0 if buf is None else (buf.numel() * 5 + 3) // 4), dtype=torch.uint8, **kw)
+
+
+class RaggedImages(object):
+    """A batch of decoded RGB images of mixed sizes, uint8 [h_b, w_b, 3] each, as one launch pre-processes them:
+    `data` uint8 (sized to a capacity), image b row-major at data[offsets[b]:] with offsets int64 [B] and its height and
+    width in hw int32 [B, 2].  `pack_images` builds it in host memory, with the three tables and the pixels in one
+    buffer, so that `to(device)` moves the batch in one copy."""
+
+    def __init__(self, data, offsets, hw, buf=None, nbytes=0):
+        self.data, self.offsets, self.hw = data, offsets, hw
+        self._buf, self._nbytes = buf, nbytes          # the packed buffer (host batches from pack_images)
+
+    def __len__(self):
+        return int(self.offsets.shape[0])
+
+    @property
+    def nbytes(self):
+        """Bytes one copy of the packed batch moves (tables + pixels)."""
+        return self._nbytes
+
+    @staticmethod
+    def _views(buf, B):
+        import torch
+        return buf[16 * B:], buf[:8 * B].view(torch.int64), buf[8 * B:16 * B].view(torch.int32).view(B, 2)
+
+    def to(self, device, out=None):
+        """One host -> device copy (asynchronous from pinned memory, on the current stream) of the packed batch into
+        `out` (a uint8 device buffer, replaced by a larger one -- see `grown` -- when it is too small)."""
+        if self._buf is None:
+            raise ValueError('only a batch built by pack_images can be copied')
+        out = grown(out, self._nbytes, device=device)
+        out[:self._nbytes].copy_(self._buf[:self._nbytes], non_blocking=True)
+        return RaggedImages(*self._views(out, len(self)), buf=out, nbytes=self._nbytes)
+
+
+_pack_pool = None
+PACK_THREADS = min(8, os.cpu_count() or 1)
+PACK_THREADED_BYTES = 16 << 20
+
+
+def _pack_copies(jobs, total):
+    """Copy (image, byte view) pairs.  A batch of camera-size images is hundreds of MB, more than one host thread copies in
+    the time the device captions it; NumPy releases the GIL while it copies, so large batches are split over a small
+    thread pool."""
+    global _pack_pool
+
+    def run(part):
+        for im, dst in part:
+            dst.reshape(im.shape)[:] = im
+    if total < PACK_THREADED_BYTES or PACK_THREADS < 2 or len(jobs) < 2:
+        return run(jobs)
+    if _pack_pool is None:
+        from concurrent.futures import ThreadPoolExecutor
+        _pack_pool = ThreadPoolExecutor(PACK_THREADS, thread_name_prefix='pack_images')
+    list(_pack_pool.map(run, [jobs[i::PACK_THREADS] for i in range(PACK_THREADS)]))
+
+
+def pack_images(images, staging=None):
+    """A list or tuple of decoded RGB images, each uint8 [h, w, 3] with h, w >= 1 (NumPy arrays or host tensors) ->
+    RaggedImages in host memory: offsets int64 [B] | hw int32 [B, 2] | the pixels, in `staging` (a uint8 host buffer,
+    pinned so that the copy to the device is asynchronous) when it is large enough, else in a new one (`grown`).
+    Raises ValueError before any device work if an image is not such an array."""
+    import torch
+    if not isinstance(images, (list, tuple)) or not images:
+        raise ValueError('images must be a non-empty list of uint8 [h, w, 3] arrays')
+    arrs = []
+    for i, im in enumerate(images):
+        if isinstance(im, torch.Tensor) and im.device.type == 'cpu':
+            im = im.numpy()
+        if not isinstance(im, np.ndarray):
+            raise ValueError('image %d is a %s, not a uint8 [h, w, 3] array' % (i, type(im).__name__))
+        if im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3 or im.shape[0] < 1 or im.shape[1] < 1:
+            raise ValueError('image %d must be uint8 [h, w, 3] with h, w >= 1, got %s %s' % (i, im.dtype, im.shape))
+        arrs.append(im)
+    B = len(arrs)
+    hw = np.array([im.shape[:2] for im in arrs], np.int32)
+    sizes = hw[:, 0].astype(np.int64) * hw[:, 1] * 3
+    offsets = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
+    nbytes = 16 * B + int(sizes.sum())
+    if staging is None or staging.numel() < nbytes:
+        staging = grown(staging, nbytes, pin_memory=torch.cuda.is_available())
+    data, off_t, hw_t = RaggedImages._views(staging, B)
+    off_t.numpy()[:] = offsets
+    hw_t.numpy()[:] = hw
+    d = data.numpy()
+    _pack_copies([(im, d[o:o + n]) for im, o, n in zip(arrs, offsets, sizes)], nbytes)
+    return RaggedImages(data, off_t, hw_t, buf=staging, nbytes=nbytes)
 
 
 class Engine(object):
@@ -304,13 +401,27 @@ class Engine(object):
         self._wstruct = w
 
     # -- E1/E2 ----------------------------------------------------------------
+    def _check_images(self, images):
+        """The encoder reads fp32 [B,224,224,3] from this engine's device; anything else would be read as if it were."""
+        if not isinstance(images, self.torch.Tensor) or images.dtype != self.torch.float32 or images.device != self.device:
+            raise ValueError('images must be an fp32 tensor on %s, got %s' % (
+                self.device, '%s on %s' % (images.dtype, images.device) if isinstance(images, self.torch.Tensor)
+                else type(images).__name__))
+        images = images.contiguous()
+        if images.dim() != 4 or tuple(images.shape[1:]) != (224, 224, 3):
+            raise ValueError('images must be [B,224,224,3] NHWC, got %s' % (tuple(images.shape),))
+        return images
+
+    def _check_ragged(self, images):
+        if images.data.device != self.device or images.data.dtype != self.torch.uint8:
+            raise ValueError('a ragged batch must be uint8 on %s (RaggedImages.to), got %s on %s'
+                             % (self.device, images.data.dtype, images.data.device))
+
     def encode(self, images, want_mixed5c=False):
         """images [B,224,224,3] fp32 NHWC on device -> (im_embed [B,1024], fm [B,M,C]) (+ Mixed_5c [B,7,7,1024]; at
         cnn_fm_attention=Mixed_5c that is a view of fm)."""
         torch = self.torch
-        images = images.contiguous()
-        if images.dim() != 4 or tuple(images.shape[1:]) != (224, 224, 3):
-            raise ValueError('images must be [B,224,224,3] NHWC, got %s' % (tuple(images.shape),))
+        images = self._check_images(images)
         B = images.shape[0]
         fm = self.f32(B, self.dims.M, self.dims.C)
         emb = self.f32(B, self.dims.E)
@@ -325,8 +436,16 @@ class Engine(object):
 
     def preprocess_eval(self, images_u8, out_hw=(224, 224)):
         """inception_preprocessing_radix.preprocess_image(is_training=False): uint8 [B,H,W,3] on device ->
-        fp32 [B,224,224,3] in [-1,1] (resize 256 bilinear, central crop, (x - 0.5) * 2)."""
+        fp32 [B,224,224,3] in [-1,1] (resize 256 bilinear, central crop, (x - 0.5) * 2).  `images_u8` may also be a
+        RaggedImages on the device (images of mixed sizes, one launch)."""
         torch = self.torch
+        if isinstance(images_u8, RaggedImages):
+            self._check_ragged(images_u8)
+            out = self.f32(len(images_u8), int(out_hw[0]), int(out_hw[1]), 3)
+            self._check(self.lib.comic_preprocess_ragged(
+                self._h, _ptr(images_u8.data), len(images_u8), _ptr(images_u8.offsets), _ptr(images_u8.hw),
+                int(out_hw[0]), int(out_hw[1]), None, None, _ptr(out), self.stream()))
+            return out
         images_u8 = images_u8.contiguous()
         if images_u8.dtype != torch.uint8 or images_u8.dim() != 4 or images_u8.shape[3] != 3:
             raise ValueError('images must be uint8 [B,H,W,3], got %s %s' % (images_u8.dtype, tuple(images_u8.shape)))
@@ -339,12 +458,18 @@ class Engine(object):
     def preprocess_train(self, images_u8, crop_yx, flip=None, out_hw=(224, 224)):
         """inception_preprocessing_radix.preprocess_image(is_training=True): uint8 [B,H,W,3] on device -> resize 256
         bilinear -> left-right flip where flip[b] -> crop at crop_yx[b] = (y0, x0) -> (x - 0.5) * 2.  `crop_yx` int32
-        [B,2] and `flip` uint8 [B] are the caller's random draws (see train.random_crop_flip)."""
+        [B,2] and `flip` uint8 [B] are the caller's random draws (see train.random_crop_flip).  `images_u8` may also be
+        a RaggedImages on the device (images of mixed sizes, one launch)."""
         torch = self.torch
-        images_u8 = images_u8.contiguous()
-        if images_u8.dtype != torch.uint8 or images_u8.dim() != 4 or images_u8.shape[3] != 3:
-            raise ValueError('images must be uint8 [B,H,W,3], got %s %s' % (images_u8.dtype, tuple(images_u8.shape)))
-        B, H, W = (int(v) for v in images_u8.shape[:3])
+        ragged = isinstance(images_u8, RaggedImages)
+        if ragged:
+            self._check_ragged(images_u8)
+            B = len(images_u8)
+        else:
+            images_u8 = images_u8.contiguous()
+            if images_u8.dtype != torch.uint8 or images_u8.dim() != 4 or images_u8.shape[3] != 3:
+                raise ValueError('images must be uint8 [B,H,W,3], got %s %s' % (images_u8.dtype, tuple(images_u8.shape)))
+            B, H, W = (int(v) for v in images_u8.shape[:3])
         crop = torch.as_tensor(crop_yx).to(device=self.device, dtype=torch.int32).contiguous()
         if tuple(crop.shape) != (B, 2):
             raise ValueError('crop_yx must be [B, 2]')
@@ -352,6 +477,11 @@ class Engine(object):
             raise ValueError('crop offsets must lie in [0, 256 - out]')
         fl = None if flip is None else torch.as_tensor(flip).to(device=self.device, dtype=torch.uint8).contiguous()
         out = self.f32(B, int(out_hw[0]), int(out_hw[1]), 3)
+        if ragged:
+            self._check(self.lib.comic_preprocess_ragged(
+                self._h, _ptr(images_u8.data), B, _ptr(images_u8.offsets), _ptr(images_u8.hw), int(out_hw[0]),
+                int(out_hw[1]), _ptr(crop), _ptr(fl), _ptr(out), self.stream()))
+            return out
         self._check(self.lib.comic_preprocess_train(self._h, _ptr(images_u8), B, H, W, int(out_hw[0]), int(out_hw[1]),
                                                     _ptr(crop), _ptr(fl), _ptr(out), self.stream()))
         return out
@@ -608,9 +738,7 @@ class Engine(object):
         """Forward that keeps every activation: -> (im_embed [B,1024], fm [B,M,C]); the tape stays
         in this engine until `encode_bwd`."""
         torch = self.torch
-        images = images.contiguous()
-        if images.dim() != 4 or tuple(images.shape[1:]) != (224, 224, 3):
-            raise ValueError('images must be [B,224,224,3] NHWC, got %s' % (tuple(images.shape),))
+        images = self._check_images(images)
         B = images.shape[0]
         nt, nw = C.c_size_t(), C.c_size_t()
         self._check(self.lib.comic_encode_train_bytes(self._h, B, C.byref(nt), C.byref(nw)))

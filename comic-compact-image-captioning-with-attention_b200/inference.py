@@ -8,8 +8,9 @@ Same result files, same keys, same text:
     <infer_save_path>/infer_speed.txt          header once, then one images/s line per run   (infer_fn.py:175-183)
 
 The reference pulls batches out of its in-graph `InputManager`; the dataset readers are out of scope here
-(DESIGN.md §7), so the caller hands over `filenames` and an iterable of image batches `[B, 224, 224, 3]` (host or
-device) in file order.  Batches go through `CaptionModel.run_stream`, i.e. the H2D copy of batch i+1 and the D2H copy
+(DESIGN.md §7), so the caller hands over `filenames` and an iterable of image batches in file order: `[B, 224, 224, 3]`
+fp32 (host or device), raw uint8 `[B, H, W, 3]` pixels, or a list of uint8 `[h, w, 3]` images of mixed sizes (pre-processed
+on the device).  Batches go through `CaptionModel.run_stream`, i.e. the H2D copy of batch i+1 and the D2H copy
 of batch i-1 overlap the compute of batch i, where the reference issues one blocking `sess.run` per batch
 (infer_fn.py:129-130).  As in the reference only whole batches are decoded (`num_batches = int(n / batch_size)`,
 infer_fn.py:107) and every file must end up with exactly one caption (infer_fn.py:160-163).
@@ -66,7 +67,8 @@ def run_inference(config, curr_ckpt_path, model, filenames, batches):
     model      `CaptionModel(config, 'infer', ...)` (anything with `run_stream(batches)` yielding
                `[word_ids [B, T], attn_maps [B, H, T, M]]` per batch)
     filenames  image files in batch order (`InputManager.filenames_infer`)
-    batches    iterable of image batches of `config.batch_size_infer` images
+    batches    iterable of image batches of `config.batch_size_infer` images (tensors / arrays, or lists of
+               per-image uint8 [h, w, 3] arrays of mixed sizes)
     Returns (raw_outputs, coco_json, seconds)."""
     c = config
     ckpt_dir, ckpt_file = os.path.split(curr_ckpt_path)

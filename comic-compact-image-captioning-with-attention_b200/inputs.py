@@ -2,9 +2,11 @@
 common/inputs/manager_image_caption.py -- vocabulary files, word / radix / char tokenisation, shuffling, bucketing by
 caption length, padding with <PAD> -- as plain Python iterators of (image paths, int32 captions [B, L]).
 
-What is NOT here: tf.data, JPEG decoding.  Images are produced by a caller-supplied `image_loader(paths) -> uint8
-[B, h, w, 3]` (decoded pixels); the device side of the reference's preprocessing then is
-`Engine.preprocess_eval` / `Engine.preprocess_train`.  With no loader the managers yield paths and captions only.
+What is NOT here: tf.data, JPEG decoding.  Images are produced by a caller-supplied `image_loader(paths)` returning
+decoded pixels: a uint8 [B, h, w, 3] array when the images share one size, or a list of uint8 [h, w, 3] arrays of
+mixed sizes (as the files of a real dataset are); the device side of the reference's preprocessing then is
+`Engine.preprocess_eval` / `Engine.preprocess_train`, which `CaptionModel.run` / `run_stream`, `Trainer.step` and
+`scst.scst_step` run themselves on such batches.  With no loader the managers yield paths and captions only.
 
 Reference behaviour reproduced (file:line of common/inputs/manager_image_caption.py):
   * vocabulary: `captions/<pattern.format('itow')>.json`, `...('wtoi')>.json`; `vocab_size = len(itow)` (:98-108);

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import rops
 from . import weights as wts
-from .engine import ComicError, Engine
+from .engine import ComicError, Engine, RaggedImages, grown, pack_images
 
 
 def number_to_base(n, base):
@@ -55,9 +55,11 @@ class ModelBase(object):
     collect_attention_maps = True
 
     def _encoder(self, images):
-        if images.dtype == self.engine.torch.uint8:
-            # raw decoded pixels: the reference's evaluation pre-processing on the device
-            # (inception_preprocessing_radix.py:229-235, 270-273)
+        if isinstance(images, (list, tuple)):
+            images = pack_images(images).to(self.engine.device)
+        if isinstance(images, RaggedImages) or images.dtype == self.engine.torch.uint8:
+            # raw decoded pixels (one size, or a packed batch of mixed sizes): the reference's evaluation
+            # pre-processing on the device (inception_preprocessing_radix.py:229-235, 270-273)
             images = self.engine.preprocess_eval(images)
         self.im_embed, self.cnn_fmaps = self.engine.encode(images)
         return self.im_embed, self.cnn_fmaps
@@ -182,7 +184,8 @@ class CaptionModel(ModelBase):
         (the reference's train graph); `seed` fixes the masks, dropout=False disables them."""
         assert self.mode == 'train'
         eng = self.engine
-        images = eng.torch.as_tensor(images).to(eng.device, non_blocking=True)
+        if not isinstance(images, (list, tuple)):
+            images = eng.torch.as_tensor(images).to(eng.device, non_blocking=True)
         out = self.trainer.step(images, np.asarray(captions), None, seed, lr, dropout)
         self.dec_log_ppl = out['loss'][1]
         return self.dec_log_ppl, self.trainer.global_step
@@ -237,17 +240,22 @@ class CaptionModel(ModelBase):
     def run(self, images=None):
         """One `sess.run(self.infer_output)` (src/infer_fn.py:130): images
         [B,224,224,3] NHWC fp32 (host numpy / torch -- pinned memory copies
-        asynchronously -- or a device tensor).  Returns [dec_preds (B,T) int32,
+        asynchronously -- or a device tensor), raw uint8 [B,H,W,3] pixels, or a
+        list of uint8 [h,w,3] images of mixed sizes (packed, one copy, one
+        pre-processing launch).  Returns [dec_preds (B,T) int32,
         attn_maps (B,H,T,M) fp32] as numpy views of pinned staging buffers that
         the next call overwrites."""
         eng = self.engine
         torch = eng.torch
         if images is None:
             images = self.batch_ops[0]
-        images = torch.as_tensor(images)
-        if images.dtype not in (torch.float32, torch.uint8):
-            images = images.float()
-        dev_images = images.to(eng.device, non_blocking=True).contiguous()
+        if isinstance(images, (list, tuple)):
+            dev_images = pack_images(images).to(eng.device)
+        else:
+            images = torch.as_tensor(images)
+            if images.dtype not in (torch.float32, torch.uint8):
+                images = images.float()
+            dev_images = images.to(eng.device, non_blocking=True).contiguous()
         self._encoder(dev_images)
         self._decoder_rnn()
         preds = self._to_host(self.dec_preds, 'preds')
@@ -266,7 +274,11 @@ class CaptionModel(ModelBase):
         following `next()`.  Device-resident batches skip the input copy.
 
         Batches may be uint8 [B,H,W,3] raw pixels: they cross PCIe as bytes (a quarter of the fp32 volume) and the
-        reference's evaluation pre-processing runs on the device.  With `collect_attention_maps = False` the second
+        reference's evaluation pre-processing runs on the device.  A batch may also be a list or tuple of uint8
+        [h,w,3] images of mixed sizes: the host packs it (pack_images) into the slot's pinned staging buffer while the
+        device computes the previous batch, one copy moves it into the slot's device buffer, and one launch
+        pre-processes it.  Both buffers grow by at least 1.25x to the largest batch seen, so the slot's graph keeps
+        replaying while the sizes change.  With `collect_attention_maps = False` the second
         element of every result is None and neither history nor maps are written or copied."""
         eng = self.engine
         torch = eng.torch
@@ -280,11 +292,25 @@ class CaptionModel(ModelBase):
 
         def stage_in(i, images):
             sl = slots[i % depth]
+            if isinstance(images, (list, tuple)):
+                if sl.get('ev_in') is not None:
+                    sl['ev_in'].synchronize()               # the slot's previous copy has read its staging buffer
+                packed = pack_images(images, sl.get('stage'))
+                sl['stage'] = packed._buf
+                buf = sl['dev_ragged'] = grown(sl.get('dev_ragged'), packed.nbytes, device=dev)
+                with torch.cuda.stream(s_in):
+                    if sl.get('ev_comp') is not None:
+                        s_in.wait_event(sl['ev_comp'])
+                    r = packed.to(dev, buf)
+                    ev = torch.cuda.Event()
+                    ev.record(s_in)
+                sl['dev'], sl['ev_in'] = (r.data, r.offsets, r.hw), ev
+                return
             images = torch.as_tensor(images)
             if images.dtype not in (torch.float32, torch.uint8):
                 images = images.float()
             if images.is_cuda:
-                sl['dev'], sl['ev_in'] = images.contiguous(), None
+                sl['dev'], sl['ev_in'] = (images.contiguous(),), None
                 return
             buf = sl.get('dev_in')
             if buf is None or buf.shape != images.shape or buf.dtype != images.dtype:
@@ -295,7 +321,7 @@ class CaptionModel(ModelBase):
                 buf.copy_(images, non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(s_in)
-            sl['dev'], sl['ev_in'] = buf, ev
+            sl['dev'], sl['ev_in'] = (buf,), ev
 
         def pinned(sl, key, t):
             b = sl.get(key)
@@ -307,8 +333,9 @@ class CaptionModel(ModelBase):
             sl = slots[i % depth]
             if sl['ev_in'] is not None:
                 comp.wait_event(sl['ev_in'])
-            def device_step(images):
+            def device_step(*images):
                 # no host sync inside (rops: _defer_T): full-length results + the device step count, trimmed in finish()
+                images = images[0] if len(images) == 1 else RaggedImages(*images)
                 self._defer_T = True
                 try:
                     self._encoder(images)
@@ -320,7 +347,7 @@ class CaptionModel(ModelBase):
                         self.dec_time.reshape(1))
             # one CUDA graph per input slot (Engine.graphed): replayed from the slot's third batch on
             preds, attn, t_dev = eng.graphed(('run_stream', i % depth, bool(self.collect_attention_maps)), device_step,
-                                             sl['dev'])
+                                             *sl['dev'])
             ev = torch.cuda.Event()
             ev.record(comp)
             sl['ev_comp'] = ev

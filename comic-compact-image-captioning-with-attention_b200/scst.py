@@ -356,10 +356,13 @@ def sample_captions(engine, config, images, beam, max_length=20):
 
 
 def scst_step(trainer, scorer, images, refs, seed=None, lr=None, dropout=True):
-    """train_fn_scst loop body.  images [B,224,224,3] device tensor; refs: list (per image) of
-    reference caption strings.  Returns dict(loss, rewards, sc_sample, sc_greedy, hypos)."""
+    """train_fn_scst loop body.  images [B,224,224,3] fp32 device tensor, or raw uint8 pixels (a [B,H,W,3] tensor or a
+    list of [h,w,3] arrays of mixed sizes) pre-processed on the device as `Trainer.prepare_images` does; refs: list (per
+    image) of reference caption strings.  Returns dict(loss, rewards, sc_sample, sc_greedy, hypos) plus the
+    augmentation draws crop_yx / flip of raw pixels under `cnn_input_augment`."""
     c, eng = trainer.c, trainer.engine
     k = c.scst_beam_size
+    images, draws = trainer.prepare_images(images, seed)
     cap_beam, cap_greedy, im_embed, fm = sample_captions(eng, c, images, k)
     cb = cap_beam.cpu().numpy()
     cb = cb.reshape(-1, cb.shape[-1])                                     # [[im0_h0]..[imN_h0],[im0_h1]..]
@@ -381,4 +384,6 @@ def scst_step(trainer, scorer, images, refs, seed=None, lr=None, dropout=True):
     out = trainer.forward_backward(fm_t, im_t, hypos_idx, rewards, masks, keeps)
     out['lr'] = trainer.apply_gradients(lr)
     out.update(rewards=rewards, sc_sample=sc_sample, sc_greedy=sc_greedy, hypos=hypos, greedy=hyp_greedy)
+    if draws:
+        out.update(draws)
     return out

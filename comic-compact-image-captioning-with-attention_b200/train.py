@@ -20,7 +20,7 @@ import os
 import numpy as np
 
 from . import weights as wts
-from .engine import Engine
+from .engine import Engine, pack_images
 
 
 def process_inputs(captions, token_type):
@@ -136,6 +136,8 @@ class Trainer(object):
             self.cnn_grad_w = [self.gradient(wts.CNN + sc + '/weights') for sc, *_ in convs]
             self.cnn_grad_b = [self.gradient(wts.CNN + sc + '/BatchNorm/beta') for sc, *_ in convs]
         self.global_step = 0
+        # crop / flip draws of `cnn_input_augment` for raw-pixel batches when a step gives no seed
+        self._augment_rng = np.random.default_rng(int(getattr(c, 'rand_seed', 48964896)))
         self.reg = torch.zeros(1, dtype=torch.float32, device=eng.device)
         # slim clip_gradient_norms: per-variable slices of the flat gradient buffer (device tables for comic_clip_by_norm)
         self.clip_norm = float(getattr(c, 'clip_gradient_norm', 0) or 0)
@@ -344,11 +346,36 @@ class Trainer(object):
             eng.refresh_packed()
         return lr
 
+    def prepare_images(self, images, seed=None):
+        """The images of one step as the encoder takes them.  fp32 [B,224,224,3] images are returned as given.  Raw
+        decoded pixels -- a uint8 [B,H,W,3] tensor or array, or a list of uint8 [h,w,3] arrays of mixed sizes (packed
+        and copied to the device in one copy) -- are pre-processed on the device: with `cnn_input_augment`,
+        `preprocess_for_train` with a random flip and crop per image (train.random_crop_flip, drawn from a host
+        generator seeded by `seed`, else by config.rand_seed), otherwise the evaluation pre-processing.  Returns
+        (fp32 images, draws): draws = dict(crop_yx, flip) of the augmentation, else None."""
+        torch, eng = self.torch, self.engine
+        if isinstance(images, (list, tuple)):
+            raw = pack_images(images).to(eng.device)
+            B = len(raw)
+        elif isinstance(images, (np.ndarray, torch.Tensor)) and images.dtype in (np.uint8, torch.uint8):
+            raw = eng.to_dev(images)
+            B = int(raw.shape[0])
+        else:
+            return images, None
+        if getattr(self.c, 'cnn_input_augment', False):
+            rng = np.random.default_rng(seed) if seed is not None else self._augment_rng
+            crop, flip = random_crop_flip(B, rng=rng)
+            return eng.preprocess_train(raw, crop, flip), dict(crop_yx=crop, flip=flip)
+        return eng.preprocess_eval(raw), None
+
     def step(self, images, captions, rewards=None, seed=None, lr=None, dropout=True):
         """One `sess.run([train_op])`: encoder forward (frozen, or with tape when fine-tuning), decoder
         fwd+bwd (+ encoder backward), optimiser.  Dropout is ON as in the reference's train graph (masks seeded by
-        `seed`, default derived from config.rand_seed and the global step); dropout=False runs without masks."""
+        `seed`, default derived from config.rand_seed and the global step); dropout=False runs without masks.
+        `images` may be raw uint8 pixels (see prepare_images); the augmentation draws are then returned as
+        out['crop_yx'] and out['flip']."""
         eng = self.engine
+        images, draws = self.prepare_images(images, seed)
         m5c = None
         if self.finetune_cnn:
             images = eng.to_dev(images)
@@ -365,4 +392,6 @@ class Trainer(object):
         out = self.forward_backward(fm, im_embed, captions, rewards, masks, keeps,
                                     images=images if self.finetune_cnn else None, mixed5c=m5c)
         out['lr'] = self.apply_gradients(lr)
+        if draws:
+            out.update(draws)
         return out

@@ -215,7 +215,8 @@ int comic_encode_fwd(comic_handle_t h, const float* images, int B, float* fm_out
 /* Evaluation pre-processing, common/inputs/preprocessing/inception_preprocessing_radix.py:229-235, 270-273
  * (convert_image_dtype -> resize_bilinear 256x256, align_corners=False -> central crop / zero pad to
  * out_h x out_w -> (x - 0.5) * 2), fused.  images uint8 [B,H,W,3] (decoded RGB, one size per call);
- * out fp32 [B,out_h,out_w,3] = the `images` argument of comic_encode_fwd. */
+ * out fp32 [B,out_h,out_w,3] = the `images` argument of comic_encode_fwd.  A batch of images of mixed sizes takes
+ * comic_preprocess_ragged instead. */
 int comic_preprocess_eval(comic_handle_t h, const uint8_t* images, int B, int H, int W, int out_h, int out_w,
                           float* out, void* stream);
 
@@ -226,6 +227,16 @@ int comic_preprocess_eval(comic_handle_t h, const uint8_t* images, int B, int H,
  * [B,out_h,out_w,3] device. */
 int comic_preprocess_train(comic_handle_t h, const uint8_t* images, int B, int H, int W, int out_h, int out_w,
                            const int32_t* crop_yx, const uint8_t* flip, float* out, void* stream);
+
+/* The same pre-processing for a batch of decoded RGB images of mixed sizes, in one launch whose grid depends on B and
+ * out_h x out_w only.  Image b is hw[b] = (h, w) uint8 [h,w,3] at bytes + offsets[b].  crop_yx == NULL: evaluation
+ * (as comic_preprocess_eval, flip must be NULL); otherwise training (as comic_preprocess_train, with its out <= 256
+ * rule).  bytes, offsets (int64 [B]), hw (int32 [B,2]), crop_yx, flip and out are device pointers; the library cannot
+ * read the tables without a synchronise, so the caller guarantees h, w >= 1 and that every image lies inside the
+ * buffer.  Each image gives the bits comic_preprocess_eval / comic_preprocess_train give it alone. */
+int comic_preprocess_ragged(comic_handle_t h, const uint8_t* bytes, int B, const int64_t* offsets, const int32_t* hw,
+                            int out_h, int out_w, const int32_t* crop_yx, const uint8_t* flip, float* out,
+                            void* stream);
 
 /* D0: MultiHeadAttV3.__init__ common/ops_rnn.py:441-477: keys = fm.W_k once per
  * IMAGE (the reference does it per tiled beam row); values_out only for
